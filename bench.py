@@ -4,6 +4,8 @@
     python bench.py --gpus N --steps K --warmup W            our arm (hand-written sm_100a kernels via the C ABI)
     python bench.py --impl reference ...                     the reference algorithm's CPU path (oracle port) on the
                                                              box's host cores, same workload / metric / unit
+    python bench.py ... --dump-outputs DIR                   also write the last timed step's loss, predictions and
+                                                             gradients as DIR/<name>.npy (compare two builds)
 
 Workload (BASELINE.json configs[1]): mm.yaml default MultiModal (5+5 layers, H 256, 8 heads, MLP 512), modalities
 ap (N=668 spike channels, the yaml's n_channels) + behavior (wheel speed, whisker motion energy), T=100 bins,
@@ -55,6 +57,11 @@ def parse():
                     help="skip timing the unmodified reference on the GPU through stock PyTorch")
     ap.add_argument("--sustained-seconds", type=float, default=2.0,
                     help="length of the extra back-to-back leg that reports throughput under sustained clocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (loss, per-modality losses, "
+                         "example counts and predictions, parameter gradients) as DIR/<name>.npy in float32 / float64, "
+                         "at most 60 MiB in all: an array over its share is replaced by a fixed, seeded sample of its "
+                         "elements (1-D, in flat-index order)")
     a = ap.parse_args()
     scaled = a.workload == "scaled"
     if a.batch is None:
@@ -347,6 +354,38 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 60 << 20       # --dump-outputs: all arrays together
+DUMP_SAMPLE_SEED = 20240601
+
+
+def dump_outputs(path, out, model, store):
+    """Write one step's results (``MultiModalOutput`` + the gradients in the engine's flat buffer) as .npy files, so two
+    builds can be compared output for output.  Smallest arrays first, each keeps at most an equal share of the bytes
+    still left; a larger array is replaced by that many elements at seeded positions (the same positions in every run
+    with the same shapes)."""
+    import numpy as np
+    import torch
+    arrays = {"loss": out.loss}
+    for m in out.mod_loss:
+        arrays[f"mod_loss.{m}"] = out.mod_loss[m]
+        arrays[f"mod_n_examples.{m}"] = out.mod_n_examples[m]
+        arrays[f"mod_preds.{m}"] = out.mod_preds[m]
+    for n, _ in model.named_parameters():
+        arrays[f"grad.{n}"] = store.g(n)
+    host = {k: v.detach().to("cpu", torch.float32 if v.is_floating_point() else torch.float64) for k, v in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES - 256 * len(host)          # .npy headers
+    items = sorted(host.items(), key=lambda kv: kv[1].numel())
+    for i, (name, v) in enumerate(items):
+        keep = min(v.numel(), left // (len(items) - i) // v.element_size())
+        if keep < v.numel():
+            g = torch.Generator().manual_seed(DUMP_SAMPLE_SEED)
+            idx = torch.randperm(v.numel(), generator=g)[:keep].sort().values
+            v = v.flatten()[idx]
+        left -= keep * v.element_size()
+        np.save(os.path.join(path, f"{name}.npy"), v.numpy())
+
+
 def main():
     a = parse()
     if a.impl == "reference":
@@ -388,11 +427,14 @@ def main():
     dev_batches = [{k: (v.to(dev) if torch.is_tensor(v) else v) for k, v in hb.items()} for hb in host_batches]
     dev_dicts = [make_mod_dict(dev_batches[i], wl.mods, MODES[i % 3], device=dev) for i in range(NB)]
 
+    last_out = [None]
+
     def step_resident(i):
         md = {k: dict(v) for k, v in dev_dicts[i % NB].items()}
         out = model(md)
         out.loss.backward()
         model.zero_grad(set_to_none=True)
+        last_out[0] = out
         return out
 
     from multi_modal_foundation_model_b200.synthetic import DevicePrefetcher
@@ -448,6 +490,9 @@ def main():
     ms = timed(step_resident, a.steps)
     clocks = sampler.stop() if rank == 0 else None
     value = B * n_gpus * a.steps / (ms / 1e3)
+    if a.dump_outputs and rank == 0:
+        # zero_grad(set_to_none) only drops the .grad views: the flat buffer still holds the last timed step's gradients
+        dump_outputs(a.dump_outputs, last_out[0], model, eng.store)
 
     # the same loop held for >= --sustained-seconds back to back: throughput under the clocks a long job really sees
     sustained = None

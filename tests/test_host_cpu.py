@@ -11,7 +11,7 @@ import pytest
 import torch
 
 import _reference as ref
-from _util import GOLDEN, small_config
+from _util import GOLDEN, load_small, small_config
 from multi_modal_foundation_model_b200 import _lib
 from multi_modal_foundation_model_b200.config import default_model_config
 from multi_modal_foundation_model_b200.masker import Masker
@@ -62,14 +62,16 @@ def test_initial_weights_match_reference_seed42():
         assert np.allclose(got, z[k], rtol=1e-12, atol=1e-12), k
 
 
-@pytest.mark.skipif(not ref.available(), reason="reference tree not mounted")
-def test_state_dict_keys_match_reference_live():
-    cfg = ref.load_config()
-    rm = ref.build_reference_model(cfg, 32, 2)
-    ours = build_model(32, 2, cfg["model"])          # accepts the reference's own DictConfig
-    assert list(ours.state_dict().keys()) == list(rm.state_dict().keys())
-    ours.load_state_dict(rm.state_dict())
-    assert ours.decoder_embeddings["ap"].embedder.mod_emb is ours.encoder_embeddings["ap"].embedder.mod_emb
+def test_state_dict_keys_match_reference_golden():
+    """The reference's state_dict keys, in its order, as stored by tests/golden/make_golden.py: the default model
+    (init_default.npz) and the small fixture model, whose reference weights load into ours unchanged (mm_small.npz)."""
+    ours = build_model(32, 2, default_model_config())
+    assert list(ours.state_dict().keys()) == list(np.load(os.path.join(GOLDEN, "init_default.npz")).files)
+    _, weights = load_small()
+    small = build_model(40, 2, small_config())
+    assert list(small.state_dict().keys()) == list(weights)
+    small.load_state_dict(weights)
+    assert small.decoder_embeddings["ap"].embedder.mod_emb is small.encoder_embeddings["ap"].embedder.mod_emb
 
 
 def test_model_pickles_without_engine_handles():
