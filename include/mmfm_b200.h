@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MMFM_ABI_VERSION 4
+#define MMFM_ABI_VERSION 5
 
 const char* mmfm_last_error(void);
 int mmfm_abi_version(void);
@@ -282,6 +282,58 @@ int mmfm_column_stats(const float* pred, const float* y, long long R, int C, int
  * the bias corrections.  Decoupled weight decay, no amsgrad, maximize = false. */
 int mmfm_adamw_step(float* p, const float* g, float* exp_avg, float* exp_avg_sq, long long n, float lr, float beta1,
                     float beta2, float eps, float weight_decay, long long step, void* stream);
+
+/* ---- deterministic mode (torch.use_deterministic_algorithms(True)) ---------------------------------------------
+ * The entry points above that reduce across CTAs with float atomics have a *_det twin with the same arguments plus a
+ * caller-owned workspace.  There every CTA writes its partial to the workspace and a ticketed pairwise tree folds the
+ * partials in an order fixed by the grid, so results are bitwise reproducible for the same inputs, shapes and device
+ * (the grid depends on the SM count).  No CTA waits for another.  The outputs accumulate (+=) exactly as in the
+ * default entry points; they differ from them in the last bits.
+ * The workspace: buf (16-byte aligned) of at least the size reported by mmfm_det_ws_bytes, and that many tickets,
+ * zeroed once by the caller; every launch leaves its tickets at zero again.  Calls on one stream may share one
+ * workspace.  A workspace that is too small is rejected (return -1), never overrun. */
+typedef struct mmfm_det_ws {
+  void* buf;
+  long long bytes;
+  unsigned int* tickets;
+  int n_tickets;
+} mmfm_det_ws;
+enum mmfm_det_kind {              /* (d0, d1, d2) of mmfm_det_ws_bytes */
+  MMFM_DET_WGRAD = 0,             /* (R, NO, KI) */
+  MMFM_DET_COLSUM = 1,            /* (R, NO, -) */
+  MMFM_DET_LN_BWD = 2,            /* (R, H, -) */
+  MMFM_DET_LN_BWD_MULTI = 3,      /* (R, H, n) */
+  MMFM_DET_SCALENORM_BWD = 4,     /* (R, H, -) */
+  MMFM_DET_EMBED_ASM_BWD = 5,     /* (B, T, H) */
+  MMFM_DET_SMALLC_EMBED_BWD = 6,  /* (B*T, C, H) */
+  MMFM_DET_SMALLC_HEAD_BWD = 7,   /* (R, H, C) */
+  MMFM_DET_COLUMN_STATS = 8       /* (R, C, -) */
+};
+/* Host only (queries the device's SM count, launches nothing): workspace bytes and tickets one *_det call of `kind`
+ * at these sizes needs, from the same grid arithmetic as its launcher.  Returns 0, or -1 on a bad kind / shape. */
+int mmfm_det_ws_bytes(int kind, long long d0, long long d1, long long d2, long long* bytes, int* n_tickets);
+int mmfm_gemm_wgrad_det(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI, float* dW,
+                        long long ldw, float* dbias, const mmfm_det_ws* ws, void* stream);
+int mmfm_colsum_bf16_det(const void* dY, long long ld, int R, int NO, float* out, const mmfm_det_ws* ws, void* stream);
+int mmfm_layernorm_bwd_det(const void* dy, const float* x, const float* mean, const float* rstd, const float* gamma,
+                           const float* dres, float* dx, void* dxb, const mmfm_dropout* drop, float* dgamma,
+                           float* dbeta, int R, int H, int modmajor_T, int S, const mmfm_det_ws* ws, void* stream);
+int mmfm_layernorm_bwd_multi_det(const mmfm_ln_multi_args* a, const mmfm_det_ws* ws, void* stream);
+int mmfm_scalenorm_bwd_det(const void* dy, const float* x, const float* rnorm, const float* g, const float* dres,
+                           float* dx, void* dxb, const mmfm_dropout* drop, float* dg, int R, int H, float eps,
+                           const mmfm_det_ws* ws, void* stream);
+/* n_pos = rows of dpos: timestamps outside [0, n_pos) contribute to dmod only.  dpos rows are summed over (b, t) in
+ * increasing b * T + t order by one CTA per row. */
+int mmfm_embed_assemble_bwd_det(const float* g, const float* g2, const long long* ts, float* dpos, float* dmod, int B,
+                                int T, int S, int off, int H, int n_pos, const mmfm_det_ws* ws, void* stream);
+int mmfm_smallc_embed_bwd_det(const float* in, const float* hid, const float* W2, const float* dx,
+                              const unsigned char* row_zero, const mmfm_dropout* drop, float act_scale, int act,
+                              float* dW1, float* db1, float* dW2, float* db2, int B, int T, int S, int off, int C, int H,
+                              const mmfm_det_ws* ws, void* stream);
+int mmfm_smallc_head_bwd_det(const void* y, const float* W, const void* dpreds, long long lddp, void* dy, float* dW,
+                             float* db, int R, int H, int C, const mmfm_det_ws* ws, void* stream);
+int mmfm_column_stats_det(const float* pred, const float* y, long long R, int C, int log_rate, double* out,
+                          const mmfm_det_ws* ws, void* stream);
 
 #ifdef __cplusplus
 }

@@ -20,7 +20,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
               "-Xptxas", "-v"]
 
 MAX_MOD = 8
-ABI_VERSION = 4
+ABI_VERSION = 5
 MASK_SITE = 8192
 
 
@@ -150,12 +150,19 @@ class CastItem(C.Structure):
     ]
 
 
+class DetWs(C.Structure):
+    _fields_ = [("buf", C.c_void_p), ("bytes", C.c_longlong), ("tickets", C.c_void_p), ("n_tickets", C.c_int)]
+
+
 ACT_NONE, ACT_GELU, ACT_SOFTSIGN, ACT_DGELU, ACT_DSOFTSIGN, ACT_GELU_DG, ACT_MULAUX, ACT_ROWDOT_DROP = 0, 1, 2, 3, 4, 5, 6, 7
 MASK_KEY, MASK_KEY_OR_DIAG, MASK_CAUSAL = 0, 1, 2
 LOSS_POISSON, LOSS_MSE, LOSS_CE = 0, 1, 2
+(DET_WGRAD, DET_COLSUM, DET_LN_BWD, DET_LN_BWD_MULTI, DET_SCALENORM_BWD, DET_EMBED_ASM_BWD, DET_SMALLC_EMBED_BWD,
+ DET_SMALLC_HEAD_BWD, DET_COLUMN_STATS) = range(9)
 
 _vp, _i, _ll, _f = C.c_void_p, C.c_int, C.c_longlong, C.c_float
 _DP = C.POINTER(Dropout)
+_WS = C.POINTER(DetWs)
 
 # name -> argtypes; every function returns int except the three listed in _SPECIAL
 SIGNATURES = {
@@ -187,6 +194,18 @@ SIGNATURES = {
     "mmfm_smallc_head_bwd": [_vp, _vp, _vp, _ll, _vp, _vp, _vp, _i, _i, _i, _vp],
     "mmfm_loss_fwd_bwd": [_vp, _vp, _vp, _i, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp, _ll, _vp],
     "mmfm_loss_finalize": [_vp, _i, _i, _vp, _vp, _vp, _vp],
+    # deterministic mode: the same arguments plus the workspace (include/mmfm_b200.h)
+    "mmfm_det_ws_bytes": [_i, _ll, _ll, _ll, C.POINTER(C.c_longlong), C.POINTER(C.c_int)],
+    "mmfm_gemm_wgrad_det": [_vp, _ll, _vp, _ll, _i, _i, _i, _vp, _ll, _vp, _WS, _vp],
+    "mmfm_colsum_bf16_det": [_vp, _ll, _i, _i, _vp, _WS, _vp],
+    "mmfm_layernorm_bwd_det": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _DP, _vp, _vp, _i, _i, _i, _i, _WS, _vp],
+    "mmfm_layernorm_bwd_multi_det": [C.POINTER(LnMultiArgs), _WS, _vp],
+    "mmfm_scalenorm_bwd_det": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _DP, _vp, _i, _i, _f, _WS, _vp],
+    "mmfm_embed_assemble_bwd_det": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _WS, _vp],
+    "mmfm_smallc_embed_bwd_det": [_vp, _vp, _vp, _vp, _vp, _DP, _f, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _WS,
+                                  _vp],
+    "mmfm_smallc_head_bwd_det": [_vp, _vp, _vp, _ll, _vp, _vp, _vp, _i, _i, _i, _WS, _vp],
+    "mmfm_column_stats_det": [_vp, _vp, _ll, _i, _i, _vp, _WS, _vp],
 }
 _SPECIAL = {
     "mmfm_last_error": ([], C.c_char_p),

@@ -505,6 +505,68 @@ MMFM_DEVINL float quad_max(float v) {
   return v;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Deterministic mode (torch.use_deterministic_algorithms): fixed-order fold of per-CTA partial vectors
+// ------------------------------------------------------------------------------------------------
+MMFM_DEVINL float det_add(float a, float b) { return a + b; }
+MMFM_DEVINL double det_add(double a, double b) { return a + b; }
+MMFM_DEVINL float4 det_add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
+
+// Ticketed pairwise tree over the n_leaves partial vectors slot(i) = ws + i * stride (n elements of V each) of one
+// reduction.  Every CTA of the reduction calls it with all its threads after writing slot(leaf) (and after pdl_wait).
+// At level l node k covers slot k << l; the nodes 2j and 2j+1 meet at ticket ((2j+1) << l) - 1.  The CTA that arrives
+// second adds the two slots into the left one and climbs; the first one exits; an unpaired last node climbs as it is.
+// The CTA that completes the root pair calls emit(i, total_i) for i in [0, n) instead of storing it.  The tree's shape
+// depends only on n_leaves and a + b == b + a in IEEE arithmetic, so the result does not depend on which CTA arrives
+// last, and no CTA ever waits for another.  The second arrival clears its ticket: a launch leaves its n_leaves - 1
+// tickets at zero for the next one (graph replays need no memset).
+template <typename V, typename Emit>
+MMFM_DEVINL void det_tree_fold(V* ws, long long stride, int n, int leaf, int n_leaves, unsigned int* tickets,
+                               Emit emit) {
+  __shared__ unsigned int s_second;
+  int node = leaf;
+  for (int l = 0; (1 << l) < n_leaves; ++l) {
+    const int width = (n_leaves + (1 << l) - 1) >> l;
+    if ((node | 1) >= width) { node >>= 1; continue; }
+    const int right = (node | 1) << l;
+    __syncthreads();   // this CTA's writes to its slot are done ...
+    if (threadIdx.x == 0) {
+      __threadfence();   // ... and visible device-wide before the ticket
+      const unsigned int t = atomicAdd(tickets + right - 1, 1u);
+      if (t != 0u) {
+        tickets[right - 1] = 0u;
+        __threadfence();   // the partner's slot writes (fenced before its ticket) are visible to this CTA
+      }
+      s_second = t;
+    }
+    __syncthreads();
+    if (s_second == 0u) return;
+    V* a = ws + (long long)((node & ~1) << l) * stride;
+    const V* b = ws + (long long)right * stride;
+    // kU elements per thread in flight: one CTA moves the whole pair, so the level time is L2 latency-bound otherwise
+    constexpr int kU = 8;
+    for (int i0 = threadIdx.x; i0 < n; i0 += kU * blockDim.x) {
+      V va[kU], vb[kU];
+#pragma unroll
+      for (int u = 0; u < kU; ++u) {
+        const int i = i0 + u * blockDim.x;
+        if (i < n) { va[u] = __ldcg(a + i); vb[u] = __ldcg(b + i); }
+      }
+#pragma unroll
+      for (int u = 0; u < kU; ++u) {
+        const int i = i0 + u * blockDim.x;
+        if (i >= n) break;
+        if (width == 2) emit(i, det_add(va[u], vb[u]));
+        else a[i] = det_add(va[u], vb[u]);
+      }
+    }
+    if (width == 2) return;
+    node >>= 1;
+  }
+  __syncthreads();   // n_leaves == 1: the total is this CTA's own slot
+  for (int i = threadIdx.x; i < n; i += blockDim.x) emit(i, __ldcg(ws + (long long)leaf * stride + i));
+}
+
 // one random byte for element (row, col) of a (rows, cols) dropout field (slow path; hot loops fetch 16 at once)
 MMFM_DEVINL uint32_t drop_byte_at(unsigned long long seed, uint32_t site, uint64_t row, uint32_t groups_per_row,
                                   uint32_t col) {

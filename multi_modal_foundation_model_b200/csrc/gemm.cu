@@ -501,12 +501,18 @@ __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_con
 // shared-memory bandwidth (every operand byte is written once by TMA and read once by the tensor core; a 128 x 128 x 16
 // MMA alone reads 128 B/clk), and the wider tile moves 25 % fewer bytes per FLOP and reads every dY box once instead of
 // once per 128-column tile.
-template <int STAGES, int BN>
+// DET (deterministic mode, no clusters): instead of red.global, each split CTA writes its fp32 tile and bias column to
+// its workspace slot [tile][split] and the splits of a tile are folded by det_tree_fold (common.cuh) into dW / dbias.
+template <int BN>
+__host__ __device__ constexpr long long wgrad_slot_f4() { return ((long long)kBM * BN + kBM) / 4; }   // float4s per workspace slot
+
+template <int STAGES, int BN, bool DET = false>
 __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_constant__ CUtensorMap tmY,
                                                                    const __grid_constant__ CUtensorMap tmX, int R,
                                                                    int NO, int KI, float* __restrict__ dW,
                                                                    long long ldw, int rows_per_split,
-                                                                   float* __restrict__ dbias, int cx, int cy) {
+                                                                   float* __restrict__ dbias, int cx, int cy,
+                                                                   float4* __restrict__ ws, unsigned int* tickets) {
   // (cx, cy) = thread-block cluster shape over (KI tiles, NO tiles), 1 or 2 each.  The CTAs of a cluster work on the
   // same rows: the two KI tiles of a cluster row share their dY boxes, the two NO tiles of a cluster column share their
   // X boxes, so each CTA loads HALF of what it consumes and TMA-multicasts it to its peer (this kernel is bound by
@@ -656,7 +662,13 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
       uint32_t bacc[16];
       tmem_ld16(t_row + (uint32_t)BN, bacc);
       tmem_ld_wait();
-      if (no0 + row_l < NO) atomicAdd(dbias + no0 + row_l, __uint_as_float(bacc[0]));
+      if constexpr (DET) {
+        float* slot = reinterpret_cast<float*>(ws + (blockIdx.z + (long long)gridDim.z * (blockIdx.y * gridDim.x + blockIdx.x)) *
+                                                        wgrad_slot_f4<BN>());
+        slot[kBM * BN + row_l] = __uint_as_float(bacc[0]);
+      } else {
+        if (no0 + row_l < NO) atomicAdd(dbias + no0 + row_l, __uint_as_float(bacc[0]));
+      }
     }
     __syncwarp();
     // coalesced accumulation: lane = 4 consecutive columns, one row (128 columns of it) per step
@@ -672,6 +684,11 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
         const int no = no0 + rl;
         if (no >= NO || nvalid <= 0) continue;
         const float4 v = *reinterpret_cast<const float4*>(stage_f + rl * kPitch + lcol);
+        if constexpr (DET) {
+          ws[(blockIdx.z + (long long)gridDim.z * (blockIdx.y * gridDim.x + blockIdx.x)) * wgrad_slot_f4<BN>() +
+             (rl * BN + lcol) / 4] = v;
+          continue;
+        }
         float* dst = dW + (long long)no * ldw + kcol;
         if (vec) {
           asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(v.x), "f"(v.y), "f"(v.z),
@@ -690,18 +707,46 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
   __syncthreads();
   if (clustered) cluster_sync_all();   // no CTA leaves while a peer's commit may still arrive on its barriers
   if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
+  if constexpr (DET) {
+    const long long tile = blockIdx.y * gridDim.x + blockIdx.x;
+    const bool vec = (ldw % 4 == 0) && ((reinterpret_cast<uintptr_t>(dW) & 15) == 0);
+    det_tree_fold(ws + tile * gridDim.z * wgrad_slot_f4<BN>(), wgrad_slot_f4<BN>(),
+                  (kBM * BN + (do_bias ? kBM : 0)) / 4, blockIdx.z, gridDim.z, tickets + tile * gridDim.z,
+                  [&](int i, float4 v) {
+                    const int e = 4 * i;
+                    if (e >= kBM * BN) {   // bias column
+                      const float vv[4] = {v.x, v.y, v.z, v.w};
+                      for (int u = 0; u < 4; ++u)
+                        if (no0 + e - kBM * BN + u < NO) dbias[no0 + e - kBM * BN + u] += vv[u];
+                      return;
+                    }
+                    const int no = no0 + e / BN, kcol = ki0 + e % BN;
+                    if (no >= NO || kcol >= KI) return;
+                    float* dst = dW + (long long)no * ldw + kcol;
+                    if (vec && kcol + 4 <= KI) {
+                      float4 o = *reinterpret_cast<float4*>(dst);
+                      *reinterpret_cast<float4*>(dst) = det_add(o, v);
+                      return;
+                    }
+                    const float vv[4] = {v.x, v.y, v.z, v.w};
+                    for (int u = 0; u < 4 && kcol + u < KI; ++u) dst[u] += vv[u];
+                  });
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
 // bias gradient: out[c] += sum_r dY[r,c]
 // ------------------------------------------------------------------------------------------------
 constexpr int kColsumRows = 256;
+// DET: the CTAs of a column slice (blockIdx.x) fold their 512 column sums with det_tree_fold instead of atomics
+template <bool DET = false>
 __global__ void __launch_bounds__(256) colsum_bf16_kernel(const bf16* __restrict__ dY, long long ld, int R, int NO,
-                                                           float* __restrict__ out) {
+                                                           float* __restrict__ out, float* __restrict__ ws,
+                                                           unsigned int* tickets) {
   const int c = (blockIdx.x * 256 + threadIdx.x) * 2;
-  if (c >= NO) return;
+  if (!DET && c >= NO) return;
   const int r0 = blockIdx.y * kColsumRows;
-  const int r1 = min(R, r0 + kColsumRows);
+  const int r1 = (DET && c >= NO) ? r0 : min(R, r0 + kColsumRows);   // (DET: every thread takes part in the fold)
   float s0 = 0.f, s1 = 0.f;
   if (c + 1 < NO && (ld & 1) == 0) {
     for (int r = r0; r < r1; ++r) {
@@ -715,6 +760,16 @@ __global__ void __launch_bounds__(256) colsum_bf16_kernel(const bf16* __restrict
       s0 += __bfloat162float(dY[(long long)r * ld + c]);
       if (c + 1 < NO) s1 += __bfloat162float(dY[(long long)r * ld + c + 1]);
     }
+  }
+  if constexpr (DET) {
+    float* slices = ws + (long long)blockIdx.x * gridDim.y * 512;
+    slices[blockIdx.y * 512 + 2 * threadIdx.x] = s0;
+    slices[blockIdx.y * 512 + 2 * threadIdx.x + 1] = s1;
+    det_tree_fold(slices, 512, 512, blockIdx.y, gridDim.y, tickets + (long long)blockIdx.x * gridDim.y,
+                  [&](int i, float v) {
+                    if (blockIdx.x * 512 + i < NO) out[blockIdx.x * 512 + i] += v;
+                  });
+    return;
   }
   atomicAdd(out + c, s0);
   if (c + 1 < NO) atomicAdd(out + c + 1, s1);
@@ -873,6 +928,26 @@ extern "C" int mmfm_gemm_tn(const mmfm_gemm_args* a, void* stream) {
   }
 }
 
+// split-R arithmetic of the wgrad launch (also the deterministic workspace size: one slot per CTA)
+static int wgrad_splits(int R, int NO, int KI, int BN, int* rows_per_split) {
+  const int tiles = ((NO + kBM - 1) / kBM) * ((KI + BN - 1) / BN);
+  const int kblocks = (R + kBK - 1) / kBK;
+  static int waves_x2 = -1;   // MMFM_WGRAD_CTAS_X2: target CTA count in half-SM-counts (default 4 = two CTAs per SM)
+  if (waves_x2 < 0) {
+    const char* e = getenv("MMFM_WGRAD_CTAS_X2");
+    waves_x2 = e ? atoi(e) : 4;
+    if (waves_x2 < 1) waves_x2 = 4;
+  }
+  // all CTAs must be resident at once (two per SM): a split count rounded UP spills a few CTAs into a second wave that
+  // costs as much as the first (measured 43 us vs 34 us on the QKV shape), so round down
+  // BN 256: one CTA per SM (144 KB of stages, 512 TMEM columns); BN 128: two
+  int splits = ((BN == 256 ? 2 : waves_x2) * device_sm_count() / 2) / tiles;
+  if (splits > kblocks) splits = kblocks;
+  if (splits < 1) splits = 1;
+  *rows_per_split = ((kblocks + splits - 1) / splits) * kBK;
+  return (R + *rows_per_split - 1) / *rows_per_split;
+}
+
 template <int BN>
 static int launch_wgrad(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI, float* dW,
                         long long ldw, float* dbias, void* stream) {
@@ -889,22 +964,8 @@ static int launch_wgrad(const void* dY, long long lddy, const void* X, long long
                                          (int)smem));
     attr_set = true;
   }
-  const int tiles = ((NO + kBM - 1) / kBM) * ((KI + BN - 1) / BN);
-  const int kblocks = (R + kBK - 1) / kBK;
-  static int waves_x2 = -1;   // MMFM_WGRAD_CTAS_X2: target CTA count in half-SM-counts (default 4 = two CTAs per SM)
-  if (waves_x2 < 0) {
-    const char* e = getenv("MMFM_WGRAD_CTAS_X2");
-    waves_x2 = e ? atoi(e) : 4;
-    if (waves_x2 < 1) waves_x2 = 4;
-  }
-  // all CTAs must be resident at once (two per SM): a split count rounded UP spills a few CTAs into a second wave that
-  // costs as much as the first (measured 43 us vs 34 us on the QKV shape), so round down
-  // BN 256: one CTA per SM (144 KB of stages, 512 TMEM columns); BN 128: two
-  int splits = ((BN == 256 ? 2 : waves_x2) * device_sm_count() / 2) / tiles;
-  if (splits > kblocks) splits = kblocks;
-  if (splits < 1) splits = 1;
-  int rows_per_split = ((kblocks + splits - 1) / splits) * kBK;
-  splits = (R + rows_per_split - 1) / rows_per_split;
+  int rows_per_split = 0;
+  const int splits = wgrad_splits(R, NO, KI, BN, &rows_per_split);
   dim3 grid((KI + BN - 1) / BN, (NO + kBM - 1) / kBM, splits);
   static int mc_env = -1;   // MMFM_WGRAD_MULTICAST=1: 2x2 clusters, each CTA loads half of its boxes and multicasts them
   if (mc_env < 0) {
@@ -927,9 +988,58 @@ static int launch_wgrad(const void* dY, long long lddy, const void* X, long long
   cfg.attrs = attr;
   cfg.numAttrs = 2;
   MMFM_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_wgrad_kernel<STAGES, BN>, tmY, tmX, R, NO, KI, dW, ldw, rows_per_split, dbias,
-                                     cx, cy));
+                                     cx, cy, (float4*)nullptr, (unsigned int*)nullptr));
   return 0;
 }
+
+// deterministic twin: always the 128-wide tile without clusters (MMFM_WGRAD_BN / MMFM_WGRAD_MULTICAST do not apply)
+static DetNeed wgrad_det_need(int R, int NO, int KI) {
+  int rows_per_split = 0;
+  const int splits = wgrad_splits(R, NO, KI, 128, &rows_per_split);
+  const long long ctas = (long long)((NO + kBM - 1) / kBM) * ((KI + 127) / 128) * splits;
+  return DetNeed{ctas * wgrad_slot_f4<128>() * 16, (int)ctas};
+}
+
+static int launch_wgrad_det(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI,
+                            float* dW, long long ldw, float* dbias, const mmfm_det_ws* ws, cudaStream_t st) {
+  constexpr int STAGES = 3, BN = 128;
+  MMFM_REQUIRE(ws != nullptr, "mmfm_gemm_wgrad_det: null workspace");
+  if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, wgrad_det_need(R, NO, KI),
+                            "mmfm_gemm_wgrad_det"))
+    return rc;
+  CUtensorMap tmY, tmX;
+  int rc = make_tmap_bf16_2d(&tmY, dY, (uint64_t)R, (uint64_t)NO, (uint64_t)lddy, 64, kBK, TMA_SW_128);
+  if (rc) return rc;
+  rc = make_tmap_bf16_2d(&tmX, X, (uint64_t)R, (uint64_t)KI, (uint64_t)ldx, 64, kBK, TMA_SW_128);
+  if (rc) return rc;
+  constexpr size_t smem = (size_t)STAGES * ((2 + BN / 64) * 64 * kBK * 2) + 2048 + 1024;
+  static bool attr_set = false;
+  if (!attr_set) {
+    MMFM_CHECK_CUDA(cudaFuncSetAttribute(gemm_wgrad_kernel<STAGES, BN, true>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr_set = true;
+  }
+  int rows_per_split = 0;
+  const int splits = wgrad_splits(R, NO, KI, BN, &rows_per_split);
+  MMFM_CHECK_CUDA(launch_pdl(gemm_wgrad_kernel<STAGES, BN, true>, dim3((KI + BN - 1) / BN, (NO + kBM - 1) / kBM, splits),
+                             dim3(kGemmThreads), smem, st, tmY, tmX, R, NO, KI, dW, ldw, rows_per_split, dbias, 1, 1,
+                             (float4*)ws->buf, ws->tickets));
+  return 0;
+}
+
+static DetNeed colsum_det_need(int R, int NO) {
+  const long long slices = (NO + 511) / 512, parts = (R + kColsumRows - 1) / kColsumRows;
+  return DetNeed{slices * parts * 512 * 4, (int)(slices * parts)};
+}
+
+namespace mmfm {
+bool det_need_gemm(int kind, long long d0, long long d1, long long d2, DetNeed* need) {
+  if (kind == MMFM_DET_WGRAD) *need = wgrad_det_need((int)d0, (int)d1, (int)d2);
+  else if (kind == MMFM_DET_COLSUM) *need = colsum_det_need((int)d0, (int)d1);
+  else return false;
+  return true;
+}
+}  // namespace mmfm
 
 
 extern "C" int mmfm_gemm_wgrad(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI,
@@ -945,10 +1055,29 @@ extern "C" int mmfm_gemm_wgrad(const void* dY, long long lddy, const void* X, lo
   return launch_wgrad<128>(dY, lddy, X, ldx, R, NO, KI, dW, ldw, dbias, stream);
 }
 
+extern "C" int mmfm_gemm_wgrad_det(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI,
+                                   float* dW, long long ldw, float* dbias, const mmfm_det_ws* ws, void* stream) {
+  MMFM_REQUIRE(dY && X && dW, "mmfm_gemm_wgrad_det: null operand");
+  MMFM_REQUIRE(R > 0 && NO > 0 && KI > 0, "mmfm_gemm_wgrad_det: bad shape R=%d NO=%d KI=%d", R, NO, KI);
+  return launch_wgrad_det(dY, lddy, X, ldx, R, NO, KI, dW, ldw, dbias, ws, (cudaStream_t)stream);
+}
+
 extern "C" int mmfm_colsum_bf16(const void* dY, long long ld, int R, int NO, float* out, void* stream) {
   MMFM_REQUIRE(dY && out && R > 0 && NO > 0, "mmfm_colsum_bf16: bad arguments");
   dim3 grid((NO + 511) / 512, (R + kColsumRows - 1) / kColsumRows);
-  colsum_bf16_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const bf16*)dY, ld, R, NO, out);
+  colsum_bf16_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const bf16*)dY, ld, R, NO, out, nullptr, nullptr);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_colsum_bf16_det(const void* dY, long long ld, int R, int NO, float* out, const mmfm_det_ws* ws,
+                                    void* stream) {
+  MMFM_REQUIRE(dY && out && R > 0 && NO > 0 && ws, "mmfm_colsum_bf16_det: bad arguments");
+  if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, colsum_det_need(R, NO), "mmfm_colsum_bf16_det"))
+    return rc;
+  dim3 grid((NO + 511) / 512, (R + kColsumRows - 1) / kColsumRows);
+  colsum_bf16_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>((const bf16*)dY, ld, R, NO, out, (float*)ws->buf,
+                                                                   ws->tickets);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

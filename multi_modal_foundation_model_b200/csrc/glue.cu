@@ -117,9 +117,13 @@ constexpr int kAsmLanes = 4;
 constexpr int kModReplicas = 16;
 __device__ float g_dmod_scratch[kModReplicas][1024];   // H <= 1024 (checked by the launcher); all zero between launches
 __device__ unsigned int g_dmod_ticket;
+// DET (called with dpos == NULL; embed_pos_bwd_det_kernel below owns dpos): the CTA's modality-embedding sum goes to
+// its workspace slot and det_tree_fold adds the slots up, instead of the scratch replicas.
+template <bool DET = false>
 __global__ void embed_assemble_bwd_kernel(const float* __restrict__ g, const float* __restrict__ g2,
                                           const long long* __restrict__ ts, float* __restrict__ dpos,
-                                          float* __restrict__ dmod, int B, int T, int S, int off, int H, int bchunk) {
+                                          float* __restrict__ dmod, int B, int T, int S, int off, int H, int bchunk,
+                                          float4* __restrict__ ws, unsigned int* tickets) {
   extern __shared__ float4 sm_acc[];                      // [kAsmLanes][H/4]
   const int t = blockIdx.x;
   const int b0 = blockIdx.y * bchunk, b1 = min(B, b0 + bchunk);
@@ -145,14 +149,14 @@ __global__ void embed_assemble_bwd_kernel(const float* __restrict__ g, const flo
             const float4 w = __ldg(reinterpret_cast<const float4*>(g2 + row) + c);
             v[u].x += w.x; v[u].y += w.y; v[u].z += w.z; v[u].w += w.w;
           }
-          if (dpos) id[u] = ts[(long long)b * T + t];
+          if (!DET && dpos) id[u] = ts[(long long)b * T + t];
         }
       }
 #pragma unroll
       for (int u = 0; u < kU; ++u) {
         if (bb + u * kAsmLanes >= b1) break;
         accm.x += v[u].x; accm.y += v[u].y; accm.z += v[u].z; accm.w += v[u].w;
-        if (dpos) {
+        if (!DET && dpos) {
           const long long idx = id[u];
           if (idx != cur) {
             if (cur >= 0) {
@@ -166,13 +170,27 @@ __global__ void embed_assemble_bwd_kernel(const float* __restrict__ g, const flo
         }
       }
     }
-    if (dpos && cur >= 0) {
+    if (!DET && dpos && cur >= 0) {
       float* d = dpos + cur * H + c * 4;
       atomicAdd(d, acc.x); atomicAdd(d + 1, acc.y); atomicAdd(d + 2, acc.z); atomicAdd(d + 3, acc.w);
     }
     sm_acc[sl * ncol + c] = accm;
   }
   __syncthreads();
+  if constexpr (DET) {
+    const int leaf = blockIdx.x + blockIdx.y * gridDim.x;
+    if (sl == 0) {
+      float4 tot = sm_acc[c];
+#pragma unroll
+      for (int l = 1; l < kAsmLanes; ++l) tot = det_add(tot, sm_acc[l * ncol + c]);
+      ws[(long long)leaf * ncol + c] = tot;
+    }
+    det_tree_fold(ws, ncol, ncol, leaf, gridDim.x * gridDim.y, tickets, [&](int i, float4 v) {
+      float4* d = reinterpret_cast<float4*>(dmod) + i;
+      *d = det_add(*d, v);
+    });
+    return;
+  }
   // Modality-embedding gradient = sum over ALL rows: hundreds of CTAs adding to the same H addresses serialise in L2
   // (600 atomics per address at B = 256), so the CTAs spread their sums over kModReplicas scratch copies and the last
   // CTA to finish (ticket) folds the copies into dmod and clears them for the next launch.  (One launch in flight per
@@ -201,6 +219,70 @@ __global__ void embed_assemble_bwd_kernel(const float* __restrict__ g, const flo
       atomicAdd(dmod + col, sum);
     }
     if (threadIdx.x == 0) g_dmod_ticket = 0u;
+  }
+}
+
+// Deterministic position-embedding gradient: CTA p owns row p of dpos and sums the gradient rows of every (b, t) with
+// ts[b, t] == p.  The CTA scans ts in chunks of 1024 (b * T + t order), compacts the hits of a chunk in order, and its
+// thread groups (256 / (H/4) of them, one float4 column per thread) take the hits round-robin; the group sums are added
+// in group order at the end.  The summation order depends only on ts, so repeated and permuted timestamps are fine.
+constexpr int kPosScan = 4;   // ts entries per thread per chunk
+__global__ void __launch_bounds__(256) embed_pos_bwd_det_kernel(const float* __restrict__ g, const float* __restrict__ g2,
+                                                                const long long* __restrict__ ts, float* __restrict__ dpos,
+                                                                int B, int T, int S, int off, int H) {
+  __shared__ int list[256 * kPosScan];
+  __shared__ int wsum[8];
+  __shared__ float4 gsum[256];
+  const int p = blockIdx.x;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int ncol = H >> 2, groups = 256 / ncol;
+  const int grp = threadIdx.x / ncol, c = threadIdx.x - grp * ncol;
+  const int BT = B * T;
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int e0 = 0; e0 < BT; e0 += 256 * kPosScan) {
+    const int eb = e0 + threadIdx.x * kPosScan;
+    unsigned int hit = 0u;
+#pragma unroll
+    for (int u = 0; u < kPosScan; ++u)
+      if (eb + u < BT && __ldg(ts + eb + u) == p) hit |= 1u << u;
+    const int nh = __popc(hit);
+    int x = nh;   // inclusive warp scan of the hit counts
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) wsum[warp] = x;
+    __syncthreads();
+    int pos = x - nh, total = 0;
+#pragma unroll
+    for (int w = 0; w < 8; ++w) {
+      if (w < warp) pos += wsum[w];
+      total += wsum[w];
+    }
+#pragma unroll
+    for (int u = 0; u < kPosScan; ++u)
+      if (hit & (1u << u)) list[pos++] = eb + u;
+    __syncthreads();
+    if (grp < groups) {
+      for (int k = grp; k < total; k += groups) {
+        const int e = list[k];
+        const int b = e / T, t = e - b * T;
+        const long long row = ((long long)b * S + off + t) * H;
+        float4 v = __ldg(reinterpret_cast<const float4*>(g + row) + c);
+        if (g2) v = det_add(v, __ldg(reinterpret_cast<const float4*>(g2 + row) + c));
+        acc = det_add(acc, v);
+      }
+    }
+    __syncthreads();   // list / wsum are rewritten by the next chunk
+  }
+  if (grp < groups) gsum[threadIdx.x] = acc;
+  __syncthreads();
+  if (grp == 0) {
+    float4 tot = gsum[c];
+    for (int j = 1; j < groups; ++j) tot = det_add(tot, gsum[j * ncol + c]);
+    float4* d = reinterpret_cast<float4*>(dpos + (long long)p * H) + c;
+    *d = det_add(*d, tot);
   }
 }
 
@@ -285,12 +367,24 @@ __global__ void __launch_bounds__(256) smallc_embed_fwd_kernel(const float* __re
 
 // CTA = chunk of rows, thread = hidden column h (blockDim == H <= 1024).  Register partials for dW2/db2 (thread h)
 // and dW1/db1 (threads j < 2C); flushed with atomics at the end.
+// Deterministic mode: a CTA's partial gradients go to its workspace slot laid out as the outputs,
+// [db2 (H) | dW2 (H x 2C) | db1 (2C) | dW1 (2C x C)], and det_tree_fold adds the slots into them.
+MMFM_DEVINL int smallc_embed_slot(int H, int C) { return H * (1 + 2 * C) + 2 * C * (1 + C); }
+MMFM_DEVINL void smallc_embed_emit(int i, float v, int H, int C, float* dW1, float* db1, float* dW2, float* db2) {
+  const int C2 = 2 * C;
+  if (i < H) db2[i] += v;
+  else if ((i -= H) < H * C2) dW2[i] += v;
+  else if ((i -= H * C2) < C2) db1[i] += v;
+  else dW1[i - C2] += v;
+}
+
+template <bool DET = false>
 __global__ void smallc_embed_bwd_kernel(const float* __restrict__ in, const float* __restrict__ hid,
                                         const float* __restrict__ W2, const float* __restrict__ dx,
                                         const unsigned char* __restrict__ row_zero, DropCfg drop, float act_scale, int act,
                                         float* __restrict__ dW1, float* __restrict__ db1, float* __restrict__ dW2,
                                         float* __restrict__ db2, int B, int T, int S, int off, int C, int H,
-                                        int rows_per_cta) {
+                                        int rows_per_cta, float* __restrict__ ws, unsigned int* tickets) {
   __shared__ float red[32][kMaxC2 + 1];
   const int h = threadIdx.x, warp = h >> 5, lane = h & 31, nw = blockDim.x >> 5;
   const int C2 = 2 * C;
@@ -344,6 +438,23 @@ __global__ void smallc_embed_bwd_kernel(const float* __restrict__ in, const floa
         if (c < C) aw1[c] += dh * in[r * C + c];
     }
     __syncthreads();
+  }
+  if constexpr (DET) {
+    const int n = smallc_embed_slot(H, C);
+    float* slot = ws + (long long)blockIdx.x * n;
+    slot[h] = ab2;
+#pragma unroll
+    for (int j = 0; j < kMaxC2; ++j)
+      if (j < C2) slot[H + h * C2 + j] = aw2[j];
+    if (h < C2) {
+      slot[H + H * C2 + h] = ab1;
+#pragma unroll
+      for (int c = 0; c < kMaxC; ++c)
+        if (c < C) slot[H + H * C2 + C2 + h * C + c] = aw1[c];
+    }
+    det_tree_fold(ws, n, n, blockIdx.x, gridDim.x, tickets,
+                  [&](int i, float v) { smallc_embed_emit(i, v, H, C, dW1, db1, dW2, db2); });
+    return;
   }
   atomicAdd(db2 + h, ab2);
 #pragma unroll
@@ -421,11 +532,12 @@ __global__ void __launch_bounds__(256) smallc_embed_fwd16_kernel(
   }
 }
 
-template <int C>
+template <int C, bool DET = false>
 __global__ void __launch_bounds__(256) smallc_embed_bwd16_kernel(
     const float* __restrict__ in, const float* __restrict__ hid, const float* __restrict__ W2, const float* __restrict__ dx,
     const unsigned char* __restrict__ row_zero, DropCfg drop, float act_scale, int act, float* __restrict__ dW1,
-    float* __restrict__ db1, float* __restrict__ dW2, float* __restrict__ db2, int B, int T, int S, int off, int H) {
+    float* __restrict__ db1, float* __restrict__ dW2, float* __restrict__ db2, int B, int T, int S, int off, int H,
+    float* __restrict__ ws, unsigned int* tickets) {
   constexpr int C2 = 2 * C;
   __shared__ float red[4096 + 256];                         // [CTA row slot][H + 1]: (256/gpr) * (16 gpr + 1) floats
   const int gpr = H >> 4;                                   // 16-column groups per row: a power of two <= 32
@@ -531,10 +643,32 @@ __global__ void __launch_bounds__(256) smallc_embed_bwd16_kernel(
     for (int col = threadIdx.x; col < H; col += 256) {
       float sum = 0.f;
       for (int rr = 0; rr < nrow; ++rr) sum += red[rr * pitch + col];
-      if (q == 0) atomicAdd(db2 + col, sum);
+      if constexpr (DET) ws[(long long)blockIdx.x * smallc_embed_slot(H, C) + (q == 0 ? col : H + col * C2 + (q - 1))] = sum;
+      else if (q == 0) atomicAdd(db2 + col, sum);
       else atomicAdd(dW2 + col * C2 + (q - 1), sum);
     }
     __syncthreads();
+  }
+  if constexpr (DET) {   // the embedder-input gradients of the g == 0 threads, reduced in thread order
+    constexpr int kIn = C2 * (1 + C);
+    if (g == 0) {
+#pragma unroll
+      for (int j = 0; j < C2; ++j) {
+        red[trow * kIn + j] = ab1[j];
+#pragma unroll
+        for (int c = 0; c < C; ++c) red[trow * kIn + C2 + j * C + c] = aw1[j][c];
+      }
+    }
+    __syncthreads();
+    const int n = smallc_embed_slot(H, C);
+    if (threadIdx.x < kIn) {
+      float sum = 0.f;
+      for (int rr = 0; rr < nrow; ++rr) sum += red[rr * kIn + threadIdx.x];
+      ws[(long long)blockIdx.x * n + H * (1 + C2) + threadIdx.x] = sum;
+    }
+    det_tree_fold(ws, n, n, blockIdx.x, gridDim.x, tickets,
+                  [&](int i, float v) { smallc_embed_emit(i, v, H, C, dW1, db1, dW2, db2); });
+    return;
   }
   if (g == 0) {
 #pragma unroll
@@ -578,10 +712,14 @@ __global__ void __launch_bounds__(256) smallc_head_fwd_kernel(const bf16* __rest
 }
 
 // head backward, C <= 8: grid (row chunks, H/256); lane owns 8 consecutive columns of the 256-wide slice
+// DET: workspace slot per CTA = [dW slice (kMaxC x 256) | db (kMaxC)]; one tree per 256-column slice (blockIdx.y)
+constexpr int kHeadSlot = kMaxC * 256 + kMaxC;
+template <bool DET = false>
 __global__ void __launch_bounds__(256) smallc_head_bwd_kernel(const bf16* __restrict__ y, const float* __restrict__ W,
                                                                const bf16* __restrict__ dp, long long lddp,
                                                                bf16* __restrict__ dy, float* __restrict__ dW,
-                                                               float* __restrict__ db, int R, int H, int C) {
+                                                               float* __restrict__ db, int R, int H, int C,
+                                                               float* __restrict__ ws, unsigned int* tickets) {
   __shared__ float red[8][256 + 1];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h0 = blockIdx.y * 256 + lane * 8;
@@ -637,9 +775,34 @@ __global__ void __launch_bounds__(256) smallc_head_bwd_kernel(const bf16* __rest
       float s = 0.f;
 #pragma unroll
       for (int wv = 0; wv < 8; ++wv) s += red[wv][hh];
-      if (blockIdx.y * 256 + hh < H) atomicAdd(dW + (long long)c * H + blockIdx.y * 256 + hh, s);
+      if constexpr (DET) ws[((long long)blockIdx.y * gridDim.x + blockIdx.x) * kHeadSlot + c * 256 + hh] = s;
+      else if (blockIdx.y * 256 + hh < H) atomicAdd(dW + (long long)c * H + blockIdx.y * 256 + hh, s);
       __syncthreads();
     }
+  }
+  if constexpr (DET) {
+    float* slot = ws + ((long long)blockIdx.y * gridDim.x + blockIdx.x) * kHeadSlot;
+    if (lane == 0) {
+#pragma unroll
+      for (int c = 0; c < kMaxC; ++c) red[warp][c] = ab[c];
+    }
+    __syncthreads();
+    if (threadIdx.x < kMaxC) {
+      float s = 0.f;
+#pragma unroll
+      for (int wv = 0; wv < 8; ++wv) s += red[wv][threadIdx.x];
+      slot[kMaxC * 256 + threadIdx.x] = s;
+    }
+    det_tree_fold(ws + (long long)blockIdx.y * gridDim.x * kHeadSlot, kHeadSlot, kHeadSlot, blockIdx.x, gridDim.x,
+                  tickets + (long long)blockIdx.y * gridDim.x, [&](int i, float v) {
+                    const int c = i >> 8, hh = blockIdx.y * 256 + (i & 255);
+                    if (i >= kMaxC * 256) {
+                      if (blockIdx.y == 0 && i - kMaxC * 256 < C) db[i - kMaxC * 256] += v;
+                    } else if (c < C && hh < H) {
+                      dW[(long long)c * H + hh] += v;
+                    }
+                  });
+    return;
   }
   if (blockIdx.y == 0 && lane == 0) {
 #pragma unroll
@@ -888,9 +1051,12 @@ __global__ void __launch_bounds__(256) u8_expand_kernel(const unsigned char* __r
 // for log-rate predictions (zero rates become 1e-9 as in eval_utils.py:1086-1091 otherwise).  Bits per spike per neuron
 // and R^2 per channel follow from these sums (metrics.py).  CTA = a slab of rows, thread = column (strided), double
 // accumulators, one atomicAdd per column per CTA.
+// DET: the CTA's 4 * C sums go to its workspace slot and det_tree_fold adds the slots into out
+template <bool DET = false>
 __global__ void __launch_bounds__(256) column_stats_kernel(const float* __restrict__ p, const float* __restrict__ y,
                                                             long long R, int C, int log_rate, int rows_per_cta,
-                                                            double* __restrict__ out) {
+                                                            double* __restrict__ out, double* __restrict__ ws,
+                                                            unsigned int* tickets) {
   const long long r0 = (long long)blockIdx.x * rows_per_cta, r1 = min(R, r0 + rows_per_cta);
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
     double sy = 0.0, syy = 0.0, se = 0.0, sn = 0.0;
@@ -905,11 +1071,20 @@ __global__ void __launch_bounds__(256) column_stats_kernel(const float* __restri
       se += (double)d * d;
       sn += (double)rate - (double)yv * lr;
     }
+    if constexpr (DET) {
+      double* slot = ws + (long long)blockIdx.x * 4 * C;
+      slot[c] = sy;
+      slot[C + c] = syy;
+      slot[2ll * C + c] = se;
+      slot[3ll * C + c] = sn;
+      continue;
+    }
     atomicAdd(out + c, sy);
     atomicAdd(out + C + c, syy);
     atomicAdd(out + 2ll * C + c, se);
     atomicAdd(out + 3ll * C + c, sn);
   }
+  if constexpr (DET) det_tree_fold(ws, 4ll * C, 4 * C, blockIdx.x, gridDim.x, tickets, [&](int i, double v) { out[i] += v; });
 }
 
 // CSR ubyte -> dense uint8 (SURVEY section 8f rank 2; dataset_utils.py:38-43 rebuilds each trial with scipy on the host).
@@ -984,19 +1159,24 @@ extern "C" int mmfm_embed_assemble(const float* mod_emb_row, const float* pos_em
   return 0;
 }
 
+static int embed_bwd_chunks(int B, int T, int* bchunk) {
+  int chunks = (4 * device_sm_count() + T - 1) / T;
+  if (chunks > B) chunks = B;
+  if (chunks < 1) chunks = 1;
+  *bchunk = (B + chunks - 1) / chunks;
+  return (B + *bchunk - 1) / *bchunk;
+}
+
 extern "C" int mmfm_embed_assemble_bwd(const float* g, const float* g2, const long long* ts, float* dpos, float* dmod,
                                        int B, int T, int S, int off, int H, void* stream) {
   MMFM_REQUIRE(g && dmod && (dpos == nullptr || ts), "mmfm_embed_assemble_bwd: null pointer");
   MMFM_REQUIRE(B > 0 && T > 0 && H % 4 == 0 && off >= 0 && off + T <= S, "mmfm_embed_assemble_bwd: bad shape");
-  int chunks = (4 * device_sm_count() + T - 1) / T;
-  if (chunks > B) chunks = B;
-  if (chunks < 1) chunks = 1;
-  const int bchunk = (B + chunks - 1) / chunks;
-  chunks = (B + bchunk - 1) / bchunk;
+  int bchunk = 0;
+  const int chunks = embed_bwd_chunks(B, T, &bchunk);
   MMFM_REQUIRE(H % 4 == 0 && H / 4 * kAsmLanes <= 1024, "mmfm_embed_assemble_bwd: H=%d not supported (H %% 4, H <= 1024)", H);
   const int threads = H / 4 * kAsmLanes;
   embed_assemble_bwd_kernel<<<dim3(T, chunks), threads, (size_t)threads * sizeof(float4), (cudaStream_t)stream>>>(
-      g, g2, ts, dpos, dmod, B, T, S, off, H, bchunk);
+      g, g2, ts, dpos, dmod, B, T, S, off, H, bchunk, nullptr, nullptr);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -1049,8 +1229,8 @@ extern "C" int mmfm_smallc_embed_bwd(const float* in, const float* hid, const fl
     const long long slots = (long long)B * T * gpr;
     int grid = device_sm_count();        // ~230 registers per thread: one CTA per SM, one wave
     if ((long long)grid * 256 > slots) grid = (int)((slots + 255) / 256);
-    if (C == 1) smallc_embed_bwd16_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act, dW1, db1, dW2, db2, B, T, S, off, H);
-    else smallc_embed_bwd16_kernel<2><<<grid, 256, 0, (cudaStream_t)stream>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act, dW1, db1, dW2, db2, B, T, S, off, H);
+    if (C == 1) smallc_embed_bwd16_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act, dW1, db1, dW2, db2, B, T, S, off, H, nullptr, nullptr);
+    else smallc_embed_bwd16_kernel<2><<<grid, 256, 0, (cudaStream_t)stream>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act, dW1, db1, dW2, db2, B, T, S, off, H, nullptr, nullptr);
     MMFM_CHECK_CUDA(cudaGetLastError());
     return 0;
   }
@@ -1060,7 +1240,8 @@ extern "C" int mmfm_smallc_embed_bwd(const float* in, const float* hid, const fl
   if (rows_per_cta < 16) rows_per_cta = 16;
   ctas = (int)((R + rows_per_cta - 1) / rows_per_cta);
   smallc_embed_bwd_kernel<<<ctas, H, 0, (cudaStream_t)stream>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act,
-                                                                dW1, db1, dW2, db2, B, T, S, off, C, H, rows_per_cta);
+                                                                dW1, db1, dW2, db2, B, T, S, off, C, H, rows_per_cta,
+                                                                nullptr, nullptr);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -1082,7 +1263,7 @@ extern "C" int mmfm_smallc_head_bwd(const void* y, const float* W, const void* d
   const int cap = 2 * device_sm_count();
   if (gx > cap) gx = cap;
   smallc_head_bwd_kernel<<<dim3(gx, (H + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-      (const bf16*)y, W, (const bf16*)dpreds, lddp, (bf16*)dy, dW, db, R, H, C);
+      (const bf16*)y, W, (const bf16*)dpreds, lddp, (bf16*)dy, dW, db, R, H, C, nullptr, nullptr);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -1164,7 +1345,7 @@ extern "C" int mmfm_column_stats(const float* pred, const float* y, long long R,
   int rows_per_cta = (int)((R + ctas - 1) / ctas);
   if (rows_per_cta < 8) rows_per_cta = 8;
   ctas = (int)((R + rows_per_cta - 1) / rows_per_cta);
-  column_stats_kernel<<<ctas, 256, 0, st>>>(pred, y, R, C, log_rate, rows_per_cta, out);
+  column_stats_kernel<<<ctas, 256, 0, st>>>(pred, y, R, C, log_rate, rows_per_cta, out, nullptr, nullptr);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -1173,6 +1354,145 @@ extern "C" int mmfm_csr_to_dense_u8(const unsigned char* data, const int* indice
                                     long long n_rows, int N, unsigned char* out, void* stream) {
   MMFM_REQUIRE(row_ptr && out && n_rows > 0 && N > 0, "mmfm_csr_to_dense_u8: bad arguments");
   csr_to_dense_u8_kernel<<<ew_grid(n_rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(data, indices, row_ptr, n_rows, N, out);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// deterministic twins (column sums folded by det_tree_fold; one workspace slot per CTA, same grids as above)
+// ------------------------------------------------------------------------------------------------------------
+static bool smallc_fast16(int C, int H) { return C <= 2 && H % 16 == 0 && H / 16 <= 32 && 32 % (H / 16) == 0; }
+static int smallc_fast16_grid(long long R, int H) {
+  const long long slots = R * (H / 16);
+  int grid = device_sm_count();
+  if ((long long)grid * 256 > slots) grid = (int)((slots + 255) / 256);
+  return grid;
+}
+static int smallc_generic_ctas(long long R, int* rows_per_cta) {
+  int ctas = 2 * device_sm_count();
+  *rows_per_cta = (int)((R + ctas - 1) / ctas);
+  if (*rows_per_cta < 16) *rows_per_cta = 16;
+  return (int)((R + *rows_per_cta - 1) / *rows_per_cta);
+}
+static int head_bwd_gx(int R) {
+  const int gx = (R + 63) / 64, cap = 2 * device_sm_count();
+  return gx > cap ? cap : gx;
+}
+static int column_stats_ctas(long long R, int* rows_per_cta) {
+  int ctas = 4 * device_sm_count();
+  *rows_per_cta = (int)((R + ctas - 1) / ctas);
+  if (*rows_per_cta < 8) *rows_per_cta = 8;
+  return (int)((R + *rows_per_cta - 1) / *rows_per_cta);
+}
+
+namespace mmfm {
+bool det_need_glue(int kind, long long d0, long long d1, long long d2, DetNeed* need) {
+  if (kind == MMFM_DET_EMBED_ASM_BWD) {   // (B, T, H)
+    int bchunk = 0;
+    const long long ctas = (long long)embed_bwd_chunks((int)d0, (int)d1, &bchunk) * d1;
+    *need = DetNeed{ctas * d2 * 4, (int)ctas};
+  } else if (kind == MMFM_DET_SMALLC_EMBED_BWD) {   // (B*T, C, H): the larger of the two kernels' needs
+    const int C = (int)d1, H = (int)d2;
+    int rows = 0;
+    long long ctas = smallc_generic_ctas(d0, &rows);
+    if (smallc_fast16(C, H)) {
+      const long long f = smallc_fast16_grid(d0, H);
+      if (f > ctas) ctas = f;
+    }
+    *need = DetNeed{ctas * (H * (1 + 2 * C) + 2 * C * (1 + C)) * 4, (int)ctas};
+  } else if (kind == MMFM_DET_SMALLC_HEAD_BWD) {   // (R, H, C)
+    const long long ctas = (long long)head_bwd_gx((int)d0) * ((d1 + 255) / 256);
+    *need = DetNeed{ctas * kHeadSlot * 4, (int)ctas};
+  } else if (kind == MMFM_DET_COLUMN_STATS) {   // (R, C)
+    int rows = 0;
+    const long long ctas = column_stats_ctas(d0, &rows);
+    *need = DetNeed{ctas * 4 * d1 * 8, (int)ctas};
+  } else {
+    return false;
+  }
+  return true;
+}
+}  // namespace mmfm
+
+#define DET_WS_CHECK(kind, d0, d1, d2, who)                                                       \
+  do {                                                                                          \
+    MMFM_REQUIRE(ws != nullptr, "%s: null workspace", who);                                     \
+    DetNeed need{0, 0};                                                                         \
+    det_need_glue(kind, d0, d1, d2, &need);                                                     \
+    if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, need, who)) return rc; \
+  } while (0)
+
+extern "C" int mmfm_embed_assemble_bwd_det(const float* g, const float* g2, const long long* ts, float* dpos, float* dmod,
+                                           int B, int T, int S, int off, int H, int n_pos, const mmfm_det_ws* ws,
+                                           void* stream) {
+  MMFM_REQUIRE(g && dmod && (dpos == nullptr || (ts && n_pos > 0)), "mmfm_embed_assemble_bwd_det: null pointer");
+  MMFM_REQUIRE(B > 0 && T > 0 && H % 4 == 0 && H <= 1024 && off >= 0 && off + T <= S,
+               "mmfm_embed_assemble_bwd_det: bad shape (H %% 4 == 0, H <= 1024)");
+  MMFM_REQUIRE(((uintptr_t)g | (uintptr_t)dmod | (uintptr_t)g2 | (uintptr_t)dpos) % 16 == 0,
+               "mmfm_embed_assemble_bwd_det: buffers must be 16-byte aligned");
+  DET_WS_CHECK(MMFM_DET_EMBED_ASM_BWD, B, T, H, "mmfm_embed_assemble_bwd_det");
+  cudaStream_t st = (cudaStream_t)stream;
+  int bchunk = 0;
+  const int chunks = embed_bwd_chunks(B, T, &bchunk);
+  const int threads = H / 4 * kAsmLanes;
+  embed_assemble_bwd_kernel<true><<<dim3(T, chunks), threads, (size_t)threads * sizeof(float4), st>>>(
+      g, g2, ts, nullptr, dmod, B, T, S, off, H, bchunk, (float4*)ws->buf, ws->tickets);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  if (dpos) {
+    embed_pos_bwd_det_kernel<<<n_pos, 256, 0, st>>>(g, g2, ts, dpos, B, T, S, off, H);
+    MMFM_CHECK_CUDA(cudaGetLastError());
+  }
+  return 0;
+}
+
+extern "C" int mmfm_smallc_embed_bwd_det(const float* in, const float* hid, const float* W2, const float* dx,
+                                         const unsigned char* row_zero, const mmfm_dropout* drop, float act_scale, int act,
+                                         float* dW1, float* db1, float* dW2, float* db2, int B, int T, int S, int off,
+                                         int C, int H, const mmfm_det_ws* ws, void* stream) {
+  MMFM_REQUIRE(in && hid && W2 && dx && dW1 && db1 && dW2 && db2, "mmfm_smallc_embed_bwd_det: null pointer");
+  MMFM_REQUIRE(C >= 1 && C <= kMaxC, "mmfm_smallc_embed_bwd_det: C=%d outside [1,%d]", C, kMaxC);
+  MMFM_REQUIRE(H % 32 == 0 && H <= 1024, "mmfm_smallc_embed_bwd_det: H=%d must be a multiple of 32 and <= 1024", H);
+  MMFM_REQUIRE(B > 0 && T > 0 && off >= 0 && off + T <= S, "mmfm_smallc_embed_bwd_det: bad shape");
+  const long long R = (long long)B * T;
+  DET_WS_CHECK(MMFM_DET_SMALLC_EMBED_BWD, R, C, H, "mmfm_smallc_embed_bwd_det");
+  cudaStream_t st = (cudaStream_t)stream;
+  float* buf = (float*)ws->buf;
+  if (smallc_fast16(C, H) && ((uintptr_t)dx & 15) == 0) {
+    const int grid = smallc_fast16_grid(R, H);
+    if (C == 1) smallc_embed_bwd16_kernel<1, true><<<grid, 256, 0, st>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act, dW1, db1, dW2, db2, B, T, S, off, H, buf, ws->tickets);
+    else smallc_embed_bwd16_kernel<2, true><<<grid, 256, 0, st>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act, dW1, db1, dW2, db2, B, T, S, off, H, buf, ws->tickets);
+    MMFM_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
+  int rows_per_cta = 0;
+  const int ctas = smallc_generic_ctas(R, &rows_per_cta);
+  smallc_embed_bwd_kernel<true><<<ctas, H, 0, st>>>(in, hid, W2, dx, row_zero, to_drop(drop), act_scale, act, dW1, db1,
+                                                    dW2, db2, B, T, S, off, C, H, rows_per_cta, buf, ws->tickets);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_smallc_head_bwd_det(const void* y, const float* W, const void* dpreds, long long lddp, void* dy,
+                                        float* dW, float* db, int R, int H, int C, const mmfm_det_ws* ws, void* stream) {
+  MMFM_REQUIRE(y && W && dpreds && dy && dW && db, "mmfm_smallc_head_bwd_det: null pointer");
+  MMFM_REQUIRE(C >= 1 && C <= kMaxC && R > 0 && H % 8 == 0, "mmfm_smallc_head_bwd_det: bad shape R=%d H=%d C=%d", R, H, C);
+  DET_WS_CHECK(MMFM_DET_SMALLC_HEAD_BWD, R, H, C, "mmfm_smallc_head_bwd_det");
+  smallc_head_bwd_kernel<true><<<dim3(head_bwd_gx(R), (H + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      (const bf16*)y, W, (const bf16*)dpreds, lddp, (bf16*)dy, dW, db, R, H, C, (float*)ws->buf, ws->tickets);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_column_stats_det(const float* pred, const float* y, long long R, int C, int log_rate, double* out,
+                                     const mmfm_det_ws* ws, void* stream) {
+  MMFM_REQUIRE(pred && y && out && R > 0 && C > 0, "mmfm_column_stats_det: bad arguments");
+  DET_WS_CHECK(MMFM_DET_COLUMN_STATS, R, C, 0, "mmfm_column_stats_det");
+  cudaStream_t st = (cudaStream_t)stream;
+  MMFM_CHECK_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * 4 * (size_t)C, st));
+  int rows_per_cta = 0;
+  const int ctas = column_stats_ctas(R, &rows_per_cta);
+  column_stats_kernel<true><<<ctas, 256, 0, st>>>(pred, y, R, C, log_rate, rows_per_cta, out, (double*)ws->buf,
+                                                  ws->tickets);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

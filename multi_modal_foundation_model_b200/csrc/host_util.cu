@@ -163,6 +163,17 @@ int device_sm_count() {
   return n;
 }
 
+int det_ws_check(const void* buf, long long bytes, const unsigned int* tickets, int n_tickets, const DetNeed& need,
+                 const char* who) {
+  MMFM_REQUIRE(bytes >= need.bytes && n_tickets >= need.tickets,
+               "%s: deterministic workspace too small (%lld bytes / %d tickets given, %lld / %d needed)", who, bytes,
+               n_tickets, need.bytes, need.tickets);
+  MMFM_REQUIRE(need.bytes == 0 || (buf != nullptr && (reinterpret_cast<uintptr_t>(buf) & 15) == 0),
+               "%s: deterministic workspace buffer missing or not 16-byte aligned", who);
+  MMFM_REQUIRE(need.tickets == 0 || tickets != nullptr, "%s: deterministic workspace has no tickets", who);
+  return 0;
+}
+
 }  // namespace mmfm
 
 extern "C" const char* mmfm_last_error(void) { return mmfm::get_error(); }
@@ -172,4 +183,18 @@ extern "C" int mmfm_sm_count(void) {
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
   if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
   return n;
+}
+
+extern "C" int mmfm_det_ws_bytes(int kind, long long d0, long long d1, long long d2, long long* bytes, int* n_tickets) {
+  MMFM_REQUIRE(bytes && n_tickets, "mmfm_det_ws_bytes: null output");
+  MMFM_REQUIRE(d0 > 0 && d1 > 0 && d2 >= 0, "mmfm_det_ws_bytes: bad sizes (%lld, %lld, %lld)", d0, d1, d2);
+  mmfm::DetNeed need{0, 0};
+  if (!mmfm::det_need_gemm(kind, d0, d1, d2, &need) && !mmfm::det_need_norm(kind, d0, d1, d2, &need) &&
+      !mmfm::det_need_glue(kind, d0, d1, d2, &need)) {
+    mmfm::set_error("mmfm_det_ws_bytes: unknown kind %d", kind);
+    return -1;
+  }
+  *bytes = need.bytes;
+  *n_tickets = need.tickets;
+  return 0;
 }

@@ -47,6 +47,19 @@ int make_tmap_bf16_3d(CUtensorMap* out, const void* base, uint64_t batch, uint64
 
 int device_sm_count();
 
+// Deterministic-mode workspace need of one *_det call (mmfm_det_ws_bytes): each source file answers for its own
+// kinds (false = not its kind) from the grid arithmetic its launchers use.
+struct DetNeed {
+  long long bytes;
+  int tickets;
+};
+bool det_need_gemm(int kind, long long d0, long long d1, long long d2, DetNeed* need);
+bool det_need_norm(int kind, long long d0, long long d1, long long d2, DetNeed* need);
+bool det_need_glue(int kind, long long d0, long long d1, long long d2, DetNeed* need);
+// 0 when the workspace can hold `need`; sets the error and returns -1 otherwise
+int det_ws_check(const void* buf, long long bytes, const unsigned int* tickets, int n_tickets, const DetNeed& need,
+                 const char* who);
+
 // MMFM_PDL=1 (default 0: measured neutral): launch the hot kernels with programmatic stream serialization (see
 // common.cuh: pdl_enter)
 bool pdl_enabled();

@@ -153,12 +153,13 @@ __global__ void __launch_bounds__(kLnWarps * 32) layernorm_fwd_kernel(const floa
 }
 
 // dx = dres + rstd * (g*dy - mean(g*dy) - xhat * mean(g*dy*xhat));  dgamma += sum dy*xhat; dbeta += sum dy
-template <int NV>
+// DET: the CTA's column sums go to its workspace slot [dgamma H | dbeta H] and det_tree_fold adds them up
+template <int NV, bool DET = false>
 __global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_kernel(
     const bf16* __restrict__ dy, const float* __restrict__ x, const float* __restrict__ mean,
     const float* __restrict__ rstd, const float* __restrict__ gamma, const float* dres, float* dx,
     bf16* __restrict__ dxb, DropCfg drop, float* __restrict__ dgamma, float* __restrict__ dbeta, int R, int H,
-    int modmajor_T, int S) {
+    int modmajor_T, int S, float* __restrict__ ws, unsigned int* tickets) {
   static_assert(NV > 0, "register path only");
   pdl_enter();
   __shared__ float red[kLnWarps][NV * 128 + 4];
@@ -243,9 +244,16 @@ __global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_kernel(
         float s = 0.f;
 #pragma unroll
         for (int w = 0; w < kLnWarps; ++w) s += red[w][c];
-        atomicAdd(out + c, s);
+        if constexpr (DET) ws[(long long)blockIdx.x * 2 * H + pass * H + c] = s;
+        else atomicAdd(out + c, s);
       }
     }
+  }
+  if constexpr (DET) {
+    det_tree_fold(ws, 2 * H, 2 * H, blockIdx.x, gridDim.x, tickets, [&](int i, float v) {
+      float* out = i < H ? dgamma : dbeta;
+      if (out) out[i < H ? i : i - H] += v;
+    });
   }
 }
 
@@ -311,8 +319,10 @@ __global__ void __launch_bounds__(kLnWarps * 32) layernorm_fwd_multi_kernel(cons
   }
 }
 
-template <int NV, int NL>
-__global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_multi_kernel(const mmfm_ln_multi_args a) {
+template <int NV, int NL, bool DET = false>
+__global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_multi_kernel(const mmfm_ln_multi_args a,
+                                                                            float* __restrict__ ws,
+                                                                            unsigned int* tickets) {
   pdl_enter();
   __shared__ float red[kLnWarps][128 * NV + 4];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -412,9 +422,17 @@ __global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_multi_kernel(cons
         float s = 0.f;
 #pragma unroll
         for (int w = 0; w < kLnWarps; ++w) s += red[w][c];
-        atomicAdd(out + c, s);
+        if constexpr (DET) ws[(long long)blockIdx.x * 2 * NL * H + pass * H + c] = s;
+        else atomicAdd(out + c, s);
       }
     }
+  }
+  if constexpr (DET) {   // slot = [dgamma_0 | dbeta_0 | dgamma_1 | ...], H each
+    det_tree_fold(ws, 2 * NL * H, 2 * NL * H, blockIdx.x, gridDim.x, tickets, [&](int i, float v) {
+      const int pass = i / H;
+      float* out = (pass & 1) ? a.dbeta[pass >> 1] : a.dgamma[pass >> 1];
+      if (out) out[i - pass * H] += v;
+    });
   }
 }
 
@@ -452,12 +470,14 @@ __global__ void __launch_bounds__(kLnWarps * 32) scalenorm_fwd_kernel(const floa
 
 // dx = dres + g * rn * (dy - xhat * <dy, xhat>), xhat = x * rn  (the projection term vanishes where the norm was clamped
 // to eps: there the scale g / eps is a constant);  dg += sum_rows <dy, xhat>
+template <bool DET = false>
 __global__ void __launch_bounds__(kLnWarps * 32) scalenorm_bwd_kernel(const bf16* __restrict__ dy,
                                                                        const float* __restrict__ x,
                                                                        const float* __restrict__ rnorm,
                                                                        const float* __restrict__ g, const float* dres,
                                                                        float* dx, bf16* __restrict__ dxb, DropCfg drop,
-                                                                       float* __restrict__ dg, int R, int H, float eps) {
+                                                                       float* __restrict__ dg, int R, int H, float eps,
+                                                                       float* __restrict__ ws, unsigned int* tickets) {
   __shared__ float red[kLnWarps];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const float gs = __ldg(g);
@@ -511,11 +531,17 @@ __global__ void __launch_bounds__(kLnWarps * 32) scalenorm_bwd_kernel(const bf16
   }
   if (lane == 0) red[warp] = acc_g;
   __syncthreads();
-  if (threadIdx.x == 0 && dg) {
+  if (threadIdx.x == 0 && (DET || dg)) {
     float t = 0.f;
 #pragma unroll
     for (int w = 0; w < kLnWarps; ++w) t += red[w];
-    atomicAdd(dg, t);
+    if constexpr (DET) ws[blockIdx.x] = t;
+    else atomicAdd(dg, t);
+  }
+  if constexpr (DET) {
+    det_tree_fold(ws, 1, 1, blockIdx.x, gridDim.x, tickets, [&](int, float v) {
+      if (dg) *dg += v;
+    });
   }
 }
 
@@ -590,7 +616,7 @@ extern "C" int mmfm_layernorm_bwd(const void* dy, const float* x, const float* m
     if (cap == 0) cap = resident_ctas(layernorm_bwd_kernel<NV>, kLnWarps * 32);                                   \
     const int grid = want < cap ? (want < 1 ? 1 : want) : cap;                                                    \
     MMFM_CHECK_CUDA(launch_pdl(layernorm_bwd_kernel<NV>, dim3(grid), dim3(kLnWarps * 32), 0, st, (const bf16*)dy, x, mean,  \
-                               rstd, gamma, dres, dx, (bf16*)dxb, dc, dgamma, dbeta, R, H, modmajor_T, S));             \
+                               rstd, gamma, dres, dx, (bf16*)dxb, dc, dgamma, dbeta, R, H, modmajor_T, S, nullptr, nullptr)); \
   } while (0)
   switch (H) {
     case 128: LN_BWD(1); break;
@@ -634,13 +660,21 @@ extern "C" int mmfm_layernorm_fwd_multi(const mmfm_ln_multi_args* a, void* strea
   return 0;
 }
 
-template <int NV>
-static int ln_bwd_multi_launch(const mmfm_ln_multi_args* a, cudaStream_t st) {
-  // one resident wave: the register-heavy kernel (2 * n * NV float4 accumulators) fits one or two CTAs per SM
-  int grid = device_sm_count() * (NV * a->n <= 4 ? 2 : 1);
-  const int max_grid = (a->R + kLnWarps - 1) / kLnWarps;
-  if (grid > max_grid) grid = max_grid;
-#define LNB(NL) MMFM_CHECK_CUDA(launch_pdl(layernorm_bwd_multi_kernel<NV, NL>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a))
+// one resident wave: the register-heavy kernel (2 * n * NV float4 accumulators) fits one or two CTAs per SM
+static int ln_bwd_multi_grid(int R, int H, int n) {
+  const int grid = device_sm_count() * ((H / 128) * n <= 4 ? 2 : 1);
+  const int max_grid = (R + kLnWarps - 1) / kLnWarps;
+  return grid > max_grid ? max_grid : grid;
+}
+
+template <int NV, bool DET>
+static int ln_bwd_multi_launch(const mmfm_ln_multi_args* a, cudaStream_t st, float* ws_buf, unsigned int* tickets) {
+  const int grid = ln_bwd_multi_grid(a->R, a->H, a->n);
+#define LNB(NL)                                                                                                  \
+  MMFM_CHECK_CUDA(DET ? launch_pdl(layernorm_bwd_multi_kernel<NV, NL, true>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a, \
+                                   ws_buf, tickets)                                                               \
+                      : launch_pdl(layernorm_bwd_multi_kernel<NV, NL>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a,   \
+                                   (float*)nullptr, (unsigned int*)nullptr))
   switch (a->n) {
     case 1: LNB(1); break;
     case 2: LNB(2); break;
@@ -660,9 +694,92 @@ extern "C" int mmfm_layernorm_bwd_multi(const mmfm_ln_multi_args* a, void* strea
   if (int rc = ln_multi_check(a, "mmfm_layernorm_bwd_multi", true)) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   switch (a->H) {
-    case 128: return ln_bwd_multi_launch<1>(a, st);
-    case 256: return ln_bwd_multi_launch<2>(a, st);
-    default: return ln_bwd_multi_launch<4>(a, st);
+    case 128: return ln_bwd_multi_launch<1, false>(a, st, nullptr, nullptr);
+    case 256: return ln_bwd_multi_launch<2, false>(a, st, nullptr, nullptr);
+    default: return ln_bwd_multi_launch<4, false>(a, st, nullptr, nullptr);
+  }
+}
+
+// ---- deterministic twins (column sums folded by det_tree_fold; one workspace slot per CTA) ----
+static int ln_bwd_det_grid(int R) {
+  const int want = (R + kLnWarps * 4 - 1) / (kLnWarps * 4);
+  const int cap = 2 * device_sm_count();
+  return want < 1 ? 1 : (want < cap ? want : cap);
+}
+static int scalenorm_bwd_grid(int R, int cap) {
+  int grid = (R + kLnWarps * 4 - 1) / (kLnWarps * 4);
+  if (grid > cap) grid = cap;
+  return grid < 1 ? 1 : grid;
+}
+
+namespace mmfm {
+bool det_need_norm(int kind, long long d0, long long d1, long long d2, DetNeed* need) {
+  const int R = (int)d0, H = (int)d1;
+  if (kind == MMFM_DET_LN_BWD) {
+    const int g = ln_bwd_det_grid(R);
+    *need = DetNeed{(long long)g * 2 * H * 4, g};
+  } else if (kind == MMFM_DET_LN_BWD_MULTI) {
+    const int g = ln_bwd_multi_grid(R, H, (int)d2);
+    *need = DetNeed{(long long)g * 2 * d2 * H * 4, g};
+  } else if (kind == MMFM_DET_SCALENORM_BWD) {
+    const int g = scalenorm_bwd_grid(R, 2 * device_sm_count());
+    *need = DetNeed{(long long)g * 4, g};
+  } else {
+    return false;
+  }
+  return true;
+}
+}  // namespace mmfm
+
+extern "C" int mmfm_layernorm_bwd_det(const void* dy, const float* x, const float* mean, const float* rstd,
+                                      const float* gamma, const float* dres, float* dx, void* dxb,
+                                      const mmfm_dropout* drop, float* dgamma, float* dbeta, int R, int H,
+                                      int modmajor_T, int S, const mmfm_det_ws* ws, void* stream) {
+  MMFM_REQUIRE(dy && x && mean && rstd && gamma && ws, "mmfm_layernorm_bwd_det: null pointer");
+  MMFM_REQUIRE(dx || dxb, "mmfm_layernorm_bwd_det: no output requested");
+  MMFM_REQUIRE(R > 0 && (H == 128 || H == 256 || H == 512 || H == 1024),
+               "mmfm_layernorm_bwd_det: hidden size %d not supported (128/256/512/1024)", H);
+  MMFM_REQUIRE(modmajor_T <= 0 || (S > 0 && S % modmajor_T == 0 && R % S == 0),
+               "mmfm_layernorm_bwd_det: modality-major remap needs S %% T == 0 and R %% S == 0");
+  DetNeed need{0, 0};
+  det_need_norm(MMFM_DET_LN_BWD, R, H, 0, &need);
+  if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, need, "mmfm_layernorm_bwd_det")) return rc;
+  DropCfg dc{nullptr, 0u, 0u, 1.0f};
+  if (drop && drop->thresh != 0u) {
+    MMFM_REQUIRE(drop->seed != nullptr && drop->thresh < 256u, "mmfm_layernorm_bwd_det: bad dropout config");
+    dc = DropCfg{drop->seed, drop->site, drop->thresh, drop->scale};
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int grid = ln_bwd_det_grid(R);
+  if (dxb) set_l2_window(dxb, (size_t)R * H * 2);
+#define LN_BWD_DET(NV)                                                                                            \
+  MMFM_CHECK_CUDA(launch_pdl(layernorm_bwd_kernel<NV, true>, dim3(grid), dim3(kLnWarps * 32), 0, st, (const bf16*)dy, x, \
+                             mean, rstd, gamma, dres, dx, (bf16*)dxb, dc, dgamma, dbeta, R, H, modmajor_T, S,      \
+                             (float*)ws->buf, ws->tickets))
+  switch (H) {
+    case 128: LN_BWD_DET(1); break;
+    case 256: LN_BWD_DET(2); break;
+    case 512: LN_BWD_DET(4); break;
+    default: LN_BWD_DET(8); break;
+  }
+#undef LN_BWD_DET
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_layernorm_bwd_multi_det(const mmfm_ln_multi_args* a, const mmfm_det_ws* ws, void* stream) {
+  if (int rc = ln_multi_check(a, "mmfm_layernorm_bwd_multi_det", true)) return rc;
+  MMFM_REQUIRE(ws != nullptr, "mmfm_layernorm_bwd_multi_det: null workspace");
+  DetNeed need{0, 0};
+  det_need_norm(MMFM_DET_LN_BWD_MULTI, a->R, a->H, a->n, &need);
+  if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, need, "mmfm_layernorm_bwd_multi_det"))
+    return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  float* buf = (float*)ws->buf;
+  switch (a->H) {
+    case 128: return ln_bwd_multi_launch<1, true>(a, st, buf, ws->tickets);
+    case 256: return ln_bwd_multi_launch<2, true>(a, st, buf, ws->tickets);
+    default: return ln_bwd_multi_launch<4, true>(a, st, buf, ws->tickets);
   }
 }
 
@@ -687,12 +804,31 @@ extern "C" int mmfm_scalenorm_bwd(const void* dy, const float* x, const float* r
     dc = DropCfg{drop->seed, drop->site, drop->thresh, drop->scale};
   }
   static int cap = 0;
-  if (cap == 0) cap = resident_ctas(scalenorm_bwd_kernel, kLnWarps * 32);
-  int grid = (R + kLnWarps * 4 - 1) / (kLnWarps * 4);
-  if (grid > cap) grid = cap;
-  if (grid < 1) grid = 1;
+  if (cap == 0) cap = resident_ctas(scalenorm_bwd_kernel<false>, kLnWarps * 32);
+  const int grid = scalenorm_bwd_grid(R, cap);
   scalenorm_bwd_kernel<<<grid, kLnWarps * 32, 0, (cudaStream_t)stream>>>((const bf16*)dy, x, rnorm, g, dres, dx, (bf16*)dxb,
-                                                                        dc, dg, R, H, eps);
+                                                                        dc, dg, R, H, eps, nullptr, nullptr);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_scalenorm_bwd_det(const void* dy, const float* x, const float* rnorm, const float* g,
+                                      const float* dres, float* dx, void* dxb, const mmfm_dropout* drop, float* dg,
+                                      int R, int H, float eps, const mmfm_det_ws* ws, void* stream) {
+  MMFM_REQUIRE(dy && x && rnorm && g && ws, "mmfm_scalenorm_bwd_det: null pointer");
+  MMFM_REQUIRE(dx || dxb, "mmfm_scalenorm_bwd_det: no output requested");
+  MMFM_REQUIRE(R > 0 && H > 0 && H % 4 == 0, "mmfm_scalenorm_bwd_det: bad shape R=%d H=%d", R, H);
+  DetNeed need{0, 0};
+  det_need_norm(MMFM_DET_SCALENORM_BWD, R, H, 0, &need);
+  if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, need, "mmfm_scalenorm_bwd_det")) return rc;
+  DropCfg dc{nullptr, 0u, 0u, 1.0f};
+  if (drop && drop->thresh != 0u) {
+    MMFM_REQUIRE(drop->seed != nullptr && drop->thresh < 256u, "mmfm_scalenorm_bwd_det: bad dropout config");
+    dc = DropCfg{drop->seed, drop->site, drop->thresh, drop->scale};
+  }
+  const int grid = scalenorm_bwd_grid(R, 2 * device_sm_count());
+  scalenorm_bwd_kernel<true><<<grid, kLnWarps * 32, 0, (cudaStream_t)stream>>>(
+      (const bf16*)dy, x, rnorm, g, dres, dx, (bf16*)dxb, dc, dg, R, H, eps, (float*)ws->buf, ws->tickets);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

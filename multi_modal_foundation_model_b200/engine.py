@@ -306,6 +306,9 @@ class Plan:
         self.S, self.R, self.BT = S, R, BT
 
         self._keep: List[Any] = []
+        # deterministic mode (torch.use_deterministic_algorithms): the cross-CTA reductions of the backward go through
+        # the *_det kernels on this one workspace, sized after recording to the largest call (one stream: shared)
+        self.det_ws = ops.DetWorkspace() if ops.deterministic() else None
 
         def raw(shape, dtype, esize):
             n = int(np.prod(shape)) * esize
@@ -369,6 +372,8 @@ class Plan:
         self._n_fwd_runs = self._n_bwd_runs = 0
         self.fwd_calls, self.bwd_calls = rec_f.calls, rec_b.calls
         self._keep += rec_f.keep + rec_b.keep
+        if self.det_ws is not None:
+            self.det_ws.materialize(dev)
         self.n_fwd, self.n_bwd = len(self.fwd_calls), len(self.bwd_calls)
 
     # ---------------------------------------------------------------------------------------------------
@@ -394,11 +399,11 @@ class Plan:
         mean, rstd = self.stats[name]
         if st.has(name + ".scale"):
             ops.scalenorm_bwd(dy, x, rstd, st.p(name + ".scale"), dres, dx, dxb, drop, st.g(name + ".scale"), R=self.R,
-                              H=self.eng.H)
+                              H=self.eng.H, ws=self.det_ws)
             return
         ops.layernorm_bwd(dy, x, mean, rstd, st.p(name + ".weight"), dres, dx, dxb, drop, st.g(name + ".weight"),
                           st.g(name + ".bias"), R=self.R, H=self.eng.H, modmajor_T=self.eng.T if modmajor else 0,
-                          S=self.S if modmajor else 0)
+                          S=self.S if modmajor else 0, ws=self.det_ws)
 
     def _bias(self, names: List[str], buf: str = "p") -> Optional[torch.Tensor]:
         """fp32 bias (possibly the concatenation of adjacent biases in the flat buffer)."""
@@ -620,7 +625,7 @@ class Plan:
                 ops.gemm_tn(dY, sh.tr[shadow_key], dX, act=act, aux=aux, act_scale=act_scale, **extra)
             bn = bnames or [wname + ".bias"]
             ops.gemm_wgrad(dY, X, self._wgrad_dst(wnames or [wname + ".weight"]),
-                           dbias=self._bias(bn, "g") if st.has(bn[0]) else None)
+                           dbias=self._bias(bn, "g") if st.has(bn[0]) else None, ws=self.det_ws)
 
         def mlp_bwd(pre, x_in, ln_name, Gs, inter, dxb, drop_prev):
             duv = du[:, :inter]
@@ -659,7 +664,7 @@ class Plan:
             dym = ddec[k * BT:(k + 1) * BT]
             if m.small:
                 ops.smallc_head_bwd(ym, st.p(pre + ".weight"), self.dpreds[m.name], dym, st.g(pre + ".weight"),
-                                    st.g(pre + ".bias"), R=BT, H=H, Cc=m.C)
+                                    st.g(pre + ".bias"), R=BT, H=H, Cc=m.C, ws=self.det_ws)
             else:
                 lin_bwd(self.dpreds[m.name], ym, pre, pre, dym)
         last_dec_drop = self._drop(SITE_MLP, eng.Ld - 1, SIDE_DEC, hp["dec_dropout"])
@@ -701,7 +706,8 @@ class Plan:
             names = [f"decoder.{i}.context_norm" for i in reversed(range(eng.Ld))]      # the order of dctx
             cmean, crstd = self.stats[names[0]]
             ops.layernorm_bwd_multi(dctx, self.ctx, cmean, crstd, [st.p(n + ".weight") for n in names], Gctx, Gcb,
-                                    [st.g(n + ".weight") for n in names], [st.g(n + ".bias") for n in names], R=R, H=H)
+                                    [st.g(n + ".weight") for n in names], [st.g(n + ".bias") for n in names], R=R, H=H,
+                                    ws=self.det_ws)
         mark("decoder_proj_context.weight")
 
         # ---- context projection + encoder ------------------------------------------------------------------
@@ -726,7 +732,7 @@ class Plan:
                 off = k * T
                 dpos = st.g(pre + ".pos_embed.weight") if st.has(pre + ".pos_embed.weight") else None
                 ops.embed_assemble_bwd(Gs, G2, self.ts[m.name], dpos, st.g(pre + ".mod_emb.weight")[m.index], B=B, T=T,
-                                       S=S, off=off, H=H)
+                                       S=S, off=off, H=H, ws=self.det_ws)
                 drop = self._drop(SITE_EMBED, m.index, side, p_emb)
                 if m.small:
                     has_b1 = st.has(pre + ".token_embed.bias")
@@ -734,7 +740,8 @@ class Plan:
                     ops.smallc_embed_bwd(self.inp[m.name], A[pre + ".hid"], st.p(pre + ".projection.weight"), Gs,
                                          self.zero, drop, eng.embed_scale, eng.embed_act,
                                          st.g(pre + ".token_embed.weight"), db1, st.g(pre + ".projection.weight"),
-                                         st.g(pre + ".projection.bias"), B=B, T=T, S=S, off=off, Cc=m.C, H=H)
+                                         st.g(pre + ".projection.bias"), B=B, T=T, S=S, off=off, Cc=m.C, H=H,
+                                         ws=self.det_ws)
                 else:
                     ops.embed_grad_prep(Gs, dtok, self.zero, drop, B=B, T=T, S=S, off=off, H=H)
                     dhid = b16(BT, 2 * m.C)
@@ -860,7 +867,7 @@ class Engine:
         self.seed = torch.tensor([key], dtype=torch.int64, device=self.device)
         self.store = ParamStore(model, self.device)
         self.shadows = Shadows(self.store, model, self.sessions)
-        self.plans: Dict[Tuple[int, bool, Any, Tuple[str, ...]], Plan] = {}
+        self.plans: Dict[Tuple[int, bool, Any, Tuple[str, ...], bool], Plan] = {}
         self.arenas: Dict[Tuple[int, bool], Arena] = {}
         self.ddp = None          # set by parallel.DataParallel
         import os as _os
@@ -884,7 +891,8 @@ class Engine:
             self.plans.clear()
             self.arenas.clear()
             self.T = T
-        key = (B, training, session, u8_mods)
+        # deterministic mode selects other kernels: its own plan (and graphs), never a change to a captured one
+        key = (B, training, session, u8_mods, ops.deterministic())
         pl = self.plans.get(key)
         if pl is None:
             arena = None

@@ -76,6 +76,54 @@ def _launch(name: str, *args, keep=(), meta=None):
     check(fn(*args, _stream()), name)
 
 
+# ------------------------------------------------------------------------------------------------------------
+# deterministic mode: on exactly when torch.are_deterministic_algorithms_enabled()
+# ------------------------------------------------------------------------------------------------------------
+def deterministic() -> bool:
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def det_ws_need(kind: int, d0: int, d1: int = 1, d2: int = 0) -> Tuple[int, int]:
+    """(bytes, tickets) of the workspace one *_det call of `kind` needs at these sizes (host only)."""
+    nb, nt = C.c_longlong(0), C.c_int(0)
+    check(lib().mmfm_det_ws_bytes(kind, int(d0), int(d1), int(d2), C.byref(nb), C.byref(nt)), "mmfm_det_ws_bytes")
+    return nb.value, nt.value
+
+
+class DetWorkspace:
+    """Workspace of the *_det entry points: a byte buffer and zeroed tickets, shared by calls on one stream.  The C
+    struct is passed by reference, so a recorded schedule can be sized after recording (``materialize``)."""
+
+    def __init__(self):
+        self.c = _lib.DetWs(None, 0, None, 0)
+        self.want_bytes, self.want_tickets = 0, 0
+        self.buf: Optional[torch.Tensor] = None
+        self.tickets: Optional[torch.Tensor] = None
+
+    def require(self, nbytes: int, n_tickets: int) -> None:
+        self.want_bytes = max(self.want_bytes, int(nbytes))
+        self.want_tickets = max(self.want_tickets, int(n_tickets))
+
+    def materialize(self, device) -> None:
+        """(Re)allocate when the recorded needs outgrow the buffers; the tickets start at zero."""
+        if self.buf is None or self.buf.numel() < self.want_bytes:
+            self.buf = torch.empty(max(16, self.want_bytes), dtype=torch.uint8, device=device)
+        if self.tickets is None or self.tickets.numel() < self.want_tickets:
+            self.tickets = torch.zeros(max(1, self.want_tickets), dtype=torch.int32, device=device)
+        self.c.buf, self.c.bytes = self.buf.data_ptr(), self.buf.numel()
+        self.c.tickets, self.c.n_tickets = self.tickets.data_ptr(), self.tickets.numel()
+
+
+def _launch_det(name: str, ws: Optional[DetWorkspace], need: Tuple[int, int], device, *args, keep=(), meta=None):
+    """Launch the *_det twin of `name` on `ws` (a private workspace when None)."""
+    if ws is None:
+        ws = DetWorkspace()
+    ws.require(*need)
+    if _REC is None:
+        ws.materialize(device)
+    _launch(name + "_det", *args, C.byref(ws.c), keep=(*keep, ws), meta=meta)
+
+
 def run_recorded(calls) -> None:
     st = _stream()
     for c in calls:
@@ -147,20 +195,30 @@ def gemm_tn(A: torch.Tensor, B: torch.Tensor, D: torch.Tensor, *, M: Optional[in
 
 def gemm_wgrad(dY: torch.Tensor, X: torch.Tensor, dW: torch.Tensor, *, R: Optional[int] = None,
                NO: Optional[int] = None, KI: Optional[int] = None, ldw: Optional[int] = None,
-               dbias: Optional[torch.Tensor] = None) -> None:
+               dbias: Optional[torch.Tensor] = None, ws: Optional[DetWorkspace] = None) -> None:
     """dW[NO,KI] += dY[R,NO]^T . X[R,KI] ; dbias[NO] += colsum(dY) (optional)"""
     assert dY.dtype == bf16 and X.dtype == bf16 and dW.dtype == torch.float32
     R = R if R is not None else dY.shape[0]
     NO = NO if NO is not None else dY.shape[1]
     KI = KI if KI is not None else X.shape[1]
-    _launch("mmfm_gemm_wgrad", dY.data_ptr(), dY.stride(0), X.data_ptr(), X.stride(0), R, NO, KI, dW.data_ptr(),
-            ldw if ldw is not None else KI, _p(dbias),
-            meta={"flops": 2.0 * R * NO * KI, "bytes": 2.0 * R * (NO + KI) + 4.0 * NO * KI, "tag": f"wgrad {R}x{NO}x{KI}"})
+    args = (dY.data_ptr(), dY.stride(0), X.data_ptr(), X.stride(0), R, NO, KI, dW.data_ptr(),
+            ldw if ldw is not None else KI, _p(dbias))
+    meta = {"flops": 2.0 * R * NO * KI, "bytes": 2.0 * R * (NO + KI) + 4.0 * NO * KI, "tag": f"wgrad {R}x{NO}x{KI}"}
+    if deterministic():
+        _launch_det("mmfm_gemm_wgrad", ws, det_ws_need(_lib.DET_WGRAD, R, NO, KI), dW.device, *args, meta=meta)
+        return
+    _launch("mmfm_gemm_wgrad", *args, meta=meta)
 
 
-def colsum_bf16(dY: torch.Tensor, out: torch.Tensor, *, R: Optional[int] = None, NO: Optional[int] = None) -> None:
-    _launch("mmfm_colsum_bf16", dY.data_ptr(), dY.stride(0), R if R is not None else dY.shape[0],
-            NO if NO is not None else dY.shape[1], out.data_ptr())
+def colsum_bf16(dY: torch.Tensor, out: torch.Tensor, *, R: Optional[int] = None, NO: Optional[int] = None,
+                ws: Optional[DetWorkspace] = None) -> None:
+    R = R if R is not None else dY.shape[0]
+    NO = NO if NO is not None else dY.shape[1]
+    args = (dY.data_ptr(), dY.stride(0), R, NO, out.data_ptr())
+    if deterministic():
+        _launch_det("mmfm_colsum_bf16", ws, det_ws_need(_lib.DET_COLSUM, R, NO), out.device, *args)
+        return
+    _launch("mmfm_colsum_bf16", *args)
 
 
 def cast_bf16(x: torch.Tensor, y: Optional[torch.Tensor], yt: Optional[torch.Tensor] = None, *, R: Optional[int] = None,
@@ -195,10 +253,15 @@ def u8_expand(x: torch.Tensor, y32: Optional[torch.Tensor], y16: Optional[torch.
             y16.stride(0) if y16 is not None else 0, meta={"bytes": float(R) * Cc * (1 + (4 if y32 is not None else 0) + (2 if y16 is not None else 0))})
 
 
-def column_stats(pred: torch.Tensor, y: torch.Tensor, out: torch.Tensor, *, log_rate: bool) -> None:
+def column_stats(pred: torch.Tensor, y: torch.Tensor, out: torch.Tensor, *, log_rate: bool,
+                 ws: Optional[DetWorkspace] = None) -> None:
     R, Cc = pred.shape
-    _launch("mmfm_column_stats", pred.data_ptr(), y.data_ptr(), R, Cc, 1 if log_rate else 0, out.data_ptr(),
-            meta={"bytes": 8.0 * R * Cc})
+    args = (pred.data_ptr(), y.data_ptr(), R, Cc, 1 if log_rate else 0, out.data_ptr())
+    if deterministic():
+        _launch_det("mmfm_column_stats", ws, det_ws_need(_lib.DET_COLUMN_STATS, R, Cc), out.device, *args,
+                    meta={"bytes": 8.0 * R * Cc})
+        return
+    _launch("mmfm_column_stats", *args, meta={"bytes": 8.0 * R * Cc})
 
 
 def adamw_step(p: torch.Tensor, g: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor, *, lr: float,
@@ -215,12 +278,16 @@ def layernorm_fwd(x, gamma, beta, y, mean, rstd, *, R: int, H: int, eps: float =
 
 
 def layernorm_bwd(dy, x, mean, rstd, gamma, dres, dx, dxb, drop: DropSpec, dgamma, dbeta, *, R: int, H: int,
-                  modmajor_T: int = 0, S: int = 0) -> None:
+                  modmajor_T: int = 0, S: int = 0, ws: Optional[DetWorkspace] = None) -> None:
     d = drop.c()
-    _launch("mmfm_layernorm_bwd", dy.data_ptr(), x.data_ptr(), mean.data_ptr(), rstd.data_ptr(), gamma.data_ptr(),
-            _p(dres), _p(dx), _p(dxb), C.byref(d), _p(dgamma), _p(dbeta), R, H, modmajor_T, S, keep=(d,),
-            meta={"bytes": float(R) * H * (2 + 4 + (4 if dres is not None else 0) + (4 if dx is not None else 0)
-                                           + (2 if dxb is not None else 0))})
+    args = (dy.data_ptr(), x.data_ptr(), mean.data_ptr(), rstd.data_ptr(), gamma.data_ptr(), _p(dres), _p(dx), _p(dxb),
+            C.byref(d), _p(dgamma), _p(dbeta), R, H, modmajor_T, S)
+    meta = {"bytes": float(R) * H * (2 + 4 + (4 if dres is not None else 0) + (4 if dx is not None else 0)
+                                     + (2 if dxb is not None else 0))}
+    if deterministic():
+        _launch_det("mmfm_layernorm_bwd", ws, det_ws_need(_lib.DET_LN_BWD, R, H), x.device, *args, keep=(d,), meta=meta)
+        return
+    _launch("mmfm_layernorm_bwd", *args, keep=(d,), meta=meta)
 
 
 def layernorm_fwd_multi(x, gammas, betas, ys, mean, rstd, *, R: int, H: int, eps: float = 1e-5) -> None:
@@ -233,15 +300,20 @@ def layernorm_fwd_multi(x, gammas, betas, ys, mean, rstd, *, R: int, H: int, eps
     _launch("mmfm_layernorm_fwd_multi", C.byref(a), keep=(a,), meta={"bytes": float(R) * H * (4 + 2 * len(ys))})
 
 
-def layernorm_bwd_multi(dys, x, mean, rstd, gammas, dx, dxb, dgammas, dbetas, *, R: int, H: int) -> None:
+def layernorm_bwd_multi(dys, x, mean, rstd, gammas, dx, dxb, dgammas, dbetas, *, R: int, H: int,
+                        ws: Optional[DetWorkspace] = None) -> None:
     """dx = LN'(sum_l dy_l . gamma_l) (written, not accumulated) + optional bf16 copy; dgamma_l / dbeta_l accumulate."""
     a = _lib.LnMultiArgs()
     a.x, a.R, a.H, a.n, a.eps = x.data_ptr(), R, H, len(dys), 0.0
     for l, (dy, g, dg, db) in enumerate(zip(dys, gammas, dgammas, dbetas)):
         a.dy[l], a.gamma[l], a.dgamma[l], a.dbeta[l] = dy.data_ptr(), g.data_ptr(), _p(dg), _p(db)
     a.mean, a.rstd, a.dx, a.dxb = mean.data_ptr(), rstd.data_ptr(), dx.data_ptr(), _p(dxb)
-    _launch("mmfm_layernorm_bwd_multi", C.byref(a), keep=(a,),
-            meta={"bytes": float(R) * H * (4 + 2 * len(dys) + 4 + (2 if dxb is not None else 0))})
+    meta = {"bytes": float(R) * H * (4 + 2 * len(dys) + 4 + (2 if dxb is not None else 0))}
+    if deterministic():
+        _launch_det("mmfm_layernorm_bwd_multi", ws, det_ws_need(_lib.DET_LN_BWD_MULTI, R, H, len(dys)), x.device,
+                    C.byref(a), keep=(a,), meta=meta)
+        return
+    _launch("mmfm_layernorm_bwd_multi", C.byref(a), keep=(a,), meta=meta)
 
 
 def scalenorm_fwd(x, g, y, rnorm, *, R: int, H: int, eps: float = 1e-5) -> None:
@@ -249,12 +321,18 @@ def scalenorm_fwd(x, g, y, rnorm, *, R: int, H: int, eps: float = 1e-5) -> None:
             meta={"bytes": 6.0 * R * H})
 
 
-def scalenorm_bwd(dy, x, rnorm, g, dres, dx, dxb, drop: DropSpec, dg, *, R: int, H: int, eps: float = 1e-5) -> None:
+def scalenorm_bwd(dy, x, rnorm, g, dres, dx, dxb, drop: DropSpec, dg, *, R: int, H: int, eps: float = 1e-5,
+                  ws: Optional[DetWorkspace] = None) -> None:
     d = drop.c()
-    _launch("mmfm_scalenorm_bwd", dy.data_ptr(), x.data_ptr(), rnorm.data_ptr(), g.data_ptr(), _p(dres), _p(dx), _p(dxb),
-            C.byref(d), _p(dg), R, H, eps, keep=(d,),
-            meta={"bytes": float(R) * H * (2 + 4 + (4 if dres is not None else 0) + (4 if dx is not None else 0)
-                                           + (2 if dxb is not None else 0))})
+    args = (dy.data_ptr(), x.data_ptr(), rnorm.data_ptr(), g.data_ptr(), _p(dres), _p(dx), _p(dxb), C.byref(d), _p(dg),
+            R, H, eps)
+    meta = {"bytes": float(R) * H * (2 + 4 + (4 if dres is not None else 0) + (4 if dx is not None else 0)
+                                     + (2 if dxb is not None else 0))}
+    if deterministic():
+        _launch_det("mmfm_scalenorm_bwd", ws, det_ws_need(_lib.DET_SCALENORM_BWD, R, H), x.device, *args, keep=(d,),
+                    meta=meta)
+        return
+    _launch("mmfm_scalenorm_bwd", *args, keep=(d,), meta=meta)
 
 
 def _attn_args(q, k, v, o, lse, key_valid, *, B, n_heads, Sq, Sk, d_head, mask_mode, mod_q=None, mod_k=None,
@@ -328,9 +406,15 @@ def embed_assemble(mod_row, pos, ts, emb, *, B, T, S, off, H) -> None:
             meta={"bytes": 4.0 * B * T * H})                       # emb rows written (the tables stay in cache)
 
 
-def embed_assemble_bwd(g, g2, ts, dpos, dmod, *, B, T, S, off, H) -> None:
-    _launch("mmfm_embed_assemble_bwd", g.data_ptr(), _p(g2), _p(ts), _p(dpos), dmod.data_ptr(), B, T, S, off, H,
-            meta={"bytes": 4.0 * B * T * H * (2 if g2 is not None else 1)})   # gradient rows read
+def embed_assemble_bwd(g, g2, ts, dpos, dmod, *, B, T, S, off, H, ws: Optional[DetWorkspace] = None) -> None:
+    args = (g.data_ptr(), _p(g2), _p(ts), _p(dpos), dmod.data_ptr(), B, T, S, off, H)
+    meta = {"bytes": 4.0 * B * T * H * (2 if g2 is not None else 1)}   # gradient rows read
+    if deterministic():
+        n_pos = dpos.shape[0] if dpos is not None else 0
+        _launch_det("mmfm_embed_assemble_bwd", ws, det_ws_need(_lib.DET_EMBED_ASM_BWD, B, T, H), g.device, *args, n_pos,
+                    meta={**meta, "kernels": 2 if dpos is not None else 1})
+        return
+    _launch("mmfm_embed_assemble_bwd", *args, meta=meta)
 
 
 def embed_grad_prep(dx, dtok, row_zero, drop: DropSpec, *, B, T, S, off, H) -> None:
@@ -348,11 +432,16 @@ def smallc_embed_fwd(inp, W1, b1, W2, b2, emb, x, hid, row_zero, drop: DropSpec,
 
 
 def smallc_embed_bwd(inp, hid, W2, dx, row_zero, drop: DropSpec, act_scale, act, dW1, db1, dW2, db2, *, B, T, S, off,
-                     Cc, H) -> None:
+                     Cc, H, ws: Optional[DetWorkspace] = None) -> None:
     d = drop.c()
-    _launch("mmfm_smallc_embed_bwd", inp.data_ptr(), hid.data_ptr(), W2.data_ptr(), dx.data_ptr(), _p(row_zero),
-            C.byref(d), float(act_scale), act, dW1.data_ptr(), db1.data_ptr(), dW2.data_ptr(), db2.data_ptr(), B, T, S,
-            off, Cc, H, keep=(d,), meta={"bytes": float(B) * T * (4.0 * H + 12.0 * Cc)})   # dx rows in
+    args = (inp.data_ptr(), hid.data_ptr(), W2.data_ptr(), dx.data_ptr(), _p(row_zero), C.byref(d), float(act_scale), act,
+            dW1.data_ptr(), db1.data_ptr(), dW2.data_ptr(), db2.data_ptr(), B, T, S, off, Cc, H)
+    meta = {"bytes": float(B) * T * (4.0 * H + 12.0 * Cc)}   # dx rows in
+    if deterministic():
+        _launch_det("mmfm_smallc_embed_bwd", ws, det_ws_need(_lib.DET_SMALLC_EMBED_BWD, B * T, Cc, H), dx.device, *args,
+                    keep=(d,), meta=meta)
+        return
+    _launch("mmfm_smallc_embed_bwd", *args, keep=(d,), meta=meta)
 
 
 def smallc_head_fwd(y, W, b, preds, *, R, H, Cc) -> None:
@@ -360,9 +449,15 @@ def smallc_head_fwd(y, W, b, preds, *, R, H, Cc) -> None:
             meta={"bytes": float(R) * (2.0 * H + 4.0 * Cc)})
 
 
-def smallc_head_bwd(y, W, dpreds, dy, dW, db, *, R, H, Cc) -> None:
-    _launch("mmfm_smallc_head_bwd", y.data_ptr(), W.data_ptr(), dpreds.data_ptr(), dpreds.stride(0), dy.data_ptr(),
-            dW.data_ptr(), db.data_ptr(), R, H, Cc, meta={"bytes": float(R) * (4.0 * H + 2.0 * Cc)})
+def smallc_head_bwd(y, W, dpreds, dy, dW, db, *, R, H, Cc, ws: Optional[DetWorkspace] = None) -> None:
+    args = (y.data_ptr(), W.data_ptr(), dpreds.data_ptr(), dpreds.stride(0), dy.data_ptr(), dW.data_ptr(), db.data_ptr(),
+            R, H, Cc)
+    meta = {"bytes": float(R) * (4.0 * H + 2.0 * Cc)}
+    if deterministic():
+        _launch_det("mmfm_smallc_head_bwd", ws, det_ws_need(_lib.DET_SMALLC_HEAD_BWD, R, H, Cc), dW.device, *args,
+                    meta=meta)
+        return
+    _launch("mmfm_smallc_head_bwd", *args, meta=meta)
 
 
 def loss_fwd_bwd(preds, targets, tok_mask, inv_n, kind, partials, dpreds, *, B, T, Cc, S, off) -> None:
