@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MMFM_ABI_VERSION 5
+#define MMFM_ABI_VERSION 6
 
 const char* mmfm_last_error(void);
 int mmfm_abi_version(void);
@@ -243,6 +243,24 @@ int mmfm_loss_fwd_bwd(const float* preds, const float* targets, const unsigned c
 /* mod_loss[m] = sum of partials[m*n_partials ...]; loss = sum_m mod_loss[m] * inv_n[0] */
 int mmfm_loss_finalize(const float* partials, int n_partials, int n_mod, const float* inv_n, float* mod_loss,
                        float* loss, void* stream);
+/* Head gradient for arbitrary upstream gradients of loss, mod_loss[m] and preds (autograd of every step output):
+ *   dpreds = mask * ell'(preds, targets) * (g_loss[0] * inv_n[0] + g_mod[0]) + g_preds
+ * preds / targets / tok_mask / S / off / kind as in mmfm_loss_fwd_bwd.  g_loss, g_mod: device scalars, NULL = that
+ * upstream gradient is absent (its term is not evaluated, so inv_n = inf with g_loss NULL stays finite).  g_preds:
+ * fp32 upstream gradient of preds with ELEMENT strides (gp_sb, gp_st, gp_sc) over (b, t, c) -- 0 for broadcast
+ * dimensions -- or NULL.  ell' is the same device code as mmfm_loss_fwd_bwd: g_loss = 1 alone reproduces its dpreds
+ * bit for bit.  Elementwise, no atomics. */
+int mmfm_loss_grad(const float* preds, const float* targets, const unsigned char* tok_mask, int S, int off,
+                   const float* inv_n, const float* g_loss, const float* g_mod, const float* g_preds, long long gp_sb,
+                   long long gp_st, long long gp_sc, int kind, int B, int T, int C, void* dpreds, long long lddp,
+                   void* stream);
+/* Input gradient of the small-channel embedder (the backward of mmfm_smallc_embed_fwd with respect to `in`), from the
+ * saved `hid` and upstream rows that mmfm_smallc_embed_bwd reads, plus W1 [2C, C] (the inputs themselves are not needed):
+ *   dX[b,t,:] (+)= W1^T . (act'(hid[b,t,:]) * (W2^T . dropout(row_zero ? 0 : dx[b, off+t, :])))
+ * dX fp32 [B*T, C] at pitch lddx; accumulate != 0 adds to it.  One warp per row, no atomics (deterministic). */
+int mmfm_smallc_embed_dx(const float* hid, const float* W1, const float* W2, const float* dx,
+                         const unsigned char* row_zero, const mmfm_dropout* drop, float act_scale, int act, float* dX,
+                         long long lddx, int accumulate, int B, int T, int S, int off, int C, int H, void* stream);
 
 /* ---- multi-tensor cast: bf16 shadows (and transposed shadows for dgrad) of all fp32 weights in one launch -- */
 typedef struct mmfm_cast_item {

@@ -20,7 +20,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
               "-Xptxas", "-v"]
 
 MAX_MOD = 8
-ABI_VERSION = 5
+ABI_VERSION = 6
 MASK_SITE = 8192
 
 
@@ -194,6 +194,8 @@ SIGNATURES = {
     "mmfm_smallc_head_bwd": [_vp, _vp, _vp, _ll, _vp, _vp, _vp, _i, _i, _i, _vp],
     "mmfm_loss_fwd_bwd": [_vp, _vp, _vp, _i, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp, _ll, _vp],
     "mmfm_loss_finalize": [_vp, _i, _i, _vp, _vp, _vp, _vp],
+    "mmfm_loss_grad": [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _ll, _ll, _ll, _i, _i, _i, _i, _vp, _ll, _vp],
+    "mmfm_smallc_embed_dx": [_vp, _vp, _vp, _vp, _vp, _DP, _f, _i, _vp, _ll, _i, _i, _i, _i, _i, _i, _i, _vp],
     # deterministic mode: the same arguments plus the workspace (include/mmfm_b200.h)
     "mmfm_det_ws_bytes": [_i, _ll, _ll, _ll, C.POINTER(C.c_longlong), C.POINTER(C.c_int)],
     "mmfm_gemm_wgrad_det": [_vp, _ll, _vp, _ll, _i, _i, _i, _vp, _ll, _vp, _WS, _vp],

@@ -13,6 +13,7 @@ from typing import Dict, Optional
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import ops
 from ._lib import LOSS_MSE, LOSS_POISSON, MmfmError
@@ -39,7 +40,9 @@ def _pad8(n: int) -> int:
 
 
 class _LinearLossFn(torch.autograd.Function):
-    """loss = sum(ell(x W^T + b, targets)) / n_examples, with d loss / d preds produced by the fused loss kernel."""
+    """loss = sum(ell(x W^T + b, targets)) / n_examples, with d loss / d preds produced by the fused loss kernel.
+    loss and preds are both differentiable, and so is x: a gradient of loss alone scales the forward's dpreds; any
+    other combination rebuilds dpreds with mmfm_loss_grad (mask of ones, T = S = 1)."""
 
     @staticmethod
     def forward(ctx, x2d, weight, bias, targets2d, kind, n_examples):
@@ -50,7 +53,7 @@ class _LinearLossFn(torch.autograd.Function):
         dev = x2d.device
         xb = torch.empty(R, _pad8(K), device=dev, dtype=bf16)[:, :K]
         wb = torch.empty(N, _pad8(K), device=dev, dtype=bf16)[:, :K]
-        ops.cast_bf16(x2d.contiguous(), xb)
+        ops.cast_bf16(x2d.detach().float().contiguous(), xb)
         ops.cast_bf16(weight.detach().contiguous(), wb)
         preds = torch.empty(R, N, device=dev, dtype=torch.float32)
         ops.gemm_tn(xb, wb, preds, bias=bias.detach() if bias is not None else None)
@@ -60,25 +63,49 @@ class _LinearLossFn(torch.autograd.Function):
         npart = 296
         partials = torch.zeros(npart, device=dev)
         dpreds = torch.empty(R, _pad8(N), device=dev, dtype=bf16)[:, :N]
-        ops.loss_fwd_bwd(preds, targets2d.contiguous(), ones, inv_n, kind, partials, dpreds, B=R, T=1, Cc=N, S=1, off=0)
+        targets = targets2d.detach().float().contiguous()
+        ops.loss_fwd_bwd(preds, targets, ones, inv_n, kind, partials, dpreds, B=R, T=1, Cc=N, S=1, off=0)
         mod_loss, loss = torch.empty(1, device=dev), torch.empty(1, device=dev)
         ops.loss_finalize(partials, npart, 1, inv_n, mod_loss, loss)
-        ctx.save_for_backward(xb, dpreds)
-        ctx.shape = (N, K, bias is not None)
-        ctx.mark_non_differentiable(preds)
+        ctx.save_for_backward(xb, dpreds, preds, targets, ones, inv_n)
+        ctx.weight = weight.detach()
+        ctx.shape = (N, K, bias is not None, kind, x2d.dtype)
+        ctx.set_materialize_grads(False)
         return loss.reshape(()), preds
 
     @staticmethod
-    def backward(ctx, g_loss, _g_preds):
-        xb, dpreds = ctx.saved_tensors
-        N, K, has_bias = ctx.shape
-        dW = torch.zeros(N, K, device=xb.device)
-        db = torch.zeros(N, device=xb.device) if has_bias else None
-        ops.gemm_wgrad(dpreds, xb, dW, dbias=db)
-        ops.scale_inplace(dW, g_loss.reshape(1).float())
-        if db is not None:
-            ops.scale_inplace(db, g_loss.reshape(1).float())
-        return None, dW, db, None, None, None
+    @once_differentiable
+    def backward(ctx, g_loss, g_preds):
+        xb, dpreds, preds, targets, ones, inv_n = ctx.saved_tensors
+        N, K, has_bias, kind, x_dtype = ctx.shape
+        R = xb.shape[0]
+        dev = xb.device
+        want_x = ctx.needs_input_grad[0]
+        plain = g_preds is None and not want_x
+        if plain:
+            scale = g_loss.reshape(1).float()
+        else:
+            scale = None
+            ops.loss_grad(preds, targets, ones, inv_n, kind, dpreds,
+                          g_loss=g_loss.reshape(1).float() if g_loss is not None else None,
+                          g_preds=g_preds.float().unsqueeze(1) if g_preds is not None else None, B=R, T=1, Cc=N, S=1,
+                          off=0)
+        dW = db = dx = None
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            dW = torch.zeros(N, K, device=dev)
+            db = torch.zeros(N, device=dev) if has_bias else None
+            ops.gemm_wgrad(dpreds, xb, dW, dbias=db)
+            if scale is not None:
+                ops.scale_inplace(dW, scale)
+                if db is not None:
+                    ops.scale_inplace(db, scale)
+        if want_x:       # dX = dpreds . W on a transposed bf16 copy of W
+            wt = torch.empty(K, _pad8(N), device=dev, dtype=bf16)[:, :N]
+            ops.cast_bf16(ctx.weight.contiguous(), None, wt)
+            dx32 = torch.empty(R, K, device=dev, dtype=torch.float32)
+            ops.gemm_tn(dpreds, wt, dx32)
+            dx = dx32.to(x_dtype)
+        return dx, dW, db, None, None, None
 
 
 class BaselineDecoder(nn.Module):

@@ -887,6 +887,10 @@ __global__ void __launch_bounds__(256) loss_kernel(const float* __restrict__ pre
 // summed under the (B,T)->(B,T,K) expanded mask and normalised by the expanded mask count like every other modality.
 // thread = one token row (K <= kMaxClasses classes in registers); grad = mask * inv_n * (softmax * sum_k t_k - t).
 constexpr int kMaxClasses = 64;
+// d ell / d preds[c] of one row, from the row's max, 1 / sum_c exp(preds - max) and sum_c targets
+MMFM_DEVINL float ce_grad_elem(float p, float t, float mx, float inv_se, float tsum) {
+  return __expf(p - mx) * inv_se * tsum - t;
+}
 __global__ void __launch_bounds__(256) loss_ce_kernel(const float* __restrict__ preds, const float* __restrict__ targets,
                                                        const unsigned char* __restrict__ tok_mask, int S, int off,
                                                        const float* __restrict__ inv_n, int B, int T, int C,
@@ -918,8 +922,7 @@ __global__ void __launch_bounds__(256) loss_ce_kernel(const float* __restrict__ 
       acc -= tc * (pr[c] - lse);
     }
     const float inv_se = 1.0f / se;
-    for (int c = 0; c < C; ++c)
-      dp[c] = __float2bfloat16_rn((__expf(pr[c] - mx) * inv_se * tsum - tg[c]) * invn);
+    for (int c = 0; c < C; ++c) dp[c] = __float2bfloat16_rn(ce_grad_elem(pr[c], tg[c], mx, inv_se, tsum) * invn);
   }
   const float s = block_sum(acc, sh);
   if (threadIdx.x == 0) partials[blockIdx.x] = s;
@@ -938,6 +941,134 @@ __global__ void __launch_bounds__(256) loss_finalize_kernel(const float* __restr
     tot += s;
   }
   if (threadIdx.x == 0) loss[0] = tot * inv_n[0];
+}
+
+// Head gradient for arbitrary upstream gradients of the step outputs (autograd of loss, mod_loss[m] and preds):
+// dpreds = mask * ell' * (g_loss * inv_n + g_mod) + g_preds.  ell' comes from the device code of the two loss kernels
+// above, so g_loss = 1 alone gives their dpreds bit for bit.  A term whose upstream gradient is absent is never
+// evaluated (inv_n is inf when no token is masked).  g_preds is read through element strides: autograd hands the
+// gradients of sum() / mean() over as stride-0 broadcasts.
+MMFM_DEVINL float loss_grad_coef(const float* g_loss, const float* g_mod, const float* inv_n) {
+  float coef = 0.f;
+  if (g_loss) coef = __ldg(g_loss) * __ldg(inv_n);
+  if (g_mod) coef += __ldg(g_mod);
+  return coef;
+}
+
+template <int KIND>
+__global__ void __launch_bounds__(256) loss_grad_kernel(const float* __restrict__ preds, const float* __restrict__ targets,
+                                                         const unsigned char* __restrict__ tok_mask, int S, int off,
+                                                         const float* __restrict__ inv_n, const float* g_loss,
+                                                         const float* g_mod, const float* __restrict__ g_preds,
+                                                         long long gp_sb, long long gp_st, long long gp_sc, int B, int T,
+                                                         int C, bf16* __restrict__ dpreds, long long lddp) {
+  const bool head = g_loss != nullptr || g_mod != nullptr;
+  const float coef = head ? loss_grad_coef(g_loss, g_mod, inv_n) : 0.f;
+  const long long total = (long long)B * T * C;
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const long long r = e / C;
+    const int c = (int)(e - r * C);
+    const long long b = r / T;
+    const int t = (int)(r - b * T);
+    float v = 0.f;
+    if (head && tok_mask[b * S + off + t]) {
+      float l, g;
+      loss_elem<KIND>(__ldg(preds + e), __ldg(targets + e), l, g);
+      v = g * coef;
+    }
+    if (g_preds) v += __ldg(g_preds + b * gp_sb + t * gp_st + c * gp_sc);
+    dpreds[r * lddp + c] = __float2bfloat16_rn(v);
+  }
+}
+
+// categorical variant: thread = one token row, as loss_ce_kernel
+__global__ void __launch_bounds__(256) loss_grad_ce_kernel(const float* __restrict__ preds, const float* __restrict__ targets,
+                                                            const unsigned char* __restrict__ tok_mask, int S, int off,
+                                                            const float* __restrict__ inv_n, const float* g_loss,
+                                                            const float* g_mod, const float* __restrict__ g_preds,
+                                                            long long gp_sb, long long gp_st, long long gp_sc, int B,
+                                                            int T, int C, bf16* __restrict__ dpreds, long long lddp) {
+  const bool head = g_loss != nullptr || g_mod != nullptr;
+  const float coef = head ? loss_grad_coef(g_loss, g_mod, inv_n) : 0.f;
+  const long long rows = (long long)B * T;
+  for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (long long)gridDim.x * blockDim.x) {
+    const long long b = r / T;
+    const int t = (int)(r - b * T);
+    const float* pr = preds + r * C;
+    const float* tg = targets + r * C;
+    const float* gp = g_preds ? g_preds + b * gp_sb + t * gp_st : nullptr;
+    bf16* dp = dpreds + r * lddp;
+    if (head && tok_mask[b * S + off + t]) {
+      float mx = -INFINITY, se = 0.f, tsum = 0.f;
+      for (int c = 0; c < C; ++c) mx = fmaxf(mx, pr[c]);
+      for (int c = 0; c < C; ++c) se += __expf(pr[c] - mx);
+      for (int c = 0; c < C; ++c) tsum += tg[c];
+      const float inv_se = 1.0f / se;
+      for (int c = 0; c < C; ++c) {
+        float v = ce_grad_elem(pr[c], tg[c], mx, inv_se, tsum) * coef;
+        if (gp) v += gp[c * gp_sc];
+        dp[c] = __float2bfloat16_rn(v);
+      }
+    } else {
+      for (int c = 0; c < C; ++c) dp[c] = __float2bfloat16_rn(gp ? gp[c * gp_sc] : 0.f);
+    }
+  }
+}
+
+// Input gradient of the small-channel embedder: warp = one token row.  The lanes stride over H for the 2C dot products
+// with W2 (butterfly sums, fixed order), then lane c < C forms dX[r, c] from the 2C hidden gradients.
+__global__ void __launch_bounds__(256) smallc_embed_dx_kernel(const float* __restrict__ hid, const float* __restrict__ W1,
+                                                               const float* __restrict__ W2, const float* __restrict__ dx,
+                                                               const unsigned char* __restrict__ row_zero, DropCfg drop,
+                                                               float act_scale, int act, float* __restrict__ dX,
+                                                               long long lddx, int accumulate, int B, int T, int S,
+                                                               int off, int C, int H) {
+  const int lane = threadIdx.x & 31;
+  const int C2 = 2 * C;
+  const long long R = (long long)B * T;
+  const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+  unsigned long long seed = 0ull;
+  if (drop.thresh != 0u) seed = *drop.seed;
+  const uint32_t gpr = (uint32_t)((H + 15) >> 4);
+  for (long long r = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < R; r += nwarps) {
+    const long long b = r / T;
+    const int t = (int)(r - b * T);
+    float acc[kMaxC2];
+#pragma unroll
+    for (int j = 0; j < kMaxC2; ++j) acc[j] = 0.f;
+    if (!(row_zero && row_zero[off + t])) {
+      for (int h = lane; h < H; h += 32) {
+        float d = __ldg(dx + (b * S + off + t) * H + h);
+        if (drop.thresh != 0u)
+          d = drop_byte_at(seed, drop.site, (uint64_t)r, gpr, (uint32_t)h) < drop.thresh ? 0.f : d * drop.scale;
+#pragma unroll
+        for (int j = 0; j < kMaxC2; ++j)
+          if (j < C2) acc[j] += d * __ldg(W2 + h * C2 + j);
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < kMaxC2; ++j) {
+      if (j < C2) {
+        float dh = warp_sum(acc[j]);
+        // derivative of act(v)*scale expressed through the saved output a = hid (as smallc_embed_bwd_kernel)
+        if (act == MMFM_ACT_SOFTSIGN) {
+          const float tt = 1.0f - fabsf(__ldg(hid + r * C2 + j) / act_scale);
+          dh *= act_scale * tt * tt;
+        } else {
+          dh *= act_scale;
+        }
+        acc[j] = dh;
+      }
+    }
+    if (lane < C) {
+      float v = 0.f;
+#pragma unroll
+      for (int j = 0; j < kMaxC2; ++j)
+        if (j < C2) v += acc[j] * __ldg(W1 + j * C + lane);
+      float* o = dX + r * lddx + lane;
+      *o = accumulate ? *o + v : v;
+    }
+  }
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1292,6 +1423,46 @@ extern "C" int mmfm_loss_finalize(const float* partials, int n_partials, int n_m
                                   float* loss, void* stream) {
   MMFM_REQUIRE(partials && inv_n && mod_loss && loss && n_partials > 0 && n_mod > 0, "mmfm_loss_finalize: bad arguments");
   loss_finalize_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(partials, n_partials, n_mod, inv_n, mod_loss, loss);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_loss_grad(const float* preds, const float* targets, const unsigned char* tok_mask, int S, int off,
+                              const float* inv_n, const float* g_loss, const float* g_mod, const float* g_preds,
+                              long long gp_sb, long long gp_st, long long gp_sc, int kind, int B, int T, int C,
+                              void* dpreds, long long lddp, void* stream) {
+  MMFM_REQUIRE(preds && targets && tok_mask && inv_n && dpreds, "mmfm_loss_grad: null pointer");
+  MMFM_REQUIRE(kind == MMFM_LOSS_POISSON || kind == MMFM_LOSS_MSE || kind == MMFM_LOSS_CE, "mmfm_loss_grad: bad loss kind %d", kind);
+  MMFM_REQUIRE(B > 0 && T > 0 && C > 0 && lddp >= C && off >= 0 && off + T <= S, "mmfm_loss_grad: bad shape");
+  MMFM_REQUIRE(gp_sb >= 0 && gp_st >= 0 && gp_sc >= 0, "mmfm_loss_grad: negative g_preds stride");
+  cudaStream_t st = (cudaStream_t)stream;
+  bf16* dp = (bf16*)dpreds;
+  if (kind == MMFM_LOSS_CE) {
+    MMFM_REQUIRE(C <= kMaxClasses, "mmfm_loss_grad: cross-entropy supports up to %d classes (got %d)", kMaxClasses, C);
+    loss_grad_ce_kernel<<<ew_grid((long long)B * T, 256), 256, 0, st>>>(preds, targets, tok_mask, S, off, inv_n, g_loss,
+                                                                         g_mod, g_preds, gp_sb, gp_st, gp_sc, B, T, C, dp, lddp);
+  } else {
+    const int grid = ew_grid((long long)B * T * C, 256);
+#define LGRAD(K) loss_grad_kernel<K><<<grid, 256, 0, st>>>(preds, targets, tok_mask, S, off, inv_n, g_loss, g_mod, g_preds, \
+                                                          gp_sb, gp_st, gp_sc, B, T, C, dp, lddp)
+    if (kind == MMFM_LOSS_POISSON) LGRAD(MMFM_LOSS_POISSON); else LGRAD(MMFM_LOSS_MSE);
+#undef LGRAD
+  }
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_smallc_embed_dx(const float* hid, const float* W1, const float* W2, const float* dx,
+                                    const unsigned char* row_zero, const mmfm_dropout* drop, float act_scale, int act,
+                                    float* dX, long long lddx, int accumulate, int B, int T, int S, int off, int C, int H,
+                                    void* stream) {
+  MMFM_REQUIRE(hid && W1 && W2 && dx && dX, "mmfm_smallc_embed_dx: null pointer");
+  MMFM_REQUIRE(C >= 1 && C <= kMaxC, "mmfm_smallc_embed_dx: C=%d outside [1,%d]", C, kMaxC);
+  MMFM_REQUIRE(act == MMFM_ACT_NONE || act == MMFM_ACT_SOFTSIGN, "mmfm_smallc_embed_dx: bad act %d", act);
+  MMFM_REQUIRE(B > 0 && T > 0 && H > 0 && off >= 0 && off + T <= S && lddx >= C, "mmfm_smallc_embed_dx: bad shape");
+  MMFM_REQUIRE(drop == nullptr || drop->thresh == 0u || drop->seed, "mmfm_smallc_embed_dx: dropout without seed pointer");
+  smallc_embed_dx_kernel<<<ew_grid((long long)B * T * 32, 256), 256, 0, (cudaStream_t)stream>>>(
+      hid, W1, W2, dx, row_zero, to_drop(drop), act_scale, act, dX, lddx, accumulate, B, T, S, off, C, H);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

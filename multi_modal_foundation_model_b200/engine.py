@@ -17,10 +17,11 @@ from __future__ import annotations
 import ctypes as C
 import os
 import weakref
-from typing import Any, Dict, List, Optional, Tuple
+from typing import Any, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import adapter, masker as _masker, ops
 from ._lib import (ACT_DGELU, ACT_DSOFTSIGN, ACT_GELU, ACT_GELU_DG, ACT_MULAUX, ACT_NONE, ACT_ROWDOT_DROP, ACT_SOFTSIGN, LOSS_CE, LOSS_MSE, LOSS_POISSON, MASK_CAUSAL,
@@ -292,9 +293,10 @@ class Plan:
     """All buffers + the recorded forward / backward launch lists for one (batch size, train/eval) shape."""
 
     def __init__(self, eng: "Engine", B: int, training: bool, session=None, arena: Optional[Arena] = None,
-                 u8_mods: Tuple[str, ...] = ()):
+                 u8_mods: Tuple[str, ...] = (), grad_inputs: Tuple[str, ...] = ()):
         self.eng, self.B, self.training = eng, B, training
         self.u8_mods = tuple(u8_mods)      # modalities whose inputs / targets arrive as uint8 counts (wire format)
+        self.grad_inputs = tuple(grad_inputs)   # modalities whose inputs get a gradient (recorded after the last mark)
         self.arena_bytes = 0
         if arena is not None:
             arena.reset()
@@ -344,6 +346,8 @@ class Plan:
         self.mask = {m.name: i64(B, T) for m in mods}
         self.seed = eng.seed               # ONE device seed per engine: every plan's launches capture the same pointer
         self.gscale = torch.ones(1, device=dev, dtype=torch.float32)
+        self.one = torch.ones(1, device=dev, dtype=torch.float32)
+        self._dpreds_dirty = False         # dpreds overwritten by head_grad since the last forward
         # per-modality 32-bit Bernoulli thresholds of the device-side mask sampler (0 = read the mask buffer); a device
         # array so that the captured graph sees per-step changes, staged through pinned host memory
         self.sample_thresh = torch.zeros(len(mods), device=dev, dtype=torch.int32)
@@ -725,6 +729,7 @@ class Plan:
 
         # ---- embeddings ------------------------------------------------------------------------------------
         dtok = b16(BT, H)
+        self.dhid: Dict[Tuple[int, str], torch.Tensor] = {}
         for side, sname, Gs, G2, p_emb in ((SIDE_DEC, "decoder_embeddings", G, None, hp["dec_embed_dropout"]),
                                            (SIDE_ENC, "encoder_embeddings", Genc, Gctx, hp["embed_dropout"])):
             for k, m in reversed(list(enumerate(mods))):
@@ -744,7 +749,7 @@ class Plan:
                                          ws=self.det_ws)
                 else:
                     ops.embed_grad_prep(Gs, dtok, self.zero, drop, B=B, T=T, S=S, off=off, H=H)
-                    dhid = b16(BT, 2 * m.C)
+                    dhid = self.dhid[(side, m.name)] = b16(BT, 2 * m.C)
                     back = ACT_DSOFTSIGN if eng.embed_act == ACT_SOFTSIGN else ACT_NONE
                     lin_bwd(dtok, A[pre + ".hid"], pre + ".projection", pre + ".projection", dhid, act=back,
                             aux=A[pre + ".hid"] if back else None, act_scale=eng.embed_scale)
@@ -752,12 +757,54 @@ class Plan:
         mark(None)
         ops.scale_inplace(st.grad, self.gscale)
 
+        # ---- input gradients (plans whose inputs require grad; they always run with gscale = 1) --------------
+        # Both embedders read the inputs: decoder side first, the encoder side adds to it.  Spike streams: the dgrad of
+        # token_embed through the GEMM (dX = dhid . W1) on a transposed bf16 copy cast here, so the shared shadow cast
+        # of the default schedule stays as it is; the second GEMM adds the first one's output as its residual.
+        self.dinp: Dict[str, torch.Tensor] = {}
+        sides = ((SIDE_DEC, "decoder_embeddings", G, hp["dec_embed_dropout"]),
+                 (SIDE_ENC, "encoder_embeddings", Genc, hp["embed_dropout"]))
+        for k, m in enumerate(mods):
+            if m.name not in self.grad_inputs:
+                continue
+            dX = None
+            for i, (side, sname, Gs, p_emb) in enumerate(sides):
+                pre = f"{self.prefix}{sname}.{m.name}.embedder"
+                if m.small:
+                    dX = f32(BT, m.C) if dX is None else dX
+                    ops.smallc_embed_dx(A[pre + ".hid"], st.p(pre + ".token_embed.weight"),
+                                        st.p(pre + ".projection.weight"), Gs, self.zero,
+                                        self._drop(SITE_EMBED, m.index, side, p_emb), eng.embed_scale, eng.embed_act, dX,
+                                        accumulate=i > 0, B=B, T=T, S=S, off=k * T, Cc=m.C, H=H)
+                else:
+                    w1t = b16(m.C, 2 * m.C)
+                    ops.cast_bf16(st.p(pre + ".token_embed.weight"), None, w1t)
+                    out = f32(BT, _pad(m.C, 4))[:, :m.C]          # fp32 rows at a 16-byte pitch
+                    ops.gemm_tn(self.dhid[(side, m.name)], w1t, out, res=dX)
+                    dX = out
+            self.dinp[m.name] = dX
+
     # ---------------------------------------------------------------------------------------------------
     # -- execution: eager the first time (module load, kernel attributes), CUDA-graph replay afterwards ------
     def _fwd_body(self):
         # every step advances the stream (dropout sites in train(), the device-side mask sampler in either mode)
         self.seed.add_(0x632BE59BD9B4E019)
         ops.run_recorded(self.fwd_calls)
+
+    def head_grad(self, g_loss: Optional[torch.Tensor], g_mod: Optional[torch.Tensor],
+                  g_preds: Sequence[Optional[torch.Tensor]]) -> None:
+        """Overwrite dpreds with the head gradient of arbitrary upstream gradients of loss (scalar), mod_loss (vector)
+        and preds (one per modality); None = absent.  The backward schedule then runs with gscale = 1."""
+        restore = g_loss is self.one and g_mod is None and not any(g is not None for g in g_preds)
+        g_loss = g_loss.reshape(1).float() if g_loss is not None else None
+        g_mod = g_mod.float() if g_mod is not None else None
+        B, T = self.B, self.eng.T
+        for k, m in enumerate(self.mods):
+            gp = g_preds[k] if k < len(g_preds) else None
+            ops.loss_grad(self.preds[m.name], self.tgt[m.name], self.tmask, self.inv_n, m.loss_kind,
+                          self.dpreds[m.name], g_loss=g_loss, g_mod=g_mod[k:k + 1] if g_mod is not None else None,
+                          g_preds=gp.float() if gp is not None else None, B=B, T=T, Cc=m.C, S=self.S, off=k * T)
+        self._dpreds_dirty = not restore       # g_loss = 1 alone gives the forward's dpreds bit for bit
 
     def set_sample_thresh(self, thresh: List[int]) -> None:
         if thresh != self._thresh_cur:
@@ -784,6 +831,7 @@ class Plan:
             self._g_fwd.replay()
         else:
             self._fwd_body()
+        self._dpreds_dirty = False
 
     def run_backward(self):
         """Zeroes the flat gradient buffer and runs the backward schedule."""
@@ -799,18 +847,31 @@ class Plan:
 # ------------------------------------------------------------------------------------------------------------
 class _StepFn(torch.autograd.Function):
     """Autograd node of one step: forward = the plan's forward schedule; backward = its backward schedule, writing
-    into the flat gradient buffer that ``Parameter.grad`` views (trainer/base.py:194-195 semantics)."""
+    into the flat gradient buffer that ``Parameter.grad`` views (trainer/base.py:194-195 semantics).
+
+    Outputs: loss, the mod_loss vector and one preds tensor per modality, all differentiable.  Extra inputs: the
+    modality inputs that require grad (``plan.grad_inputs``, in that order); their gradients are returned."""
 
     @staticmethod
-    def forward(ctx, anchor, eng, plan):
+    def forward(ctx, anchor, eng, plan, *inputs):
         plan.run_forward()
         ctx.eng, ctx.plan = eng, plan
-        return plan.loss.clone().reshape(())
+        ctx.in_meta = [(x.shape, x.dtype) for x in inputs]
+        ctx.set_materialize_grads(False)        # unused outputs arrive as None: their terms are skipped
+        preds = [plan.preds[m.name].clone() for m in plan.mods]
+        return (plan.loss.clone().reshape(()), plan.mod_loss.clone(), *preds)
 
     @staticmethod
-    def backward(ctx, grad_loss):
-        ctx.eng.backward(ctx.plan, grad_loss)
-        return None, None, None
+    @once_differentiable
+    def backward(ctx, grad_loss, grad_mod, *grad_preds):
+        ctx.eng.backward(ctx.plan, grad_loss, grad_mod, grad_preds)
+        pl = ctx.plan
+        dinp = []
+        for name, (shape, dtype) in zip(pl.grad_inputs, ctx.in_meta):
+            g = torch.empty(shape, device=pl.eng.device, dtype=dtype)
+            g.copy_(pl.dinp[name].reshape(shape))             # fresh tensor: the plan buffer is reused next step
+            dinp.append(g)
+        return (None, None, None, *dinp)
 
 
 class Engine:
@@ -884,7 +945,8 @@ class Engine:
         self.output_cls = MultiModalOutput      # dropin.install() swaps in the reference's own dataclass
 
     # ---------------------------------------------------------------------------------------------------
-    def _plan(self, B: int, T: int, training: bool, session=None, u8_mods: Tuple[str, ...] = ()) -> Plan:
+    def _plan(self, B: int, T: int, training: bool, session=None, u8_mods: Tuple[str, ...] = (),
+              grad_inputs: Tuple[str, ...] = ()) -> Plan:
         if self.T is None:
             self.T = T
         elif self.T != T:
@@ -892,20 +954,24 @@ class Engine:
             self.arenas.clear()
             self.T = T
         # deterministic mode selects other kernels: its own plan (and graphs), never a change to a captured one
-        key = (B, training, session, u8_mods, ops.deterministic())
+        # input-gradient plans record extra launches after the default schedule: their own plan, like the two above
+        key = (B, training, session, u8_mods, ops.deterministic(), grad_inputs)
         pl = self.plans.get(key)
         if pl is None:
             arena = None
             if self.multi_session:
-                arena = self.arenas.get((B, training))
+                akey = (B, training, bool(grad_inputs))
+                arena = self.arenas.get(akey)
                 if arena is None:
-                    # size the shared arena from the widest session (buffers grow monotonically with the channels)
+                    # size the shared arena from the widest session (buffers grow monotonically with the channels);
+                    # with input gradients, probe with every modality's
                     widest = max(self.sessions, key=lambda k: sum(m.C for m in self.sessions[k][1]))
-                    probe = Plan(self, B, training, widest)
+                    gi = tuple(m.name for m in self.sessions[widest][1]) if grad_inputs else ()
+                    probe = Plan(self, B, training, widest, grad_inputs=gi)
                     nbytes = probe.arena_bytes + (1 << 20)
                     del probe
-                    arena = self.arenas[(B, training)] = Arena(nbytes, self.device)
-            pl = Plan(self, B, training, session, arena, u8_mods)
+                    arena = self.arenas[akey] = Arena(nbytes, self.device)
+            pl = Plan(self, B, training, session, arena, u8_mods, grad_inputs)
             self.plans[key] = pl
         return pl
 
@@ -939,7 +1005,16 @@ class Engine:
         for m in mods:
             if mod_dict[m.name]["inputs"].dtype == torch.uint8 and m.name not in u8_mods:
                 raise MmfmError(f"modality {m.name}: uint8 inputs are only supported for spike-count modalities (C > {SMALL_C})")
-        pl = self._plan(B, T, training, session, u8_mods)
+        grad_on = torch.is_grad_enabled()
+        if grad_on:
+            for m in mods:
+                tg = mod_dict[m.name]["targets"]
+                if torch.is_tensor(tg) and tg.requires_grad:
+                    raise NotImplementedError(f"modality {m.name}: targets that require grad are not supported (the "
+                                              "targets are data here; only inputs and parameters get gradients)")
+        # modalities whose (floating-point) inputs require grad: extra inputs of the autograd node
+        grad_inputs = tuple(m.name for m in mods if grad_on and mod_dict[m.name]["inputs"].requires_grad)
+        pl = self._plan(B, T, training, session, u8_mods, grad_inputs)
         thresh = [0] * len(mods)
         for k, m in enumerate(mods):
             d = mod_dict[m.name]
@@ -957,7 +1032,7 @@ class Engine:
                 pl.inp_u8[m.name].copy_(d["inputs"], non_blocking=True)
                 pl.tgt_u8[m.name].copy_(d["targets"], non_blocking=True)
             else:
-                pl.inp[m.name].copy_(d["inputs"], non_blocking=True)
+                pl.inp[m.name].copy_(d["inputs"].detach(), non_blocking=True)
                 pl.tgt[m.name].copy_(d["targets"], non_blocking=True)
             pl.attn[m.name].copy_(d["inputs_attn_mask"], non_blocking=True)
             pl.ts[m.name].copy_(d["inputs_timestamp"], non_blocking=True)
@@ -991,23 +1066,24 @@ class Engine:
         pl.set_sample_thresh(thresh)
         self.last_plan = pl
         anchor = None
-        if torch.is_grad_enabled():
+        if grad_on:
             anchor = next((p for p in self.store.params.values() if p.requires_grad), None)
-        if anchor is not None:
-            loss = _StepFn.apply(anchor, self, pl)
+        if anchor is not None or grad_inputs:
+            loss, mod_loss, *preds = _StepFn.apply(anchor, self, pl, *[mod_dict[n]["inputs"] for n in grad_inputs])
         else:
             pl.run_forward()
             loss = pl.loss.clone().reshape(())
+            mod_loss = pl.mod_loss.clone()
+            # fresh tensors, like the reference: the plan's buffers are overwritten by the next step
+            preds = [pl.preds[m.name].clone() for m in mods]
         out_loss, out_n, out_p, out_t = {}, {}, {}, {}
-        mod_loss = pl.mod_loss.clone()
         nex = pl.nex.clone()
         tmask = pl.tmask.view(B, len(mods), T).to(torch.int64)
         for k, m in enumerate(mods):
             d = mod_dict[m.name]
             out_loss[m.name] = mod_loss[k]
             out_n[m.name] = nex[k]
-            # fresh tensors, like the reference: the plan's buffers are overwritten by the next step
-            out_p[m.name] = pl.preds[m.name].clone()
+            out_p[m.name] = preds[k]
             out_t[m.name] = d["targets"]
             # the reference leaves these keys in the caller's dict (mm.py:272-275, decoder_embeddings.py:91,107)
             d["preds"] = out_p[m.name]
@@ -1017,7 +1093,11 @@ class Engine:
         return MultiModalOutput(loss=loss, mod_loss=out_loss, mod_n_examples=out_n, mod_preds=out_p, mod_targets=out_t)
 
     # ---------------------------------------------------------------------------------------------------
-    def backward(self, pl: Plan, grad_loss: torch.Tensor) -> None:
+    def backward(self, pl: Plan, grad_loss: Optional[torch.Tensor], grad_mod: Optional[torch.Tensor] = None,
+                 grad_preds: Sequence[Optional[torch.Tensor]] = ()) -> None:
+        """Backward of the plan's last forward for upstream gradients of loss, mod_loss and preds (None = absent).
+        A gradient of loss alone runs the default schedule with gscale = grad_loss; anything else first rewrites the
+        head gradient dpreds (Plan.head_grad) and runs the same schedule with gscale = 1."""
         st = self.store
         fresh = all(p.grad is None for p in st.params.values())
         prev = None
@@ -1030,7 +1110,13 @@ class Engine:
                 for n, p in st.params.items():
                     if p.grad is not None:
                         st.view(prev, n).copy_(p.grad)
-        pl.gscale.copy_(grad_loss.reshape(1).to(torch.float32))
+        if grad_loss is not None and grad_mod is None and all(g is None for g in grad_preds) and not pl.grad_inputs:
+            if pl._dpreds_dirty:
+                pl.head_grad(pl.one, None, ())
+            pl.gscale.copy_(grad_loss.reshape(1).to(torch.float32))
+        else:
+            pl.head_grad(grad_loss, grad_mod, grad_preds)
+            pl.gscale.fill_(1.0)
         if self.ddp is not None:
             self.ddp.run_backward(pl)
         else:

@@ -469,3 +469,27 @@ def loss_fwd_bwd(preds, targets, tok_mask, inv_n, kind, partials, dpreds, *, B, 
 def loss_finalize(partials, n_partials, n_mod, inv_n, mod_loss, loss) -> None:
     _launch("mmfm_loss_finalize", partials.data_ptr(), n_partials, n_mod, inv_n.data_ptr(), mod_loss.data_ptr(),
             loss.data_ptr())
+
+
+def loss_grad(preds, targets, tok_mask, inv_n, kind, dpreds, *, g_loss=None, g_mod=None, g_preds=None, B, T, Cc, S,
+              off) -> None:
+    """dpreds = mask * ell' * (g_loss * inv_n + g_mod) + g_preds: the head gradient for any upstream gradients of the
+    step outputs.  g_loss / g_mod: fp32 device scalars or None; g_preds: fp32 (B, T, Cc) of any strides or None."""
+    for g in (g_loss, g_mod, g_preds):
+        assert g is None or (g.dtype == torch.float32 and g.is_cuda)
+    if g_preds is not None:
+        assert tuple(g_preds.shape) == (B, T, Cc)
+    sb, st, sc = g_preds.stride() if g_preds is not None else (0, 0, 0)
+    _launch("mmfm_loss_grad", preds.data_ptr(), targets.data_ptr(), tok_mask.data_ptr(), S, off, inv_n.data_ptr(),
+            _p(g_loss), _p(g_mod), _p(g_preds), sb, st, sc, kind, B, T, Cc, dpreds.data_ptr(), dpreds.stride(0),
+            meta={"bytes": float(B) * T * Cc * (10 + (4 if g_preds is not None else 0))})
+
+
+def smallc_embed_dx(hid, W1, W2, dx, row_zero, drop: DropSpec, act_scale, act, dX, *, accumulate: bool, B, T, S, off,
+                    Cc, H) -> None:
+    """dX (fp32 [B*T, Cc], pitch from the tensor) (+)= input gradient of the small-channel embedder."""
+    assert dX.dtype == torch.float32
+    d = drop.c()
+    _launch("mmfm_smallc_embed_dx", hid.data_ptr(), W1.data_ptr(), W2.data_ptr(), dx.data_ptr(), _p(row_zero),
+            C.byref(d), float(act_scale), act, dX.data_ptr(), dX.stride(0), 1 if accumulate else 0, B, T, S, off, Cc, H,
+            keep=(d,), meta={"bytes": float(B) * T * (4.0 * H + 8.0 * Cc)})

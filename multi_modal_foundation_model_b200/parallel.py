@@ -94,11 +94,13 @@ class DataParallel:
         seg = getattr(pl, "_ddp_segments", None)
         if seg is None:
             calls = pl.bwd_calls
-            # the trailing whole-buffer scale is replaced by per-bucket scaling before each all-reduce
-            n_calls = len(calls) - 1 if calls and calls[-1][2] == "mmfm_scale_inplace" else len(calls)
+            # the whole-buffer scale right after the last mark is replaced by per-bucket scaling before each
+            # all-reduce; calls after it (input gradients, no parameter gradient) run once the buckets are enqueued
+            n_calls = pl.grad_marks[-1][0] if pl.grad_marks else len(calls)
+            tail = n_calls + 1 if n_calls < len(calls) and calls[n_calls][2] == "mmfm_scale_inplace" else n_calls
             marks = [(min(ci, n_calls), off) for ci, off in pl.grad_marks]
             buckets = plan_buckets(marks, self.eng.store.total, self.bucket_elems)
-            seg = (n_calls, buckets)
+            seg = (n_calls, buckets, tail)
             pl._ddp_segments = seg
         return seg
 
@@ -130,7 +132,7 @@ class DataParallel:
 
     def _run_backward_eager(self, pl) -> None:
         from . import ops
-        n_calls, buckets = self._segments(pl)
+        n_calls, buckets, tail = self._segments(pl)
         grad = self.eng.store.grad
         grad.zero_()
         works = []
@@ -144,6 +146,8 @@ class DataParallel:
             if self.world > 1:
                 works.append(all_reduce_mean(view, self.pg, async_op=True))
         assert done == n_calls, "bucket plan must end at the end of the backward schedule"
+        if tail < len(pl.bwd_calls):
+            ops.run_recorded(pl.bwd_calls[tail:])
         for w in works:
             if w is not None:
                 w.wait()
