@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MMFM_ABI_VERSION 6
+#define MMFM_ABI_VERSION 7
 
 const char* mmfm_last_error(void);
 int mmfm_abi_version(void);
@@ -300,6 +300,31 @@ int mmfm_column_stats(const float* pred, const float* y, long long R, int C, int
  * the bias corrections.  Decoupled weight decay, no amsgrad, maximize = false. */
 int mmfm_adamw_step(float* p, const float* g, float* exp_avg, float* exp_avg_sq, long long n, float lr, float beta1,
                     float beta2, float eps, float weight_decay, long long step, void* stream);
+
+/* Parameter groups and subsets (ABI 7): one launch updates the segments [lo, hi) of the same four flat buffers, each
+ * with the hyper-parameters of its class; elements outside every segment are neither read nor written.  A class is
+ * one (parameter group, step count) pair; the bias corrections are computed from `step` on the host in double
+ * precision, as mmfm_adamw_step does (which is the one-segment case of the same kernel).
+ * segs_dev: n_segs segments in device memory, sorted, non-overlapping, lo a multiple of 4, and chunk0 the prefix sum
+ * over the preceding segments of max(1, ceil((hi/4 - lo/4) / MMFM_ADAMW_CHUNK4)); n_chunks is the total.  The table
+ * is read by the kernel only: it can be uploaded once and reused while the parameter set stays the same.  A segment
+ * with an out-of-range class or bounds is skipped.  classes: n_classes (1..MMFM_ADAMW_MAX_CLASSES) host structs,
+ * passed to the kernel by value, so the host array may be reused as soon as the call returns. */
+#define MMFM_ADAMW_MAX_CLASSES 64
+#define MMFM_ADAMW_CHUNK4 1024
+typedef struct {
+  long long lo, hi;   /* element range of the flat buffers */
+  int cls;            /* index into classes */
+  int chunk0;         /* first work chunk of this segment */
+} mmfm_adamw_seg;
+typedef struct {
+  float lr, beta1, beta2, eps, weight_decay;
+  int pad_;
+  long long step;     /* >= 1: the 1-based update count of the class's parameters */
+} mmfm_adamw_class;
+int mmfm_adamw_multi(float* p, const float* g, float* exp_avg, float* exp_avg_sq, long long n,
+                     const mmfm_adamw_seg* segs_dev, int n_segs, int n_chunks, const mmfm_adamw_class* classes,
+                     int n_classes, void* stream);
 
 /* ---- deterministic mode (torch.use_deterministic_algorithms(True)) ---------------------------------------------
  * The entry points above that reduce across CTAs with float atomics have a *_det twin with the same arguments plus a

@@ -20,7 +20,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
               "-Xptxas", "-v"]
 
 MAX_MOD = 8
-ABI_VERSION = 6
+ABI_VERSION = 7
 MASK_SITE = 8192
 
 
@@ -150,6 +150,19 @@ class CastItem(C.Structure):
     ]
 
 
+ADAMW_MAX_CLASSES = 64
+ADAMW_CHUNK4 = 1024
+
+
+class AdamwSeg(C.Structure):
+    _fields_ = [("lo", C.c_longlong), ("hi", C.c_longlong), ("cls", C.c_int), ("chunk0", C.c_int)]
+
+
+class AdamwClass(C.Structure):
+    _fields_ = [("lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float),
+                ("weight_decay", C.c_float), ("pad_", C.c_int), ("step", C.c_longlong)]
+
+
 class DetWs(C.Structure):
     _fields_ = [("buf", C.c_void_p), ("bytes", C.c_longlong), ("tickets", C.c_void_p), ("n_tickets", C.c_int)]
 
@@ -176,6 +189,7 @@ SIGNATURES = {
     "mmfm_u8_expand": [_vp, _ll, _i, _vp, _ll, _vp, _ll, _vp],
     "mmfm_column_stats": [_vp, _vp, _ll, _i, _i, _vp, _vp],
     "mmfm_adamw_step": [_vp, _vp, _vp, _vp, _ll, _f, _f, _f, _f, _f, _ll, _vp],
+    "mmfm_adamw_multi": [_vp, _vp, _vp, _vp, _ll, _vp, _i, _i, C.POINTER(AdamwClass), _i, _vp],
     "mmfm_layernorm_fwd": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _i, _i, _vp],
     "mmfm_layernorm_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _DP, _vp, _vp, _i, _i, _i, _i, _vp],
     "mmfm_layernorm_fwd_multi": [C.POINTER(LnMultiArgs), _vp],

@@ -1126,28 +1126,62 @@ __global__ void __launch_bounds__(256) scale_inplace_kernel(float* __restrict__ 
 // Fused multi-tensor AdamW over the flat master-parameter / gradient buffers (torch.optim.AdamW semantics,
 // reference train_multi_modal.py:197-202): p *= 1 - lr*wd ; m = b1 m + (1-b1) g ; v = b2 v + (1-b2) g^2 ;
 // p -= (lr / bc1) * m / (sqrt(v) / sqrt(bc2) + eps).  One pass, 28 bytes of traffic per parameter.
+// The update runs over segments [lo, hi) of the buffers, each with the hyper-parameters of its class (one parameter
+// group at one step count); elements outside every segment are neither read nor written.  Work is split into chunks
+// of MMFM_ADAMW_CHUNK4 float4 per segment (grid-stride over chunks; a chunk finds its segment by binary search over
+// chunk0); the scalar tail of a segment belongs to its last chunk.  Classes travel by value in the parameter space.
+struct AdamwClass {
+  float lr, beta1, beta2, eps, wd, inv_bc1, inv_sqrt_bc2;
+};
+struct AdamwParams {
+  const mmfm_adamw_seg* segs;   // device table; nullptr = the single segment `one`
+  mmfm_adamw_seg one;
+  int n_segs, n_chunks, n_classes;
+  long long n;
+  AdamwClass cls[MMFM_ADAMW_MAX_CLASSES];
+};
+
 __global__ void __launch_bounds__(256) adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
-                                                     float* __restrict__ m, float* __restrict__ v, long long n,
-                                                     float lr, float beta1, float beta2, float eps, float wd,
-                                                     float inv_bc1, float inv_sqrt_bc2) {
-  const long long n4 = n >> 2;
-  const float decay = 1.0f - lr * wd, step = lr * inv_bc1, c1 = 1.0f - beta1, c2 = 1.0f - beta2;
-  auto upd = [&](float& pp, float gg, float& mm, float& vv) {
-    pp *= decay;
-    mm = fmaf(beta1, mm, c1 * gg);
-    vv = fmaf(beta2, vv, c2 * gg * gg);
-    pp -= step * mm / (sqrtf(vv) * inv_sqrt_bc2 + eps);
-  };
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
-    float4 P = reinterpret_cast<float4*>(p)[i], M = reinterpret_cast<float4*>(m)[i], V = reinterpret_cast<float4*>(v)[i];
-    const float4 G = reinterpret_cast<const float4*>(g)[i];
-    upd(P.x, G.x, M.x, V.x); upd(P.y, G.y, M.y, V.y); upd(P.z, G.z, M.z, V.z); upd(P.w, G.w, M.w, V.w);
-    reinterpret_cast<float4*>(p)[i] = P;
-    reinterpret_cast<float4*>(m)[i] = M;
-    reinterpret_cast<float4*>(v)[i] = V;
+                                                     float* __restrict__ m, float* __restrict__ v,
+                                                     const __grid_constant__ AdamwParams P) {
+  for (int c = blockIdx.x; c < P.n_chunks; c += gridDim.x) {
+    int s = 0;
+    if (P.segs != nullptr) {      // last segment with chunk0 <= c
+      int lo_s = 0, hi_s = P.n_segs - 1;
+      while (lo_s < hi_s) {
+        const int mid = (lo_s + hi_s + 1) >> 1;
+        if (P.segs[mid].chunk0 <= c) lo_s = mid; else hi_s = mid - 1;
+      }
+      s = lo_s;
+    }
+    const mmfm_adamw_seg sg = P.segs != nullptr ? P.segs[s] : P.one;
+    if (sg.cls < 0 || sg.cls >= P.n_classes || sg.lo < 0 || sg.hi > P.n || sg.lo >= sg.hi || (sg.lo & 3)) continue;
+    const AdamwClass& k = P.cls[sg.cls];
+    const float decay = 1.0f - k.lr * k.wd, step = k.lr * k.inv_bc1, c1 = 1.0f - k.beta1, c2 = 1.0f - k.beta2;
+    const float beta1 = k.beta1, beta2 = k.beta2, eps = k.eps, inv_sqrt_bc2 = k.inv_sqrt_bc2;
+    auto upd = [&](float& pp, float gg, float& mm, float& vv) {
+      pp *= decay;
+      mm = fmaf(beta1, mm, c1 * gg);
+      vv = fmaf(beta2, vv, c2 * gg * gg);
+      pp -= step * mm / (sqrtf(vv) * inv_sqrt_bc2 + eps);
+    };
+    const long long v_lo = sg.lo >> 2, v_hi = sg.hi >> 2;          // float4 range of the segment
+    const long long k0 = (long long)(c - sg.chunk0) * MMFM_ADAMW_CHUNK4;
+    if (k0 < 0 || (k0 > 0 && v_lo + k0 >= v_hi)) continue;   // a chunk past the segment's end (malformed table)
+    const long long i0 = v_lo + k0, i1 = min(v_hi, i0 + MMFM_ADAMW_CHUNK4);
+    for (long long i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+      float4 Pv = reinterpret_cast<float4*>(p)[i], M = reinterpret_cast<float4*>(m)[i], V = reinterpret_cast<float4*>(v)[i];
+      const float4 G = reinterpret_cast<const float4*>(g)[i];
+      upd(Pv.x, G.x, M.x, V.x); upd(Pv.y, G.y, M.y, V.y); upd(Pv.z, G.z, M.z, V.z); upd(Pv.w, G.w, M.w, V.w);
+      reinterpret_cast<float4*>(p)[i] = Pv;
+      reinterpret_cast<float4*>(m)[i] = M;
+      reinterpret_cast<float4*>(v)[i] = V;
+    }
+    if (i1 == v_hi) {                                               // last chunk: the scalar tail
+      const long long e = (v_hi << 2) + threadIdx.x;
+      if (e < sg.hi) upd(p[e], g[e], m[e], v[e]);
+    }
   }
-  for (long long i = (n4 << 2) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
-    upd(p[i], g[i], m[i], v[i]);
 }
 
 // uint8 spike counts -> fp32 and / or bf16 (SURVEY section 8f rank 2: the loader's counts are small non-negative
@@ -1482,17 +1516,54 @@ extern "C" int mmfm_scale_inplace(float* x, long long n, const float* scale_dev,
   return 0;
 }
 
+static int adamw_class(const mmfm_adamw_class& c, AdamwClass* out) {
+  MMFM_REQUIRE(c.step >= 1, "mmfm_adamw: step must be >= 1");
+  const double bc1 = 1.0 - pow((double)c.beta1, (double)c.step), bc2 = 1.0 - pow((double)c.beta2, (double)c.step);
+  *out = AdamwClass{c.lr, c.beta1, c.beta2, c.eps, c.weight_decay, (float)(1.0 / bc1), (float)(1.0 / sqrt(bc2))};
+  return 0;
+}
+
+static int adamw_launch(float* p, const float* g, float* exp_avg, float* exp_avg_sq, AdamwParams& P, void* stream) {
+  MMFM_REQUIRE(p && g && exp_avg && exp_avg_sq && P.n > 0, "mmfm_adamw: bad arguments");
+  MMFM_REQUIRE((((uintptr_t)p | (uintptr_t)g | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0,
+               "mmfm_adamw: buffers must be 16-byte aligned");
+  adamw_kernel<<<ew_grid((long long)P.n_chunks * 256, 256), 256, 0, (cudaStream_t)stream>>>(p, g, exp_avg, exp_avg_sq, P);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
 extern "C" int mmfm_adamw_step(float* p, const float* g, float* exp_avg, float* exp_avg_sq, long long n, float lr,
                                float beta1, float beta2, float eps, float weight_decay, long long step, void* stream) {
   MMFM_REQUIRE(p && g && exp_avg && exp_avg_sq && n > 0 && step >= 1, "mmfm_adamw_step: bad arguments");
-  MMFM_REQUIRE((((uintptr_t)p | (uintptr_t)g | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0,
-               "mmfm_adamw_step: buffers must be 16-byte aligned");
-  const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
-  adamw_kernel<<<ew_grid(n / 4 + 1, 256), 256, 0, (cudaStream_t)stream>>>(p, g, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps,
-                                                                         weight_decay, (float)(1.0 / bc1),
-                                                                         (float)(1.0 / sqrt(bc2)));
-  MMFM_CHECK_CUDA(cudaGetLastError());
-  return 0;
+  AdamwParams P{};
+  const long long chunks = ((n >> 2) + MMFM_ADAMW_CHUNK4 - 1) / MMFM_ADAMW_CHUNK4;
+  MMFM_REQUIRE(chunks < (1LL << 31), "mmfm_adamw_step: n too large");
+  P.segs = nullptr;
+  P.one = mmfm_adamw_seg{0, n, 0, 0};
+  P.n_segs = 1;
+  P.n_chunks = chunks > 0 ? (int)chunks : 1;
+  P.n_classes = 1;
+  P.n = n;
+  if (adamw_class(mmfm_adamw_class{lr, beta1, beta2, eps, weight_decay, 0, step}, &P.cls[0]) != 0) return -1;
+  return adamw_launch(p, g, exp_avg, exp_avg_sq, P, stream);
+}
+
+extern "C" int mmfm_adamw_multi(float* p, const float* g, float* exp_avg, float* exp_avg_sq, long long n,
+                                const mmfm_adamw_seg* segs_dev, int n_segs, int n_chunks,
+                                const mmfm_adamw_class* classes, int n_classes, void* stream) {
+  MMFM_REQUIRE(segs_dev && classes, "mmfm_adamw_multi: null pointer");
+  MMFM_REQUIRE(n_segs >= 1 && n_chunks >= n_segs, "mmfm_adamw_multi: bad segment count");
+  MMFM_REQUIRE(n_classes >= 1 && n_classes <= MMFM_ADAMW_MAX_CLASSES,
+               "mmfm_adamw_multi: n_classes must be in [1, MMFM_ADAMW_MAX_CLASSES]");
+  AdamwParams P{};
+  P.segs = segs_dev;
+  P.n_segs = n_segs;
+  P.n_chunks = n_chunks;
+  P.n_classes = n_classes;
+  P.n = n;
+  for (int i = 0; i < n_classes; ++i)
+    if (adamw_class(classes[i], &P.cls[i]) != 0) return -1;
+  return adamw_launch(p, g, exp_avg, exp_avg_sq, P, stream);
 }
 
 extern "C" int mmfm_u8_expand(const unsigned char* x, long long R, int C, float* y32, long long ld32, void* y16,

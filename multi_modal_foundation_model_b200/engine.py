@@ -118,6 +118,7 @@ class ParamStore:
         self.grad = torch.zeros(off, device=device, dtype=torch.float32)
         self.params = {n: named[n] for n in self.offset}
         self.bucket_order = [n for n in order if self.alias[n] == n]
+        self._grad_views: Optional[Dict[str, torch.Tensor]] = None
         self.adopt()
 
     @staticmethod
@@ -178,6 +179,13 @@ class ParamStore:
 
     def g(self, name: str) -> torch.Tensor:
         return self.view(self.grad, name)
+
+    def grad_views(self) -> Dict[str, torch.Tensor]:
+        """One gradient view per parameter, the same objects every call: engine.backward installs them as
+        ``Parameter.grad`` and optim.AdamW recognises them by identity."""
+        if self._grad_views is None:
+            self._grad_views = {n: self.g(n) for n in self.params}
+        return self._grad_views
 
     def adopted(self) -> bool:
         for n in (self.bucket_order[0], self.bucket_order[-1]):
@@ -375,6 +383,12 @@ class Plan:
         self._g_fwd = self._g_bwd = None
         self._n_fwd_runs = self._n_bwd_runs = 0
         self.fwd_calls, self.bwd_calls = rec_f.calls, rec_b.calls
+        # frozen parameters: the wgrad launches that write only frozen parameters are left out of the backward; one
+        # call list (and captured graph) per such set, derived from the recorded one (same buffers, same plan)
+        params = eng.store.params
+        self._wgrad_params = [(ci, tuple(params[n] for n in names)) for ci, names in self.wgrad_writes]
+        self._skip_of: Dict[Tuple[bool, ...], Tuple[int, ...]] = {}
+        self._variants: Dict[Tuple[int, ...], Dict[str, Any]] = {}
         self._keep += rec_f.keep + rec_b.keep
         if self.det_ws is not None:
             self.det_ws.materialize(dev)
@@ -616,6 +630,7 @@ class Plan:
         self.delta = f32(B, max(hp["enc_heads"], hp["dec_heads"]), S)
         ddec = b16(R, H)                                       # gradient wrt decoder_norm output (modality-major)
         self.grad_marks: List[Tuple[int, int]] = []           # (calls issued, flat-gradient offset that is final)
+        self.wgrad_writes: List[Tuple[int, Tuple[str, ...]]] = []   # (wgrad call index, parameters it writes)
 
         def mark(next_param: Optional[str]):
             rec = ops._REC
@@ -628,8 +643,11 @@ class Plan:
             if dX is not None:
                 ops.gemm_tn(dY, sh.tr[shadow_key], dX, act=act, aux=aux, act_scale=act_scale, **extra)
             bn = bnames or [wname + ".bias"]
-            ops.gemm_wgrad(dY, X, self._wgrad_dst(wnames or [wname + ".weight"]),
-                           dbias=self._bias(bn, "g") if st.has(bn[0]) else None, ws=self.det_ws)
+            wn = wnames or [wname + ".weight"]
+            ops.gemm_wgrad(dY, X, self._wgrad_dst(wn), dbias=self._bias(bn, "g") if st.has(bn[0]) else None,
+                           ws=self.det_ws)
+            writes = wn + ([st.alias[n] for n in bn] if st.has(bn[0]) else [])
+            self.wgrad_writes.append((len(ops._REC.calls) - 1, tuple(writes)))
 
         def mlp_bwd(pre, x_in, ln_name, Gs, inter, dxb, drop_prev):
             duv = du[:, :inter]
@@ -813,9 +831,30 @@ class Plan:
             self.sample_thresh.copy_(self._thresh_host, non_blocking=True)
             self._thresh_cur = list(thresh)
 
-    def _bwd_body(self):
+    def backward_schedule(self) -> Tuple[Tuple[int, ...], List[Any], List[Tuple[int, int]]]:
+        """(skipped wgrad call indices, backward call list, gradient marks) for the parameters' current requires_grad
+        flags.  A wgrad launch is skipped when every parameter it writes is frozen; its gradient range stays zero.  The
+        marks keep their flat-gradient offsets (so data-parallel buckets are unchanged) with call indices counted in
+        the filtered list.  Nothing frozen: the recorded list itself."""
+        rg = tuple(p.requires_grad for p in self.eng.store.params.values())
+        skip = self._skip_of.get(rg)
+        if skip is None:
+            skip = self._skip_of[rg] = tuple(ci for ci, ps in self._wgrad_params
+                                             if not any(p.requires_grad for p in ps))
+        if not skip:
+            return skip, self.bwd_calls, self.grad_marks
+        v = self._variants.get(skip)
+        if v is None:
+            drop = set(skip)
+            kept_before = np.cumsum([0] + [i not in drop for i in range(len(self.bwd_calls))])
+            v = self._variants[skip] = {
+                "calls": [c for i, c in enumerate(self.bwd_calls) if i not in drop],
+                "marks": [(int(kept_before[ci]), off) for ci, off in self.grad_marks], "graph": None, "runs": 0}
+        return skip, v["calls"], v["marks"]
+
+    def _bwd_body(self, calls=None):
         self.eng.store.grad.zero_()
-        ops.run_recorded(self.bwd_calls)
+        ops.run_recorded(self.bwd_calls if calls is None else calls)
 
     def _capture(self, body):
         g = torch.cuda.CUDAGraph()
@@ -834,7 +873,19 @@ class Plan:
         self._dpreds_dirty = False
 
     def run_backward(self):
-        """Zeroes the flat gradient buffer and runs the backward schedule."""
+        """Zeroes the flat gradient buffer and runs the backward schedule (without the wgrad launches of frozen
+        parameters)."""
+        skip, calls, _ = self.backward_schedule()
+        if skip:
+            v = self._variants[skip]
+            if self.eng.use_graphs and v["graph"] is None and v["runs"] >= 1:
+                v["graph"] = self._capture(lambda: self._bwd_body(calls))
+            v["runs"] += 1
+            if v["graph"] is not None:
+                v["graph"].replay()
+            else:
+                self._bwd_body(calls)
+            return
         if self.eng.use_graphs and self._g_bwd is None and self._n_bwd_runs >= 1:
             self._g_bwd = self._capture(self._bwd_body)
         self._n_bwd_runs += 1
@@ -940,7 +991,6 @@ class Engine:
         self.fuse_attn_prep = (_os.environ.get("MMFM_FUSE_ATTN_PREP", "1") != "0" and self.H > 64 and self.H % 32 == 0
                                and _os.environ.get("MMFM_GEMM_TS", "1") != "0")
         self.last_plan: Optional[Plan] = None
-        self._grad_views = None
         from .model import MultiModalOutput
         self.output_cls = MultiModalOutput      # dropin.install() swaps in the reference's own dataclass
 
@@ -1123,9 +1173,7 @@ class Engine:
             pl.run_backward()
         if prev is not None:
             st.grad.add_(prev)
-        gv = self._grad_views
-        if gv is None:
-            gv = self._grad_views = {n: st.g(n) for n in st.params}
+        gv = st.grad_views()
         for n, p in st.params.items():
             if p.grad is not gv[n] and p.requires_grad:
                 p.grad = gv[n]

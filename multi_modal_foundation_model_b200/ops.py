@@ -271,6 +271,16 @@ def adamw_step(p: torch.Tensor, g: torch.Tensor, exp_avg: torch.Tensor, exp_avg_
             float(beta1), float(beta2), float(eps), float(weight_decay), int(step), meta={"bytes": 28.0 * n})
 
 
+def adamw_multi(p: torch.Tensor, g: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor,
+                segs_dev: torch.Tensor, n_segs: int, n_chunks: int, classes, n_elems: int) -> None:
+    """AdamW over the segments of an uploaded table (``segs_dev``: bytes of ``_lib.AdamwSeg[n_segs]`` on the device),
+    one ``_lib.AdamwClass`` per class; ``n_elems`` = elements the segments cover (traffic accounting only)."""
+    arr = (_lib.AdamwClass * len(classes))(*classes)
+    _launch("mmfm_adamw_multi", p.data_ptr(), g.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), p.numel(),
+            segs_dev.data_ptr(), int(n_segs), int(n_chunks), arr, len(classes), keep=(arr,),
+            meta={"bytes": 28.0 * n_elems})
+
+
 def layernorm_fwd(x, gamma, beta, y, mean, rstd, *, R: int, H: int, eps: float = 1e-5, modmajor_T: int = 0,
                   S: int = 0) -> None:
     _launch("mmfm_layernorm_fwd", x.data_ptr(), gamma.data_ptr(), beta.data_ptr(), y.data_ptr(), mean.data_ptr(),

@@ -90,28 +90,32 @@ class DataParallel:
         torch.cuda.synchronize()
 
     def _segments(self, pl):
+        """(skipped wgrad calls, (backward call list, n_calls, buckets, tail)) for the plan's current frozen set
+        (engine.Plan.backward_schedule)."""
+        skip, calls, grad_marks = pl.backward_schedule()
         # cached on the plan object itself (an id()-keyed table could hand a new plan the entry of a freed one)
-        seg = getattr(pl, "_ddp_segments", None)
+        cache = pl.__dict__.setdefault("_ddp_segments", {})
+        seg = cache.get(skip)
         if seg is None:
-            calls = pl.bwd_calls
             # the whole-buffer scale right after the last mark is replaced by per-bucket scaling before each
             # all-reduce; calls after it (input gradients, no parameter gradient) run once the buckets are enqueued
-            n_calls = pl.grad_marks[-1][0] if pl.grad_marks else len(calls)
+            n_calls = grad_marks[-1][0] if grad_marks else len(calls)
             tail = n_calls + 1 if n_calls < len(calls) and calls[n_calls][2] == "mmfm_scale_inplace" else n_calls
-            marks = [(min(ci, n_calls), off) for ci, off in pl.grad_marks]
+            marks = [(min(ci, n_calls), off) for ci, off in grad_marks]
             buckets = plan_buckets(marks, self.eng.store.total, self.bucket_elems)
-            seg = (n_calls, buckets, tail)
-            pl._ddp_segments = seg
-        return seg
+            seg = cache[skip] = (calls, n_calls, buckets, tail)
+        return skip, seg
 
     def run_backward(self, pl) -> None:
         """Backward schedule with the bucket all-reduces enqueued at their completion marks.  The first call per plan
         runs eagerly (NCCL communicator set-up, kernel attributes); afterwards the whole sequence -- kernels, per-bucket
         scaling and the NCCL all-reduces on their side stream -- is captured once into a CUDA graph and replayed, so the
         multi-GPU step has the same launch-gap-free backward as the single-GPU one."""
-        st = getattr(pl, "_ddp_graph", None)
+        skip, _ = self._segments(pl)
+        graphs = pl.__dict__.setdefault("_ddp_graph", {})       # one per frozen set
+        st = graphs.get(skip)
         if st is None:
-            st = pl._ddp_graph = {"runs": 0, "graph": None}
+            st = graphs[skip] = {"runs": 0, "graph": None}
             self._graphs.append(st)
         if self.eng.use_graphs and self.graph_ddp and st["graph"] is None and st["runs"] >= 1 and self.world > 1:
             try:
@@ -132,22 +136,22 @@ class DataParallel:
 
     def _run_backward_eager(self, pl) -> None:
         from . import ops
-        n_calls, buckets, tail = self._segments(pl)
+        _, (calls, n_calls, buckets, tail) = self._segments(pl)
         grad = self.eng.store.grad
         grad.zero_()
         works = []
         done = 0
         for ci, lo, hi in buckets:
             if ci > done:
-                ops.run_recorded(pl.bwd_calls[done:ci])
+                ops.run_recorded(calls[done:ci])
                 done = ci
             view = grad[lo:hi]
             ops.scale_inplace(view, pl.gscale)
             if self.world > 1:
                 works.append(all_reduce_mean(view, self.pg, async_op=True))
         assert done == n_calls, "bucket plan must end at the end of the backward schedule"
-        if tail < len(pl.bwd_calls):
-            ops.run_recorded(pl.bwd_calls[tail:])
+        if tail < len(calls):
+            ops.run_recorded(calls[tail:])
         for w in works:
             if w is not None:
                 w.wait()
