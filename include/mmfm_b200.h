@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define MMFM_ABI_VERSION 7
+#define MMFM_ABI_VERSION 8
 
 const char* mmfm_last_error(void);
 int mmfm_abi_version(void);
@@ -275,6 +275,17 @@ int mmfm_cast_bf16_multi(const mmfm_cast_item* items_dev, int n_items, int total
 /* x[0..n) *= scale_dev[0]; returns at once on the device when the scale is exactly 1 (upstream gradient of the
  * scalar loss, trainer/base.py:195 always passes 1) */
 int mmfm_scale_inplace(float* x, long long n, const float* scale_dev, void* stream);
+
+/* ---- data-parallel multi-session step (ABI 8): each rank runs its own session and all-gathers its session id and
+ *      that session's gradient slab; this kernel writes the rank mean of every session some rank ran ------------- */
+/* gathered: fp32 [world, slab_stride], row r = the slab of rank r.  ids_dev: int32 [world], the session of each row.
+ * ranges_dev: int64 [n_sessions][4] = (lo0, hi0, lo1, hi1), two element ranges of `grad`; a session's slab is
+ * grad[lo0, hi0) followed by grad[lo1, hi1), and must fit in slab_stride (a session whose entry does not is skipped).
+ * For every distinct session s in ids, grad over its ranges = inv_world * (sum over the rows r with ids[r] == s, in
+ * ascending r, from 0.0f).  One CTA row, that of the first row carrying s, writes s: no atomics, the same bits on every
+ * rank and from run to run.  Ranges of sessions absent from ids, and ids outside [0, n_sessions), are not touched. */
+int mmfm_session_grad_combine(float* grad, const float* gathered, int world, long long slab_stride, const int* ids_dev,
+                              const long long* ranges_dev, int n_sessions, float inv_world, void* stream);
 
 /* ---- batch wire format (SURVEY section 8f rank 2: spike counts are small non-negative integers, stored as ubyte by
  *      the reference's datasets, dataset_utils.py:29; the dense fp32 (B,T,N) batch of loader/base.py:436-450 can be

@@ -20,7 +20,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
               "-Xptxas", "-v"]
 
 MAX_MOD = 8
-ABI_VERSION = 7
+ABI_VERSION = 8
 MASK_SITE = 8192
 
 
@@ -185,6 +185,7 @@ SIGNATURES = {
     "mmfm_cast_bf16": [_vp, _ll, _vp, _ll, _vp, _ll, _i, _i, _vp],
     "mmfm_cast_bf16_multi": [_vp, _i, _i, _vp],
     "mmfm_scale_inplace": [_vp, _ll, _vp, _vp],
+    "mmfm_session_grad_combine": [_vp, _vp, _i, _ll, _vp, _vp, _i, _f, _vp],
     "mmfm_csr_to_dense_u8": [_vp, _vp, _vp, _ll, _i, _vp, _vp],
     "mmfm_u8_expand": [_vp, _ll, _i, _vp, _ll, _vp, _ll, _vp],
     "mmfm_column_stats": [_vp, _vp, _ll, _i, _i, _vp, _vp],

@@ -1123,6 +1123,53 @@ __global__ void __launch_bounds__(256) scale_inplace_kernel(float* __restrict__ 
     x[i] *= s;
 }
 
+// Data-parallel multi-session step: every rank all-gathered its session id and its session's gradient slab (the
+// session's ranges of the flat gradient, back to back).  Row y of the grid serves gathered slab y; only the first rank
+// carrying a session writes it, as inv_world * (sum over the ranks carrying it, in ascending order, from 0.0f).  No
+// atomics, and every rank computes the same bits.  Sessions no rank carries are neither read nor written.
+__device__ __forceinline__ float4 f4_add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
+
+__global__ void __launch_bounds__(256) session_grad_combine_kernel(float* __restrict__ grad,
+                                                                   const float* __restrict__ gathered, int world,
+                                                                   long long stride, const int* __restrict__ ids,
+                                                                   const long long* __restrict__ ranges, int n_sessions,
+                                                                   float inv_world) {
+  const int r0 = blockIdx.y;
+  const int s = ids[r0];
+  if (s < 0 || s >= n_sessions) return;
+  for (int r = 0; r < r0; ++r)
+    if (ids[r] == s) return;                      // an earlier rank's CTA row writes this session
+  const long long* rg = ranges + 4LL * s;
+  const long long lo0 = rg[0], hi0 = rg[1], lo1 = rg[2], hi1 = rg[3];
+  if (lo0 < 0 || hi0 < lo0 || lo1 < 0 || hi1 < lo1 || (hi0 - lo0) + (hi1 - lo1) > stride) return;   // malformed table
+  const long long step = (long long)gridDim.x * blockDim.x, t0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  long long soff = 0;                             // position of the range inside the slab
+  for (int part = 0; part < 2; ++part) {
+    const long long lo = part ? lo1 : lo0, n = (part ? hi1 : hi0) - lo;
+    float* dst = grad + lo;
+    const float* src = gathered + soff;
+    long long done = 0;
+    if (((lo | soff | stride) & 3) == 0 && (((uintptr_t)grad | (uintptr_t)gathered) & 15) == 0) {
+      const long long n4 = n >> 2;
+      for (long long i = t0; i < n4; i += step) {
+        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int r = r0; r < world; ++r)
+          if (ids[r] == s) acc = f4_add(acc, __ldg(reinterpret_cast<const float4*>(src + r * stride) + i));
+        reinterpret_cast<float4*>(dst)[i] = make_float4(acc.x * inv_world, acc.y * inv_world, acc.z * inv_world,
+                                                        acc.w * inv_world);
+      }
+      done = n4 << 2;
+    }
+    for (long long i = done + t0; i < n; i += step) {
+      float acc = 0.f;
+      for (int r = r0; r < world; ++r)
+        if (ids[r] == s) acc += __ldg(src + r * stride + i);
+      dst[i] = acc * inv_world;
+    }
+    soff += n;
+  }
+}
+
 // Fused multi-tensor AdamW over the flat master-parameter / gradient buffers (torch.optim.AdamW semantics,
 // reference train_multi_modal.py:197-202): p *= 1 - lr*wd ; m = b1 m + (1-b1) g ; v = b2 v + (1-b2) g^2 ;
 // p -= (lr / bc1) * m / (sqrt(v) / sqrt(bc2) + eps).  One pass, 28 bytes of traffic per parameter.
@@ -1512,6 +1559,20 @@ extern "C" int mmfm_scale_inplace(float* x, long long n, const float* scale_dev,
   MMFM_REQUIRE(x && scale_dev && n > 0, "mmfm_scale_inplace: bad arguments");
   MMFM_REQUIRE(((uintptr_t)x & 15) == 0, "mmfm_scale_inplace: buffer must be 16-byte aligned");
   scale_inplace_kernel<<<ew_grid(n / 4 + 1, 256), 256, 0, (cudaStream_t)stream>>>(x, n, scale_dev);
+  MMFM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int mmfm_session_grad_combine(float* grad, const float* gathered, int world, long long slab_stride,
+                                         const int* ids_dev, const long long* ranges_dev, int n_sessions,
+                                         float inv_world, void* stream) {
+  MMFM_REQUIRE(grad && gathered && ids_dev && ranges_dev, "mmfm_session_grad_combine: null pointer");
+  MMFM_REQUIRE(world >= 1 && world <= 65535, "mmfm_session_grad_combine: world=%d outside [1, 65535]", world);
+  MMFM_REQUIRE(slab_stride >= 1 && n_sessions >= 1, "mmfm_session_grad_combine: bad slab stride or session count");
+  MMFM_REQUIRE(isfinite(inv_world), "mmfm_session_grad_combine: inv_world must be finite");
+  const dim3 grid(ew_grid((slab_stride + 3) / 4, 256), world);
+  session_grad_combine_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(grad, gathered, world, slab_stride, ids_dev,
+                                                                       ranges_dev, n_sessions, inv_world);
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

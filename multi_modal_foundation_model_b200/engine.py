@@ -86,6 +86,65 @@ def fuse_context_norms(named, n_dec: int) -> bool:
     return H in (128, 256, 512) and (H // 128) * n_dec <= 12
 
 
+def flat_layout(order: Sequence[str], named) -> Tuple[Dict[str, str], Dict[str, int], Dict[str, torch.Size], int]:
+    """(alias, offset, shape, total) of the flat buffers: parameters in ``order``, each at a 64-element aligned offset;
+    a parameter met again under another name (shared mod_emb) is an alias of the first name."""
+    uniq: Dict[int, str] = {}
+    alias: Dict[str, str] = {}
+    offset: Dict[str, int] = {}
+    shape: Dict[str, torch.Size] = {}
+    off = 0
+    for name in order:
+        p = named[name]
+        if id(p) in uniq:
+            alias[name] = uniq[id(p)]
+            continue
+        uniq[id(p)] = name
+        alias[name] = name
+        offset[name] = off
+        shape[name] = p.shape
+        off += _pad(p.numel(), 64)
+    return alias, offset, shape, off
+
+
+def session_ranges(offset: Dict[str, int], shape: Dict[str, torch.Size], prefixes: Sequence[str]
+                   ) -> Tuple[Tuple[int, int], List[Tuple[int, int, int, int]]]:
+    """((core_lo, core_hi), [(head_lo, head_hi, emb_lo, emb_hi)] per session prefix) of a multi-session flat layout.
+
+    A session's heads are its ``decoder_embeddings.<m>.out`` parameters, its embedders the rest of its prefix; the shared
+    core is every parameter outside all prefixes.  Each range covers its parameters and their pads exactly, starts and
+    ends on the 64-element pad (16-byte aligned), and no session range overlaps the core or another session's."""
+    def span(names, what):
+        names = sorted(names, key=offset.__getitem__)
+        if not names:
+            raise MmfmError(f"empty {what} range")
+        lo = offset[names[0]]
+        hi = lo
+        for n in names:       # contiguous: each parameter starts where the previous one's pad ends
+            if offset[n] != hi:
+                raise MmfmError(f"{what} range is not contiguous at {n}")
+            hi += _pad(shape[n].numel(), 64)
+        assert lo % 64 == 0 and hi % 64 == 0
+        return lo, hi
+
+    owned = set()
+    out = []
+    for prefix in prefixes:
+        mine = [n for n in offset if n.startswith(prefix)]
+        parts = {n: n[len(prefix):].split(".") for n in mine}        # decoder_embeddings.<m>.out.<weight|bias>
+        heads = [n for n in mine if parts[n][0] == "decoder_embeddings" and parts[n][2] == "out"]
+        h = span(heads, f"{prefix} head")
+        e = span([n for n in mine if n not in heads], f"{prefix} embedder")
+        out.append(h + e)
+        owned.update(mine)
+    core = span([n for n in offset if n not in owned], "shared core")
+    spans = sorted([(lo, hi) for r in out for lo, hi in (r[:2], r[2:])] + [core])
+    for (_, hi0), (lo1, _) in zip(spans, spans[1:]):
+        if lo1 < hi0:
+            raise MmfmError("session ranges overlap each other or the shared core")
+    return core, out
+
+
 # ------------------------------------------------------------------------------------------------------------
 class ParamStore:
     """Flat fp32 master-parameter and gradient buffers + bf16 shadows."""
@@ -95,25 +154,19 @@ class ParamStore:
         self.device = device
         named = dict(model.named_parameters(remove_duplicate=False))
         order = self._execution_reverse_order(model, named)
-        uniq: Dict[int, str] = {}
-        self.alias: Dict[str, str] = {}          # name -> canonical name (shared mod_emb)
-        self.offset: Dict[str, int] = {}
-        self.shape: Dict[str, torch.Size] = {}
-        off = 0
-        for name in order:
-            p = named[name]
-            if id(p) in uniq:
-                self.alias[name] = uniq[id(p)]
-                continue
-            uniq[id(p)] = name
-            self.alias[name] = name
-            self.offset[name] = off
-            self.shape[name] = p.shape
-            off += _pad(p.numel(), 64)
+        # alias: name -> canonical name (shared mod_emb)
+        self.alias, self.offset, self.shape, off = flat_layout(order, named)
         missing = set(named) - set(order)
         if missing:
             raise MmfmError(f"parameters outside the step schedule: {sorted(missing)[:5]} ...")
         self.total = off
+        # multi-session model: the shared core's range and, per session (in embedding_groups order), its head and
+        # embedder ranges (the data-parallel session exchange); None for the single-session model
+        self.core_range: Optional[Tuple[int, int]] = None
+        self.session_ranges: Optional[List[Tuple[int, int, int, int]]] = None
+        if getattr(model, "session_embeddings", None) is not None:
+            self.core_range, self.session_ranges = session_ranges(
+                self.offset, self.shape, [prefix for prefix, _, _ in embedding_groups(model)])
         self.flat = torch.zeros(off, device=device, dtype=torch.float32)
         self.grad = torch.zeros(off, device=device, dtype=torch.float32)
         self.params = {n: named[n] for n in self.offset}
@@ -310,6 +363,10 @@ class Plan:
             arena.reset()
         self.prefix, self.mods = eng.sessions[session]
         dev = eng.device
+        # the session's index in eng.sessions (= in store.session_ranges), also as an int32 device scalar: the id this
+        # plan contributes to the data-parallel session exchange
+        self.session_index = list(eng.sessions).index(session)
+        self.session_id = torch.tensor([self.session_index], device=dev, dtype=torch.int32)
         mods, T, H = self.mods, eng.T, eng.H
         S = T * len(mods)
         R, BT = B * S, B * T

@@ -239,6 +239,19 @@ def scale_inplace(x: torch.Tensor, scale_dev: torch.Tensor) -> None:
     _launch("mmfm_scale_inplace", x.data_ptr(), x.numel(), scale_dev.data_ptr())
 
 
+def session_grad_combine(grad: torch.Tensor, gathered: torch.Tensor, ids: torch.Tensor, ranges: torch.Tensor,
+                         inv_world: float) -> None:
+    """grad over the ranges of every session in ``ids`` = inv_world * the rank-ordered sum of the gathered slabs that
+    carry it (include/mmfm_b200.h).  gathered fp32 [world, L], ids int32 [world], ranges int64 [n_sessions, 4]."""
+    assert grad.dtype == torch.float32 and grad.is_contiguous()
+    assert gathered.dtype == torch.float32 and gathered.dim() == 2 and gathered.stride(1) == 1
+    assert ids.dtype == torch.int32 and ids.numel() == gathered.shape[0]
+    assert ranges.dtype == torch.int64 and ranges.is_contiguous() and ranges.dim() == 2 and ranges.shape[1] == 4
+    _launch("mmfm_session_grad_combine", grad.data_ptr(), gathered.data_ptr(), gathered.shape[0], gathered.stride(0),
+            ids.data_ptr(), ranges.data_ptr(), ranges.shape[0], float(inv_world),
+            meta={"bytes": float(gathered.numel()) * 4})
+
+
 def csr_to_dense_u8(data: torch.Tensor, indices: torch.Tensor, row_ptr: torch.Tensor, out: torch.Tensor, *,
                     n_rows: int, n_cols: int) -> None:
     assert out.dtype == torch.uint8 and out.is_contiguous() and out.numel() == n_rows * n_cols

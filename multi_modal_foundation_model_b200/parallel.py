@@ -42,6 +42,16 @@ def plan_buckets(marks: Sequence[Tuple[int, int]], total: int, target_elems: int
     return out
 
 
+def core_buckets(marks: Sequence[Tuple[int, int]], core: Tuple[int, int], target_elems: int
+                 ) -> List[Tuple[int, int, int]]:
+    """plan_buckets over the shared core [lo, hi) of a multi-session flat gradient only: the marks clipped to that
+    span.  The core parameters and their marks' offsets are the same for every session, so every session's plan
+    gets the same ranges (its call indices may differ)."""
+    lo, hi = core
+    clipped = [(ci, min(max(off, lo), hi) - lo) for ci, off in marks]
+    return [(ci, a + lo, b + lo) for ci, a, b in plan_buckets(clipped, hi - lo, target_elems)]
+
+
 def all_reduce_mean(t: torch.Tensor, group=None, async_op: bool = False):
     """Mean over ranks, in place (DDP semantics).  NCCL averages inside the collective; gloo (CPU tests) sums and
     divides."""
@@ -52,9 +62,70 @@ def all_reduce_mean(t: torch.Tensor, group=None, async_op: bool = False):
     return w
 
 
+class SessionExchange:
+    """Session gradients of a multi-session model under data parallelism, where every rank may run another session.
+
+    Only the shared core goes through the all-reduce buckets.  A rank's own session gradient (its head range and its
+    embedder range of the flat gradient) travels as two fixed-size all-gathers instead: the head slab, padded to the
+    widest session's head range, and the embedder slab, padded likewise; the session ids travel with the head slab.
+    The sizes depend on the engine only, so every rank issues the same collectives with the same counts in the same
+    order, whichever session it ran, and plans of different sessions can be captured and replayed side by side.
+    mmfm_session_grad_combine then writes, on every rank alike, the rank mean of each session some rank ran; the
+    ranges of the other sessions keep the zero the backward left there."""
+
+    def __init__(self, store, world: int, group=None):
+        dev = store.device
+        self.world, self.pg = world, group
+        self.ranges = store.session_ranges
+        self.head_len = max(h1 - h0 for h0, h1, _, _ in self.ranges)
+        self.emb_len = max(e1 - e0 for _, _, e0, e1 in self.ranges)
+        # the combine kernel's range tables: one range per session each (the second one empty)
+        self.head_tab = torch.tensor([[h0, h1, 0, 0] for h0, h1, _, _ in self.ranges], dtype=torch.int64, device=dev)
+        self.emb_tab = torch.tensor([[e0, e1, 0, 0] for _, _, e0, e1 in self.ranges], dtype=torch.int64, device=dev)
+        self.ids = torch.zeros(world, dtype=torch.int32, device=dev)
+        self.send_head = torch.zeros(self.head_len, device=dev)
+        self.send_emb = torch.zeros(self.emb_len, device=dev)
+        self.recv_head = torch.zeros(world, self.head_len, device=dev)
+        self.recv_emb = torch.zeros(world, self.emb_len, device=dev)
+
+    def bytes_per_step(self) -> Tuple[int, int]:
+        """(sent, received) bytes of one rank's session exchange per step (ids included)."""
+        n = 4 * (1 + self.head_len + self.emb_len)
+        return n, n * self.world
+
+    def _send(self, pl, grad: torch.Tensor, lo: int, hi: int, send: torch.Tensor, recv: torch.Tensor):
+        from . import ops
+        ops.scale_inplace(grad[lo:hi], pl.gscale)
+        send[:hi - lo].copy_(grad[lo:hi])                 # cudaMemcpyAsync; the pad past hi - lo is never read
+        return dist.all_gather_into_tensor(recv.view(-1), send, group=self.pg, async_op=True)
+
+    def send_heads(self, pl, grad: torch.Tensor) -> list:
+        """Enqueued once the head wgrads are done: the ids and the head slab."""
+        h0, h1, _, _ = self.ranges[pl.session_index]
+        return [dist.all_gather_into_tensor(self.ids, pl.session_id, group=self.pg, async_op=True),
+                self._send(pl, grad, h0, h1, self.send_head, self.recv_head)]
+
+    def send_embedders(self, pl, grad: torch.Tensor) -> list:
+        """Enqueued after the last embedder launch: the embedder slab."""
+        _, _, e0, e1 = self.ranges[pl.session_index]
+        return [self._send(pl, grad, e0, e1, self.send_emb, self.recv_emb)]
+
+    def combine(self, grad: torch.Tensor) -> None:
+        """After the gathers are waited for: every ran session's ranges = the rank mean of its gathered slabs."""
+        from . import ops
+        ops.session_grad_combine(grad, self.recv_head, self.ids, self.head_tab, 1.0 / self.world)
+        ops.session_grad_combine(grad, self.recv_emb, self.ids, self.emb_tab, 1.0 / self.world)
+
+
 class DataParallel:
     """Attach to a ``MultiModal`` (B200 path) so that ``loss.backward()`` leaves rank-averaged gradients in
-    ``Parameter.grad`` -- DDP semantics (mean over ranks of the per-rank gradients, SURVEY.md section 8e)."""
+    ``Parameter.grad`` -- DDP semantics (mean over ranks of the per-rank gradients, SURVEY.md section 8e).
+
+    A ``MultiSessionMultiModal`` rank may feed any session in any step: the shared core is all-reduced in buckets and
+    the session gradients go through a SessionExchange, so each session's gradient is the sum of the gradients of the
+    ranks that ran it, over the world size, and a session no rank ran stays zero."""
+
+    xchg: Optional[SessionExchange] = None       # set for a multi-session model on more than one rank
 
     def __init__(self, model, process_group=None, bucket_mb: float = 8.0, broadcast: bool = True):
         self.model = model
@@ -65,6 +136,8 @@ class DataParallel:
         eng = model.engine()
         eng.ddp = self
         self.eng = eng
+        multi = eng.store.session_ranges is not None and self.world > 1
+        self.xchg = SessionExchange(eng.store, self.world, process_group) if multi else None
         if broadcast and self.world > 1:
             dist.broadcast(eng.store.flat, src=0, group=process_group)   # same initial weights on every rank
         self._graphs = []            # per-plan capture states (held here only so close() can drop the graphs)
@@ -102,7 +175,10 @@ class DataParallel:
             n_calls = grad_marks[-1][0] if grad_marks else len(calls)
             tail = n_calls + 1 if n_calls < len(calls) and calls[n_calls][2] == "mmfm_scale_inplace" else n_calls
             marks = [(min(ci, n_calls), off) for ci, off in grad_marks]
-            buckets = plan_buckets(marks, self.eng.store.total, self.bucket_elems)
+            if self.xchg is None:
+                buckets = plan_buckets(marks, self.eng.store.total, self.bucket_elems)
+            else:
+                buckets = core_buckets(marks, self.eng.store.core_range, self.bucket_elems)
             seg = cache[skip] = (calls, n_calls, buckets, tail)
         return skip, seg
 
@@ -141,6 +217,12 @@ class DataParallel:
         grad.zero_()
         works = []
         done = 0
+        xchg = self.xchg
+        if xchg is not None:
+            # at the first gradient mark, after the last decoder layer: the heads are final from there on
+            done = min(pl.backward_schedule()[2][0][0], n_calls)
+            ops.run_recorded(calls[:done])
+            works += xchg.send_heads(pl, grad)
         for ci, lo, hi in buckets:
             if ci > done:
                 ops.run_recorded(calls[done:ci])
@@ -150,8 +232,12 @@ class DataParallel:
             if self.world > 1:
                 works.append(all_reduce_mean(view, self.pg, async_op=True))
         assert done == n_calls, "bucket plan must end at the end of the backward schedule"
+        if xchg is not None:       # right behind the last core bucket, after the last embedder launch
+            works += xchg.send_embedders(pl, grad)
         if tail < len(calls):
             ops.run_recorded(calls[tail:])
         for w in works:
             if w is not None:
                 w.wait()
+        if xchg is not None:
+            xchg.combine(grad)
