@@ -15,7 +15,7 @@ _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 _CSRC = os.path.join(_PKG_DIR, "csrc")
 # MMFM_LIB_PATH: load another build of the library (A/B measurements of a kernel change against a saved build)
 LIB_PATH = os.environ.get("MMFM_LIB_PATH") or os.path.join(_PKG_DIR, "libmmfm_b200.so")
-SOURCES = ["host_util.cu", "gemm.cu", "gemm_ts.cu", "norm.cu", "attention.cu", "attention_pipe.cu", "attention_bwd_stream.cu", "attention_bwd_persist.cu", "attention_bwd_ws.cu", "glue.cu"]
+SOURCES = ["host_util.cu", "gemm.cu", "gemm_ts.cu", "norm.cu", "attention.cu", "attention_pipe.cu", "attention_bwd_stream.cu", "attention_bwd_ws.cu", "glue.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-Xptxas", "-v"]
 

@@ -22,17 +22,6 @@
 //   bwd dq    rows = queries, cols = keys : dQ += (P * (dP - delta)) K
 //   bwd dkv   rows = keys, cols = queries : dV += P_drop^T dO ; dK += dS^T Q
 #include "attn_common.cuh"
-#include <stdlib.h>
-
-#ifdef MMFM_DBG_TIMING
-__device__ long long g_dbg_t[64];
-#define DBG_T(slot) do { if (blockIdx.x == 3 && blockIdx.y == 100 && threadIdx.x == 64) g_dbg_t[slot] = clock64(); } while (0)
-extern "C" int mmfm_debug_read(long long* out, int n) {
-  return (int)cudaMemcpyFromSymbol(out, g_dbg_t, sizeof(long long) * (n < 64 ? n : 64));
-}
-#else
-#define DBG_T(slot) do { } while (0)
-#endif
 
 namespace mmfm {
 
@@ -762,368 +751,6 @@ __global__ void __launch_bounds__(kAttnThreads, D == 32 ? 3 : 2) attn_bwd_dkv_ke
   }
 }
 
-// ------------------------------------------------------------------------------------------------------------
-// backward, fused + software-pipelined tcgen05 kernel (d_head = 32, Sq, Sk <= 256): ONE CTA per (batch, head) computes
-// dQ, dK and dV, so every score element goes through the softmax / dropout / dS arithmetic once.  This is the
-// non-persistent form of attention_bwd_persist.cu (used when the side data are not 16-byte aligned, Sq % 4 != 0):
-//   pass A  thread = (query row, column group): p = exp2(s*scale - lse) under the mask; P_drop (bf16) -> smem slabs;
-//           p and p*keep stay in registers as packed bf16
-//   pass B  dS = p_drop * dP - p * delta -> smem slabs
-// The slabs are the canonical 128-byte-swizzled layout ([128 query rows] x [64 keys] per slab), written with 16-byte
-// stores from registers, so one copy of dS serves both the dQ (K-major A) and the dK (MN-major A) products.
-// The key range is split into two 128-key halves with their own S / dP buffer in TMEM (columns [0,128) and [128,256))
-// and their own barriers, and the passes run in the order  A(h0) A(h1) B(h0) B(h1) per query tile.  Every MMA batch is issued right after the pass that produces its operands and is waited for one
-// pass later, so the threads never sit on a tensor-pipe round trip:
-//   after A(h):  dP_h = dO V_h^T (over the dead S_h) ; dV_h += P_drop_h^T dO
-//   after B(h):  dQ += dS_h K_h ; dK_h += dS_h^T Q ; S_h of the NEXT query tile
-// Both query tiles' Q / dO are loaded up front; dQ has one accumulator per query tile, so nothing is read out of
-// tensor memory before the end.  TMEM: S/dP 2 x 128 | dQ 2 x 32 | dK 2 x 32 | dV 2 x 32 = 448 columns.
-// ------------------------------------------------------------------------------------------------------------
-template <bool DROP>
-__global__ void __launch_bounds__(kFusedThreads, 1) attn_bwd_fused2_tc_kernel(
-    const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmdO,
-    const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmV, const AttnParams p, int npad) {
-  constexpr int D = 32;
-  constexpr uint32_t kRowBytes = 64, kSbo64 = 512;   // operand tiles: [rows][32 bf16], 64-byte swizzle
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t ld_kv_bar, ld_q_bar[2], s_bar[2], dp_bar[2], done_bar;
-  __shared__ uint32_t tmem_slot;
-  __shared__ uint32_t s_colbits[8];
-
-  DBG_T(0);
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t sK = smem_base, sV = sK + 256 * kRowBytes, sQ = sV + 256 * kRowBytes, sdO = sQ + 256 * kRowBytes;
-  const uint32_t sdS = sdO + 256 * kRowBytes, sPd = sdS + 4 * kSlabBytes;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int quad = warp & 3, grp = warp >> 2;
-  const int h = blockIdx.x, b = blockIdx.y;
-  const int mode = p.mask_mode;
-  const long long bh = (long long)(b * p.nh + h);
-  const int nqt = (p.Sq + 127) >> 7;
-  const int nkh = (npad + 127) >> 7;                 // 128-key halves
-  const int wlast = npad - 128 * (nkh - 1);          // width of the last half (multiple of 16)
-
-  if (tid == 0) {
-    tma_prefetch_desc(&tmQ); tma_prefetch_desc(&tmdO); tma_prefetch_desc(&tmK); tma_prefetch_desc(&tmV);
-    mbar_init(&ld_kv_bar, 1);
-    mbar_init(&ld_q_bar[0], 1); mbar_init(&ld_q_bar[1], 1);
-    mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1);
-    mbar_init(&dp_bar[0], 1); mbar_init(&dp_bar[1], 1);
-    mbar_init(&done_bar, 1);
-    fence_mbar_init();
-    mbar_arrive_expect_tx(&ld_kv_bar, (uint32_t)(2 * npad * kRowBytes));
-    tma_load_2d_addr(sK, &tmK, &ld_kv_bar, h * D, b * p.Sk);
-    tma_load_2d_addr(sV, &tmV, &ld_kv_bar, h * D, b * p.Sk);
-    for (int qt = 0; qt < nqt && qt < 2; ++qt) {
-      mbar_arrive_expect_tx(&ld_q_bar[qt], (uint32_t)(256 * kRowBytes));
-      tma_load_2d_addr(sQ + qt * 128 * kRowBytes, &tmQ, &ld_q_bar[qt], h * D, b * p.Sq + qt * 128);
-      tma_load_2d_addr(sdO + qt * 128 * kRowBytes, &tmdO, &ld_q_bar[qt], h * D, b * p.Sq + qt * 128);
-    }
-  }
-  // per-row side data of both query tiles, requested before anything is waited for (their global-memory latency
-  // overlaps the operand loads and the TMEM allocation)
-  const int row = quad * 32 + lane;
-  const int nch = (npad + 31) >> 5;
-  const int nkb = (p.Sk + kTile - 1) / kTile;
-  float lse_r[2], dl_r[2];
-  uint2 kpre_r[2][2];
-#pragma unroll
-  for (int qt = 0; qt < 2; ++qt) {
-    const int i = qt * 128 + row;
-    const bool ok = i < p.Sq;
-    lse_r[qt] = ok ? p.lse[bh * p.Sq + i] : INFINITY;
-    dl_r[qt] = ok ? p.delta[bh * p.Sq + i] : 0.f;
-#pragma unroll
-    for (int kh = 0; kh < 2; ++kh) {
-      const int c = grp + 4 * kh;
-      kpre_r[qt][kh] = make_uint2(0xFFFFFFFFu, 0xFFFFFFFFu);
-      if (DROP && ok && c < nch) kpre_r[qt][kh] = *reinterpret_cast<const uint2*>(p.p_keep + ((bh * p.Sq + i) * nkb + (c >> 1)) * 4);
-    }
-  }
-  if (warp == 1) {
-    tmem_alloc(&tmem_slot, 512u);
-    tmem_relinquish();
-  }
-  if (warp >= 8) {
-    const unsigned char* kvg = p.key_valid + (long long)b * p.Sk;
-    const int w = warp - 8;
-    const int j = w * 32 + lane;
-    const bool v = (j < p.Sk) && (mode == MMFM_MASK_CAUSAL || kvg[j] != 0);
-    const uint32_t m = __ballot_sync(0xffffffffu, v);
-    if (lane == 0) s_colbits[w] = m;
-  }
-  DBG_T(1);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  DBG_T(2);
-  const uint32_t tmem_base = tmem_slot;
-  constexpr uint32_t dq_col = 256u, dk_col = 320u, dv_col = 384u;
-
-  const float sl2 = p.scale * kLog2e;
-  const float dsc = DROP ? p.drop_p.scale : 1.0f;
-  const float inv_dsc = 1.0f / dsc;
-  const uint32_t t_row = tmem_base + ((uint32_t)(quad * 32) << 16);
-  const uint32_t idesc_q = make_idesc_bf16(128, D, 0, 1);                // dQ: A K-major (slabs), B MN-major (K tile)
-  const uint32_t idesc_t = make_idesc_bf16(128, D, 1, 1);                // dK / dV: A MN-major (slabs), B MN-major
-
-  // ---- MMA batches (one elected thread of warp 0) ----
-  auto issue_s = [&](int qt, int kh) {     // S_h = Q_qt K_h^T -> buffer kh
-    const uint32_t n = (uint32_t)(kh == nkh - 1 ? wlast : 128);
-    const uint32_t idesc = make_idesc_bf16(128, n, 0, 0);
-    const uint32_t aq = sQ + (uint32_t)qt * 128u * kRowBytes, bk = sK + (uint32_t)kh * 128u * kRowBytes;
-#pragma unroll
-    for (int k = 0; k < D / 16; ++k)
-      umma_bf16(tmem_base + 128u * kh, make_smem_desc(aq + k * 32, 16, kSbo64, 4), make_smem_desc(bk + k * 32, 16, kSbo64, 4),
-                idesc, k > 0 ? 1u : 0u);
-    umma_commit(&s_bar[kh]);
-  };
-  auto issue_dp_dv = [&](int qt, int kh) {  // dP_h = dO_qt V_h^T over S_h ; dV_h += P_drop_h^T dO_qt
-    const uint32_t n = (uint32_t)(kh == nkh - 1 ? wlast : 128);
-    const uint32_t idesc = make_idesc_bf16(128, n, 0, 0);
-    const uint32_t ad = sdO + (uint32_t)qt * 128u * kRowBytes, bv = sV + (uint32_t)kh * 128u * kRowBytes;
-#pragma unroll
-    for (int k = 0; k < D / 16; ++k)
-      umma_bf16(tmem_base + 128u * kh, make_smem_desc(ad + k * 32, 16, kSbo64, 4), make_smem_desc(bv + k * 32, 16, kSbo64, 4),
-                idesc, k > 0 ? 1u : 0u);
-    for (int kk = 0; kk < 8; ++kk)
-      umma_bf16(tmem_base + dv_col + 32u * kh,
-                make_smem_desc(sPd + (uint32_t)(2 * kh) * kSlabBytes + (uint32_t)kk * 2048u, kSlabBytes, 1024, 2),
-                make_smem_desc(ad + (uint32_t)kk * 16u * kRowBytes, kSbo64, kSbo64, 4), idesc_t, (qt > 0 || kk > 0) ? 1u : 0u);
-    umma_commit(&dp_bar[kh]);
-  };
-  auto issue_dq_dk = [&](int qt, int kh) {  // dQ_qt += dS_h K_h ; dK_h += dS_h^T Q_qt
-    const int nks = (kh == nkh - 1 ? wlast : 128) >> 4;
-    const uint32_t aq = sQ + (uint32_t)qt * 128u * kRowBytes;
-    for (int k2 = 0; k2 < nks; ++k2) {
-      const int kk = 8 * kh + k2;           // 16-key step inside the whole key range
-      umma_bf16(tmem_base + dq_col + 32u * qt,
-                make_smem_desc(sdS + (uint32_t)(kk >> 2) * kSlabBytes + (uint32_t)(kk & 3) * 32u, 16, 1024, 2),
-                make_smem_desc(sK + (uint32_t)kk * 16u * kRowBytes, kSbo64, kSbo64, 4), idesc_q, (kh > 0 || k2 > 0) ? 1u : 0u);
-    }
-    for (int kk = 0; kk < 8; ++kk)
-      umma_bf16(tmem_base + dk_col + 32u * kh,
-                make_smem_desc(sdS + (uint32_t)(2 * kh) * kSlabBytes + (uint32_t)kk * 2048u, kSlabBytes, 1024, 2),
-                make_smem_desc(aq + (uint32_t)kk * 16u * kRowBytes, kSbo64, kSbo64, 4), idesc_t, (qt > 0 || kk > 0) ? 1u : 0u);
-  };
-
-  if (warp == 0) {
-    if (elect_one()) {
-      mbar_wait(&ld_kv_bar, 0);
-      mbar_wait(&ld_q_bar[0], 0);
-      tc_fence_after();
-      for (int kh = 0; kh < nkh; ++kh) issue_s(0, kh);
-    }
-    __syncwarp();
-  }
-
-#pragma unroll 1
-  for (int qt = 0; qt < nqt; ++qt) {
-    const uint32_t par = (uint32_t)(qt & 1);
-    const int i = qt * 128 + row;
-    const float lse2 = lse_r[qt & 1] * kLog2e;
-    const float dl = dl_r[qt & 1] * inv_dsc;
-    uint32_t aws[2] = {0u, 0u};
-    const uint2 kpre[2] = {kpre_r[qt & 1][0], kpre_r[qt & 1][1]};
-#pragma unroll
-    for (int kh = 0; kh < 2; ++kh) {
-      const int c = grp + 4 * kh;
-      if (c < nch) {
-        uint32_t aw = s_colbits[c];
-        const int rel = i - 32 * c;
-        if (mode == MMFM_MASK_KEY_OR_DIAG) {
-          if (rel >= 0 && rel < 32 && i < p.Sk) aw |= 1u << rel;
-        } else if (mode == MMFM_MASK_CAUSAL) {
-          aw &= (rel >= 31) ? 0xFFFFFFFFu : (rel < 0 ? 0u : ((2u << rel) - 1u));
-        }
-        aws[kh] = aw;
-      }
-    }
-    uint32_t pk[2][16];    // p as packed bf16, kept for pass B
-    uint32_t pdq[2][16];   // p * keep as packed bf16, kept for pass B
-
-    // ---------------- pass A (both halves): probabilities ----------------
-#pragma unroll
-    for (int kh = 0; kh < 2; ++kh) {
-      if (kh >= nkh) break;
-      const int c = grp + 4 * kh;
-      DBG_T(4 + 16 * qt + 4 * kh);
-      mbar_wait(&s_bar[kh], par);
-      tc_fence_after();
-      DBG_T(5 + 16 * qt + 4 * kh);
-      if (c < nch) {
-        const uint32_t aw = aws[kh];
-        uint32_t km[4][2] = {{0u, 0u}, {0u, 0u}, {0u, 0u}, {0u, 0u}};
-        if (DROP) {
-          const uint2 w2 = kpre[kh];
-          const int sh = 8 * (c & 1);   // second 32-column chunk of the 64-key block: n-tiles 4..7 -> bits 8..15
-          keep_msb_words((w2.x & 0xFFFFu) >> sh, km[0]);
-          keep_msb_words((w2.x >> 16) >> sh, km[1]);
-          keep_msb_words((w2.y & 0xFFFFu) >> sh, km[2]);
-          keep_msb_words((w2.y >> 16) >> sh, km[3]);
-        }
-        const bool masked = __any_sync(0xffffffffu, aw != 0xFFFFFFFFu);
-        uint32_t rs[2][16];
-        tmem_ld16(t_row + 32u * c, rs[0]);
-        tmem_ld16(t_row + 32u * c + 16u, rs[1]);
-        tmem_ld_wait();
-        uint32_t pdk[2][8];
-        if (masked) {
-          bwd_prob_half<true, DROP, 0>(rs[0], aw, sl2, lse2, km, &pk[kh][0], pdk[0]);
-          bwd_prob_half<true, DROP, 1>(rs[1], aw, sl2, lse2, km, &pk[kh][8], pdk[1]);
-        } else {
-          bwd_prob_half<false, DROP, 0>(rs[0], aw, sl2, lse2, km, &pk[kh][0], pdk[0]);
-          bwd_prob_half<false, DROP, 1>(rs[1], aw, sl2, lse2, km, &pk[kh][8], pdk[1]);
-        }
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-#pragma unroll
-          for (int t = 0; t < 8; ++t) pdq[kh][8 * hf + t] = pdk[hf][t];
-#pragma unroll
-          for (int q4 = 0; q4 < 2; ++q4) {
-            const int j16 = (c & 1) * 4 + hf * 2 + q4;
-            const uint32_t addr = sPd + (uint32_t)(c >> 1) * kSlabBytes + (uint32_t)row * 128u + (uint32_t)((j16 ^ (row & 7)) * 16);
-            st_shared_v4(addr, pdk[hf][4 * q4], pdk[hf][4 * q4 + 1], pdk[hf][4 * q4 + 2], pdk[hf][4 * q4 + 3]);
-          }
-        }
-      }
-      DBG_T(6 + 16 * qt + 4 * kh);
-      tc_fence_before();
-      fence_proxy_async();
-      __syncthreads();
-      DBG_T(7 + 16 * qt + 4 * kh);
-      if (warp == 0) {
-        if (elect_one()) {
-          tc_fence_after();
-          issue_dp_dv(qt, kh);
-        }
-        __syncwarp();
-      }
-    }
-
-    // ---------------- pass B (both halves): dS ----------------
-#pragma unroll
-    for (int kh = 0; kh < 2; ++kh) {
-      if (kh >= nkh) break;
-      const int c = grp + 4 * kh;
-      DBG_T(12 + 16 * qt + 4 * kh);
-      mbar_wait(&dp_bar[kh], par);
-      tc_fence_after();
-      DBG_T(13 + 16 * qt + 4 * kh);
-      if (c < nch) {
-        const uint32_t aw = aws[kh];
-        const bool masked = __any_sync(0xffffffffu, aw != 0xFFFFFFFFu);
-        uint32_t rd[2][16];
-        tmem_ld16(t_row + 32u * c, rd[0]);
-        tmem_ld16(t_row + 32u * c + 16u, rd[1]);
-        tmem_ld_wait();
-        uint32_t dsk[2][8];
-        if (masked) {
-          bwd_ds_half<true>(rd[0], aw & 0xFFFFu, dl, &pk[kh][0], &pdq[kh][0], dsk[0]);
-          bwd_ds_half<true>(rd[1], aw >> 16, dl, &pk[kh][8], &pdq[kh][8], dsk[1]);
-        } else {
-          bwd_ds_half<false>(rd[0], 0xFFFFu, dl, &pk[kh][0], &pdq[kh][0], dsk[0]);
-          bwd_ds_half<false>(rd[1], 0xFFFFu, dl, &pk[kh][8], &pdq[kh][8], dsk[1]);
-        }
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-#pragma unroll
-          for (int q4 = 0; q4 < 2; ++q4) {
-            const int j16 = (c & 1) * 4 + hf * 2 + q4;
-            const uint32_t addr = sdS + (uint32_t)(c >> 1) * kSlabBytes + (uint32_t)row * 128u + (uint32_t)((j16 ^ (row & 7)) * 16);
-            st_shared_v4(addr, dsk[hf][4 * q4], dsk[hf][4 * q4 + 1], dsk[hf][4 * q4 + 2], dsk[hf][4 * q4 + 3]);
-          }
-        }
-      }
-      DBG_T(14 + 16 * qt + 4 * kh);
-      tc_fence_before();
-      fence_proxy_async();
-      __syncthreads();
-      DBG_T(15 + 16 * qt + 4 * kh);
-      if (warp == 0) {
-        if (elect_one()) {
-          tc_fence_after();
-          issue_dq_dk(qt, kh);
-          if (qt + 1 < nqt) {
-            if (kh == 0) { mbar_wait(&ld_q_bar[(qt + 1) & 1], 0); tc_fence_after(); }
-            issue_s(qt + 1, kh);        // its commit also covers the dQ / dK batch above
-          } else if (kh == nkh - 1) {
-            umma_commit(&done_bar);
-          }
-        }
-        __syncwarp();
-      }
-    }
-  }
-
-  DBG_T(40);
-  mbar_wait(&done_bar, 0);
-  tc_fence_after();
-  DBG_T(41);
-  // ---------------- read-out: pieces of 16 columns over the 4 thread groups ----------------
-  //   piece 0..3   : dQ of query tile piece/2, column half piece&1          (TMEM lane = query row)
-  //   piece 4..11  : (kh, which, half) = ((piece-4)/4, ((piece-4)/2)&1, (piece-4)&1); which 0 dK, 1 dV (lane = key row)
-  uint32_t r[3][16];
-#pragma unroll
-  for (int u = 0; u < 3; ++u) {
-    const int piece = grp + 4 * u;
-    uint32_t col;
-    if (piece < 4) col = dq_col + 32u * (piece >> 1) + 16u * (piece & 1);
-    else {
-      const int q = piece - 4;
-      col = ((q >> 1) & 1 ? dv_col : dk_col) + 32u * (q >> 2) + 16u * (q & 1);
-    }
-    tmem_ld16(t_row + col, r[u]);
-  }
-  tmem_ld_wait();
-  tc_fence_before();
-  __syncthreads();
-  DBG_T(42);
-  if (warp == 1) tmem_dealloc(tmem_base, 512u);
-  // Stage the 6 output tiles (dQ x2, dK x2, dV x2: [128 rows][32 bf16]) in the dead operand buffers, then copy them out
-  // with 4 lanes per 64-byte row: a warp store covers 8 full rows (16 full sectors) instead of 32 half-filled ones --
-  // the row-strided form kept the load/store unit busy for ~4000 cycles per CTA.
-  constexpr int kOutPitch = 80;   // bytes per staged row (64 + 16): 16-byte accesses of a quarter-warp hit distinct banks
-  uint8_t* stage_o = smem_raw + (smem_base - smem_u32(smem_raw));
-#pragma unroll
-  for (int u = 0; u < 3; ++u) {
-    const int piece = grp + 4 * u;
-    int tile, half;
-    float fs;
-    if (piece < 4) { tile = piece >> 1; half = piece & 1; fs = p.scale * dsc; }
-    else {
-      const int q = piece - 4, kh = q >> 2, which = (q >> 1) & 1;
-      tile = 2 + 2 * kh + which; half = q & 1; fs = which ? dsc : p.scale * dsc;
-    }
-    uint8_t* dst = stage_o + (tile * 128 + row) * kOutPitch + half * 32;
-#pragma unroll
-    for (int k = 0; k < 16; k += 8)
-      *reinterpret_cast<uint4*>(dst + 2 * k) =
-          make_uint4(pack_bf16x2(__uint_as_float(r[u][k]) * fs, __uint_as_float(r[u][k + 1]) * fs),
-                     pack_bf16x2(__uint_as_float(r[u][k + 2]) * fs, __uint_as_float(r[u][k + 3]) * fs),
-                     pack_bf16x2(__uint_as_float(r[u][k + 4]) * fs, __uint_as_float(r[u][k + 5]) * fs),
-                     pack_bf16x2(__uint_as_float(r[u][k + 6]) * fs, __uint_as_float(r[u][k + 7]) * fs));
-  }
-  __syncthreads();
-#pragma unroll 1
-  for (int it = 0; it < 6; ++it) {
-    const int idx = it * kFusedThreads + tid;      // (tile, row, 16-byte piece)
-    const int tile = idx >> 9, rr = (idx >> 2) & 127, q4 = idx & 3;
-    bf16* dst = nullptr;
-    if (tile < 2) {
-      const int i = tile * 128 + rr;
-      if (tile < nqt && i < p.Sq) dst = p.dq + ((long long)b * p.Sq + i) * p.lddq + h * D + 8 * q4;
-    } else {
-      const int kh = (tile - 2) >> 1, which = (tile - 2) & 1, j = kh * 128 + rr;
-      if (kh < nkh && j < p.Sk)
-        dst = (which ? p.dv + ((long long)b * p.Sk + j) * p.lddv : p.dk + ((long long)b * p.Sk + j) * p.lddk) + h * D + 8 * q4;
-    }
-    if (dst != nullptr)
-      *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(stage_o + (tile * 128 + rr) * kOutPitch + q4 * 16);
-  }
-  DBG_T(43);
-}
-
 }  // namespace mmfm
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1206,23 +833,6 @@ static AttnParams to_params(const mmfm_attn_args* a) {
     }                                                                                             \
   } while (0)
 
-// MMFM_ATTN_TC=0 forces the mma.sync kernels everywhere (A/B measurements)
-static bool attn_tc_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MMFM_ATTN_TC");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
-static bool env_on(const char* name, int* cache) {   // default on; "<name>=0" switches a kernel family off
-  if (*cache < 0) {
-    const char* e = getenv(name);
-    *cache = (e && e[0] == '0') ? 0 : 1;
-  }
-  return *cache != 0;
-}
-
 // Forward dispatch:
 //   no modality-separation mask, 16-byte aligned operands -> persistent warp-specialised tcgen05 kernel (attention_pipe.cu)
 //   otherwise                                             -> mma.sync flash kernel (modality ids, odd alignments)
@@ -1232,9 +842,7 @@ extern "C" int mmfm_attention_fwd(const mmfm_attn_args* a, void* stream) {
   const AttnParams p = to_params(a);
   const bool al16 = ((reinterpret_cast<uintptr_t>(a->q) | reinterpret_cast<uintptr_t>(a->k) |
                       reinterpret_cast<uintptr_t>(a->v) | reinterpret_cast<uintptr_t>(a->o)) & 15) == 0;
-  static int pipe = -1;   // MMFM_ATTN_PIPE=0
-  if (attn_tc_enabled() && env_on("MMFM_ATTN_PIPE", &pipe) && !sep && al16)
-    return launch_attn_fwd_pipe(a, p, (cudaStream_t)stream);
+  if (!sep && al16) return launch_attn_fwd_pipe(a, p, (cudaStream_t)stream);
   dim3 grid((a->Sq + kTile - 1) / kTile, a->n_heads, a->B);
   cudaStream_t st = (cudaStream_t)stream;
   const int nkb = (a->Sk + kTile - 1) / kTile;
@@ -1253,35 +861,9 @@ static int launch_dkv(const mmfm_attn_args* a, const AttnParams& p, cudaStream_t
   ATTN_DISPATCH(attn_bwd_dkv_kernel, grid, 6 * TileCfg<D>::kBytes + 4 * kTile * 4 + 2 * kTile * 4 * 2);
 }
 
-static int launch_bwd_fused2(const mmfm_attn_args* a, const AttnParams& p, cudaStream_t st) {
-  constexpr int D = 32;
-  const int npk = (a->Sk + 15) / 16 * 16;
-  const uint64_t width = (uint64_t)a->n_heads * D;
-  const bool drop = a->drop_p.thresh != 0u;
-  CUtensorMap tq, tdo, tk, tv;
-  if (int rc = make_tmap_bf16_2d(&tq, a->q, (uint64_t)a->B * a->Sq, width, (uint64_t)a->ldq, D, 128, TMA_SW_64)) return rc;
-  if (int rc = make_tmap_bf16_2d(&tdo, a->d_o, (uint64_t)a->B * a->Sq, width, (uint64_t)a->lddo, D, 128, TMA_SW_64)) return rc;
-  if (int rc = make_tmap_bf16_2d(&tk, a->k, (uint64_t)a->B * a->Sk, width, (uint64_t)a->ldk, D, npk, TMA_SW_64)) return rc;
-  if (int rc = make_tmap_bf16_2d(&tv, a->v, (uint64_t)a->B * a->Sk, width, (uint64_t)a->ldv, D, npk, TMA_SW_64)) return rc;
-  const int smem = 1024 + 4 * 256 * 64 + 8 * 128 * 128;   // K, V, Q x2, dO x2 (256 rows each) + 8 slabs
-  static bool attr_set = false;
-  if (!attr_set) {
-    MMFM_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_fused2_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    MMFM_CHECK_CUDA(cudaFuncSetAttribute(attn_bwd_fused2_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    attr_set = true;
-  }
-  dim3 grid(a->n_heads, a->B);
-  if (drop) attn_bwd_fused2_tc_kernel<true><<<grid, kFusedThreads, smem, st>>>(tq, tdo, tk, tv, p, npk);
-  else attn_bwd_fused2_tc_kernel<false><<<grid, kFusedThreads, smem, st>>>(tq, tdo, tk, tv, p, npk);
-  MMFM_CHECK_CUDA(cudaGetLastError());
-  return 0;
-}
-
 // Backward dispatch (after the prep kernel: delta = rowsum(dO * O), dO <- dO * output-dropout mask):
-//   d_head 32, Sq, Sk <= 256 (the default model)  -> persistent warp-specialised fused kernel (attention_bwd_ws.cu;
-//                                                     MMFM_ATTN_WS=0: its block-synchronous predecessor
-//                                                     attention_bwd_persist.cu), or the one-CTA-per-(batch, head) form
-//                                                     when the side data are unaligned
+//   d_head 32, Sq, Sk <= 256 (the default model), 16-byte aligned lse / delta / p_keep, Sq % 4 == 0
+//                                                  -> persistent warp-specialised fused kernel (attention_bwd_ws.cu)
 //   any other shape without modality-separation    -> streamed tcgen05 dq / dkv pair (attention_bwd_stream.cu)
 //   modality-separation mask, odd alignments        -> mma.sync dq / dkv pair
 extern "C" int mmfm_attention_bwd(const mmfm_attn_args* a, void* stream) {
@@ -1305,16 +887,12 @@ extern "C" int mmfm_attention_bwd(const mmfm_attn_args* a, void* stream) {
                       reinterpret_cast<uintptr_t>(a->v) | reinterpret_cast<uintptr_t>(a->d_o) |
                       reinterpret_cast<uintptr_t>(a->dq) | reinterpret_cast<uintptr_t>(a->dk) |
                       reinterpret_cast<uintptr_t>(a->dv)) & 15) == 0;
-  static int tc_bwd = -1, fused = -1, persist = -1, streamed = -1, ws = -1;
-  const bool tc = attn_tc_enabled() && env_on("MMFM_ATTN_TC_BWD", &tc_bwd) && a->mod_q == nullptr && al16;
-  if (tc && env_on("MMFM_ATTN_FUSED_BWD", &fused) && a->d_head == 32 && a->Sq <= 256 && a->Sk <= 256) {
+  if (a->mod_q == nullptr && al16) {
     const bool side_al = ((reinterpret_cast<uintptr_t>(a->lse) | reinterpret_cast<uintptr_t>(a->delta) |
-                           reinterpret_cast<uintptr_t>(a->p_keep)) & 15) == 0 && a->Sq % 4 == 0;
-    if (env_on("MMFM_ATTN_WS", &ws) && side_al) return launch_attn_bwd_ws(a, p, st);
-    if (env_on("MMFM_ATTN_PERSIST", &persist) && side_al) return launch_attn_bwd_persist(a, p, st);
-    return launch_bwd_fused2(a, p, st);
+                           reinterpret_cast<uintptr_t>(a->p_keep)) & 15) == 0;
+    if (a->d_head == 32 && a->Sq <= 256 && a->Sk <= 256 && a->Sq % 4 == 0 && side_al) return launch_attn_bwd_ws(a, p, st);
+    return launch_attn_bwd_stream(a, p, st);
   }
-  if (tc && env_on("MMFM_ATTN_STREAM_BWD", &streamed)) return launch_attn_bwd_stream(a, p, st);
   if (int rc = launch_dq(a, p, st)) return rc;
   return launch_dkv(a, p, st);
 }

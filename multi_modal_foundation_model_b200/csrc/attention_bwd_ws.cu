@@ -1,9 +1,27 @@
 // Masked multi-head attention backward for the default model (d_head 32, Sq, Sk <= 256): persistent, WARP-SPECIALISED
-// tcgen05 / TMEM kernel.  Same mathematics, operand layout and barriers-per-product as attention_bwd_persist.cu (whose
-// header derives dS = P_drop . dP - P . delta and the slab layout; reference: autograd of src/multi_modal/mm_utils.py:
-// 105-112 / :143-150), with the three serialisations of that kernel removed -- a globaltimer trace of it
-// (tools/micro/bwd_persist_timing.py) showed 12.7 us per (batch, head) item of which only ~5.8 us were the four
-// probability / dS passes:
+// tcgen05 / TMEM kernel (autograd of F.scaled_dot_product_attention, reference src/multi_modal/mm_utils.py:105-112,
+// :143-150).  One CTA per SM loops over (batch, head) items and computes dQ, dK and dV of an item in one go, so every
+// score element goes through the softmax / dropout / dS arithmetic once.
+//
+// Mathematics: the forward computes O = P_drop V with P_drop = P . keep . s (s = 1 / (1 - dropout p)), so
+// dP_drop = dO V^T and the softmax gradient is dS = P . (s keep . dP_drop - delta), where delta = rowsum(dO . O)
+// = rowsum(P . dP) comes from the preparation step.  The factor s stays out of the inner loop: the passes compute
+// dS / s = (P . keep) . dP_drop - P . (delta / s), and s is applied when dQ / dK / dV leave tensor memory.
+//
+// Data flow of an item: the key range is split into two 128-key halves, each with its own S / dP buffer in TMEM and its
+// own barriers; per 128-query tile the passes run in the order A(h0) A(h1) B(h0) B(h1) and every MMA batch is issued
+// right after the pass that produces its operands and waited for one pass later:
+//   pass A(h)  p = exp2(s*scale - lse) under the mask, P_drop -> swizzled smem slab ; then  dP_h = dO V_h^T (over the
+//              dead S_h), dV_h += P_drop_h^T dO
+//   pass B(h)  dS -> the SAME slab (P_drop is dead by then) ; then  dQ += dS_h K_h, dK_h += dS_h^T Q, and the S_h of the
+//              next query tile -- or of the NEXT ITEM
+// The slabs are the canonical 128-byte-swizzled layout ([128 query rows] x [64 keys] per slab), written with 16-byte
+// stores from registers, so one copy of dS serves both the dQ (K-major A) and the dK (MN-major A) products.  The
+// operands (K, V, Q, dO) and the per-row side data (lse, delta, keep words -- bulk-copied to shared memory) of item n+1
+// are loaded while item n computes.
+//
+// The block-synchronous form of this kernel took 12.7 us per item (globaltimer trace), of which only ~5.8 us were the
+// four probability / dS passes.  Its three serialisations and what replaced them:
 //   * the MMA batches were issued by math warp 0 between block-wide barriers, so every pass waited for that warp
 //     (0.5 us per query tile)                     -> a dedicated issuer warp; passes hand over through mbarriers only
 //   * after the last pass the CTA drained the tensor pipe, staged and copied the six output tiles out (2.4 us) and only
@@ -32,7 +50,6 @@
 // (the register pool only holds what a warpgroup released: the math warps cannot get past 112, and a 32-register issuer
 // spills inside its MMA batches).
 #include "attn_common.cuh"
-#include <stdlib.h>
 
 #ifdef MMFM_DBG_TIMING
 __device__ long long g_dbg_ws[64];
@@ -72,7 +89,6 @@ __global__ void __launch_bounds__(kWsThreads, 1) attn_bwd_ws_kernel(
     const __grid_constant__ CUtensorMap tmdV, const AttnParams p, int npad, int n_items) {
   constexpr int D = 32;
   constexpr uint32_t kSbo64 = 512;
-  pdl_enter();
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t ld_bar[2], s_bar[2], dp_bar[2], pa_bar[2], ds_bar[2], done_bar, staged_bar;
   __shared__ uint32_t tmem_slot;
@@ -499,10 +515,9 @@ int launch_attn_bwd_ws(const mmfm_attn_args* a, const AttnParams& p, cudaStream_
   const int n_items = a->B * a->n_heads;
   int grid = device_sm_count();
   if (grid > n_items) grid = n_items;
-  // dq / dk / dv are column blocks of one [B Sq, 3 H] gradient buffer in the model: the QKV dgrad GEMM reads it next
-  set_l2_window(a->dq, (size_t)a->B * a->Sq * (size_t)a->lddq * 2);
-  if (drop) MMFM_CHECK_CUDA(launch_pdl(attn_bwd_ws_kernel<true>, dim3(grid), dim3(kWsThreads), kWsSmem, st, tq, tdo, tk, tv, tdq, tdk, tdv, p, npk, n_items));
-  else MMFM_CHECK_CUDA(launch_pdl(attn_bwd_ws_kernel<false>, dim3(grid), dim3(kWsThreads), kWsSmem, st, tq, tdo, tk, tv, tdq, tdk, tdv, p, npk, n_items));
+  if (drop) attn_bwd_ws_kernel<true><<<grid, kWsThreads, kWsSmem, st>>>(tq, tdo, tk, tv, tdq, tdk, tdv, p, npk, n_items);
+  else attn_bwd_ws_kernel<false><<<grid, kWsThreads, kWsSmem, st>>>(tq, tdo, tk, tv, tdq, tdk, tdv, p, npk, n_items);
+  MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 }  // namespace mmfm

@@ -142,7 +142,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) attn_fwd_pipe_kernel(const __
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int bl = ((p.Sk - (nb - 1) * bn) + 15) & ~15;   // width of the last key block (multiple of 16)
 
-  pdl_trigger();
   if (tid == 0) {
     tma_prefetch_desc(&tmQ);
     tma_prefetch_desc(&tmK);
@@ -168,7 +167,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) attn_fwd_pipe_kernel(const __
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = tmem_slot;
-  pdl_wait();
 
   // item -> (b, h, q0): query-tile pair fastest, then head, then batch
   auto decode = [&](int item, int& b, int& h, int& q0) {
@@ -571,10 +569,9 @@ static int launch_fwd_pipe_d(const mmfm_attn_args* a, const AttnParams& p, cudaS
   const int n_items = (int)n_items_ll;
   int grid = device_sm_count();
   if (grid > n_items) grid = n_items;
-  const size_t o_bytes = (size_t)a->B * a->Sq * (size_t)a->ldo * 2;
-  set_l2_window(a->o, o_bytes);   // read next by the out-projection GEMM
-  if (drop) MMFM_CHECK_CUDA(launch_pdl(attn_fwd_pipe_kernel<D, true>, dim3(grid), dim3(kPipeThreads), Cfg::kSmem, st, tq, tk, tv, p, bn, nb, n_qp, n_items));
-  else MMFM_CHECK_CUDA(launch_pdl(attn_fwd_pipe_kernel<D, false>, dim3(grid), dim3(kPipeThreads), Cfg::kSmem, st, tq, tk, tv, p, bn, nb, n_qp, n_items));
+  if (drop) attn_fwd_pipe_kernel<D, true><<<grid, kPipeThreads, Cfg::kSmem, st>>>(tq, tk, tv, p, bn, nb, n_qp, n_items);
+  else attn_fwd_pipe_kernel<D, false><<<grid, kPipeThreads, Cfg::kSmem, st>>>(tq, tk, tv, p, bn, nb, n_qp, n_items);
+  MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 

@@ -46,7 +46,6 @@ MMFM_DEVINL uint4 pdrop_bytes(unsigned long long seed, uint32_t site, unsigned l
   return philox4x32((uint32_t)g, (uint32_t)(g >> 32), site, 1u, (uint32_t)seed, (uint32_t)(seed >> 32));
 }
 
-constexpr int kFusedThreads = 512;
 constexpr uint32_t kSlabBytes = 128 * 128;   // 128 query rows x 64 keys (bf16)
 
 MMFM_DEVINL void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
@@ -68,47 +67,6 @@ MMFM_DEVINL void keep_msb_words(uint32_t bits8, uint32_t (&w)[2]) {
   w[0] = (bits8 & 0xFu) * 0x10204080u;
   w[1] = ((bits8 >> 4) & 0xFu) * 0x10204080u;
 }
-// probabilities of one 16-column half of a chunk: p (packed bf16) and p * keep (packed bf16)
-template <bool MASKED, bool DROP, int HF>
-MMFM_DEVINL void bwd_prob_half(const uint32_t (&rs)[16], uint32_t aw, float sl2, float lse2,
-                               const uint32_t (&km)[4][2], uint32_t* pk, uint32_t (&pdk)[8]) {
-#pragma unroll
-  for (int t = 0; t < 8; ++t) {
-    float e0 = fast_exp2(fmaf(__uint_as_float(rs[2 * t]), sl2, -lse2));
-    float e1 = fast_exp2(fmaf(__uint_as_float(rs[2 * t + 1]), sl2, -lse2));
-    if (MASKED) {   // select, never multiply: masked columns may hold stale TMEM bits
-      if (!((aw >> (16 * HF + 2 * t)) & 1u)) e0 = 0.f;
-      if (!((aw >> (16 * HF + 2 * t + 1)) & 1u)) e1 = 0.f;
-    }
-    const uint32_t pp = pack_bf16x2(e0, e1);
-    pk[t] = pp;
-    if (DROP) {
-      // pair T = 8*HF + t of the chunk: n-tile n = T/4, quad lane ql = T%4 -> word n/2 of km[ql], byte pair n&1
-      const int T = 8 * HF + t, n = T >> 2;
-      pdk[t] = pp & prmt_b(km[T & 3][n >> 1], (n & 1) ? 0xBBAAu : 0x9988u);
-    } else {
-      pdk[t] = pp;
-    }
-  }
-}
-// dS of one 16-column half: ds = p_drop * dP - p * delta  (= p * (keep * dP - delta)), packed bf16
-template <bool MASKED>
-MMFM_DEVINL void bwd_ds_half(const uint32_t (&rd)[16], uint32_t aw16, float dl, const uint32_t* pk, const uint32_t* pdk,
-                             uint32_t (&dsk)[8]) {
-#pragma unroll
-  for (int t = 0; t < 8; ++t) {
-    const float p0 = __uint_as_float(pk[t] << 16), p1 = __uint_as_float(pk[t] & 0xFFFF0000u);
-    const float q0 = __uint_as_float(pdk[t] << 16), q1 = __uint_as_float(pdk[t] & 0xFFFF0000u);
-    float s0 = fmaf(q0, __uint_as_float(rd[2 * t]), -p0 * dl);
-    float s1 = fmaf(q1, __uint_as_float(rd[2 * t + 1]), -p1 * dl);
-    if (MASKED) {
-      if (!((aw16 >> (2 * t)) & 1u)) s0 = 0.f;
-      if (!((aw16 >> (2 * t + 1)) & 1u)) s1 = 0.f;
-    }
-    dsk[t] = pack_bf16x2(s0, s1);
-  }
-}
-
 
 // the four quad-lane calls of one 64-key block at once (g = (row*nblk + blk)*4 + ql: the low two counter bits are ql and
 // g is a multiple of 4, so the +ql never carries into the high word)
@@ -122,9 +80,7 @@ MMFM_DEVINL void pdrop_bytes_x4(unsigned long long seed, uint32_t site, unsigned
 int launch_attn_fwd_pipe(const mmfm_attn_args* a, const AttnParams& p, cudaStream_t st);
 // attention_bwd_stream.cu: tcgen05 backward pair for long sequences (runs after the prep kernel)
 int launch_attn_bwd_stream(const mmfm_attn_args* a, const AttnParams& p, cudaStream_t st);
-// attention_bwd_persist.cu: persistent software-pipelined fused backward (d_head 32, Sq, Sk <= 256, Sq % 4 == 0)
-int launch_attn_bwd_persist(const mmfm_attn_args* a, const AttnParams& p, cudaStream_t st);
-// attention_bwd_ws.cu: the same data flow, warp-specialised (issuer / loader warps, deferred read-out, TMA stores)
+// attention_bwd_ws.cu: persistent warp-specialised fused backward (d_head 32, Sq, Sk <= 256, Sq % 4 == 0)
 int launch_attn_bwd_ws(const mmfm_attn_args* a, const AttnParams& p, cudaStream_t st);
 
 }  // namespace mmfm

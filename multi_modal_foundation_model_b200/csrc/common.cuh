@@ -30,20 +30,6 @@ MMFM_DEVINL bool elect_one() {
 }
 
 // ------------------------------------------------------------------------------------------------
-// programmatic dependent launch: every hot kernel starts with pdl_enter().  The trigger lets the NEXT kernel of the
-// stream / graph be scheduled while this one is still running (its CTAs become resident as SMs drain and park at their
-// own wait), the wait blocks until every prerequisite grid has completed and its writes are visible -- so kernel-to-
-// kernel launch latency and the tail of a persistent grid overlap instead of adding up.  Without the launch attribute
-// (host_util.h: launch_pdl; off unless MMFM_PDL=1 -- measured neutral on the default step) both instructions are no-ops.
-// ------------------------------------------------------------------------------------------------
-MMFM_DEVINL void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-MMFM_DEVINL void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-MMFM_DEVINL void pdl_enter() {
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-
-// ------------------------------------------------------------------------------------------------
 // mbarrier
 // ------------------------------------------------------------------------------------------------
 MMFM_DEVINL void mbar_init(uint64_t* bar, uint32_t count) {
@@ -156,30 +142,6 @@ MMFM_DEVINL void bulk_wait_group_read() {
 template <int N>
 MMFM_DEVINL void bulk_wait_group() {
   asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
-}
-
-// Multicast load: the box lands at the same shared-memory offset of every CTA of the cluster whose rank bit is set in
-// `mask`, and completes `bytes` on the mbarrier at the same offset in each of them.
-MMFM_DEVINL void tma_load_2d_mc(uint32_t smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_dst), "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-// tcgen05.commit that arrives on the mbarrier at this offset in every CTA of `mask`
-MMFM_DEVINL void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
-MMFM_DEVINL uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-MMFM_DEVINL void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 
 // Pull one box of the tensor into L2 without touching shared memory: issued a tile or two ahead of the real load, it
@@ -513,7 +475,7 @@ MMFM_DEVINL double det_add(double a, double b) { return a + b; }
 MMFM_DEVINL float4 det_add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
 
 // Ticketed pairwise tree over the n_leaves partial vectors slot(i) = ws + i * stride (n elements of V each) of one
-// reduction.  Every CTA of the reduction calls it with all its threads after writing slot(leaf) (and after pdl_wait).
+// reduction.  Every CTA of the reduction calls it with all its threads after writing slot(leaf).
 // At level l node k covers slot k << l; the nodes 2j and 2j+1 meet at ticket ((2j+1) << l) - 1.  The CTA that arrives
 // second adds the two slots into the left one and climbs; the first one exits; an unpaired last node climbs as it is.
 // The CTA that completes the root pair calls emit(i, total_i) for i in [0, n) instead of storing it.  The tree's shape

@@ -11,7 +11,6 @@
 //              token-zeroing / residual, direct vectorised global stores
 // Several CTAs are resident per SM (smem- and TMEM-limited), so one CTA's epilogue overlaps another's main loop.
 #include "common.cuh"
-#include <stdlib.h>
 #include "host_util.h"
 #include "../../include/mmfm_b200.h"
 
@@ -96,8 +95,7 @@ enum EpiKind : int {
 template <int BN, int STAGES, int EPI>
 __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA,
                                                                  const __grid_constant__ CUtensorMap tmB,
-                                                                 const mmfm_gemm_args p, int tiles_n, int n_tiles,
-                                                                 int bstat) {
+                                                                 const mmfm_gemm_args p, int tiles_n, int n_tiles) {
   constexpr uint32_t kABytes = kBM * kBK * 2;  // 16 KB
   constexpr uint32_t kBBytes = BN * kBK * 2;
   constexpr uint32_t kStageBytes = kABytes + kBBytes;
@@ -106,14 +104,9 @@ __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_con
   constexpr int kHalf = BN / (kEpiWarps / 4);   // columns per epilogue warp
   constexpr bool GEN = EPI == EPI_GENERIC;
 
-  // Weight-stationary mode (bstat): the grid is a multiple of tiles_n, so every tile of this CTA has the same column
-  // block; its whole K extent of B (<= half of the ring area) is loaded ONCE and stays resident, the ring carries A
-  // k-blocks only.  These skinny-K GEMMs are bound by L2 -> SM traffic, which this halves.
-  constexpr int kMaxStages = 8;
   extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t full_bar[kMaxStages];
-  __shared__ __align__(8) uint64_t empty_bar[kMaxStages];
-  __shared__ __align__(8) uint64_t b_full;
+  __shared__ __align__(8) uint64_t full_bar[STAGES];
+  __shared__ __align__(8) uint64_t empty_bar[STAGES];
   __shared__ __align__(8) uint64_t acc_full[2];
   __shared__ __align__(8) uint64_t acc_empty[2];
   __shared__ uint32_t tmem_slot;
@@ -124,22 +117,15 @@ __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_con
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int nkb = (p.K + kBK - 1) / kBK;
-  const uint32_t b_res_bytes = bstat ? (uint32_t)nkb * kBBytes : 0u;
-  const uint32_t ring_base = smem_base + b_res_bytes;
-  const uint32_t st_bytes = bstat ? kABytes : kStageBytes;
-  uint32_t nst = bstat ? (STAGES * kStageBytes - b_res_bytes) / kABytes : (uint32_t)STAGES;
-  if (nst > (uint32_t)kMaxStages) nst = kMaxStages;
 
-  pdl_trigger();
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
 #pragma unroll
-    for (int s = 0; s < kMaxStages; ++s) {
+    for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full_bar[s], 1);
       mbar_init(&empty_bar[s], 1);
     }
-    mbar_init(&b_full, 1);
     mbar_init(&acc_full[0], 1);
     mbar_init(&acc_full[1], 1);
     mbar_init(&acc_empty[0], kEpiWarps);
@@ -154,16 +140,10 @@ __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_con
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = tmem_slot;
-  pdl_wait();
 
   if (warp == 0) {
     if (elect_one()) {
       uint32_t it = 0;
-      if (bstat) {
-        const int n0 = ((int)blockIdx.x % tiles_n) * BN;
-        mbar_arrive_expect_tx(&b_full, b_res_bytes);
-        for (int kb = 0; kb < nkb; ++kb) tma_load_2d_addr(smem_base + kb * kBBytes, &tmB, &b_full, kb * kBK, n0);
-      }
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int m0 = (tile / tiles_n) * kBM, n0 = (tile % tiles_n) * BN;
         // L2 prefetch of the activation rows this CTA needs two tiles from now (the ring itself holds about one
@@ -176,12 +156,12 @@ __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_con
           }
         }
         for (int kb = 0; kb < nkb; ++kb, ++it) {
-          const uint32_t s = it % nst;
-          if (it >= nst) mbar_wait(&empty_bar[s], ((it / nst) - 1) & 1);
-          mbar_arrive_expect_tx(&full_bar[s], st_bytes);
-          const uint32_t a_dst = ring_base + s * st_bytes;
+          const uint32_t s = it % STAGES;
+          if (it >= STAGES) mbar_wait(&empty_bar[s], ((it / STAGES) - 1) & 1);
+          mbar_arrive_expect_tx(&full_bar[s], kStageBytes);
+          const uint32_t a_dst = smem_base + s * kStageBytes;
           tma_load_2d_addr(a_dst, &tmA, &full_bar[s], kb * kBK, m0);
-          if (!bstat) tma_load_2d_addr(a_dst + kABytes, &tmB, &full_bar[s], kb * kBK, n0);
+          tma_load_2d_addr(a_dst + kABytes, &tmB, &full_bar[s], kb * kBK, n0);
         }
       }
     }
@@ -189,18 +169,17 @@ __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_con
     if (elect_one()) {
       const uint32_t idesc = make_idesc_bf16(kBM, BN, 0, 0);
       uint32_t it = 0, t = 0;
-      if (bstat) mbar_wait(&b_full, 0);
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++t) {
         const uint32_t buf = t & 1u;
         if (t >= 2) mbar_wait(&acc_empty[buf], ((t >> 1) - 1) & 1);   // epilogue drained this TMEM buffer
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + buf * BN;
         for (int kb = 0; kb < nkb; ++kb, ++it) {
-          const uint32_t s = it % nst;
-          mbar_wait(&full_bar[s], (it / nst) & 1);
+          const uint32_t s = it % STAGES;
+          mbar_wait(&full_bar[s], (it / STAGES) & 1);
           tc_fence_after();
-          const uint32_t a_addr = ring_base + s * st_bytes;
-          const uint32_t b_addr = bstat ? smem_base + kb * kBBytes : a_addr + kABytes;
+          const uint32_t a_addr = smem_base + s * kStageBytes;
+          const uint32_t b_addr = a_addr + kABytes;
 #pragma unroll
           for (int k = 0; k < kBK / 16; ++k) {
             const uint64_t da = make_smem_desc(a_addr + k * 32, 16, 1024, 2);
@@ -497,26 +476,21 @@ __global__ void __launch_bounds__(kTnThreads, 1) gemm_tn_kernel(const __grid_con
 // wgrad kernel: dW[NO,KI] += sum over a slice of rows of dY[r,NO]^T X[r,KI];  optionally db[NO] += colsum(dY)
 // (the bias gradient rides on the tensor pipe: one extra N=16 MMA per k-step against a tile of ones)
 // ------------------------------------------------------------------------------------------------
-// BN = 256 (KI % 256 == 0): one CTA per SM owns a 128 x 256 tile of dW.  As in gemm_ts.cu the main loop is bound by
-// shared-memory bandwidth (every operand byte is written once by TMA and read once by the tensor core; a 128 x 128 x 16
-// MMA alone reads 128 B/clk), and the wider tile moves 25 % fewer bytes per FLOP and reads every dY box once instead of
-// once per 128-column tile.
-// DET (deterministic mode, no clusters): instead of red.global, each split CTA writes its fp32 tile and bias column to
-// its workspace slot [tile][split] and the splits of a tile are folded by det_tree_fold (common.cuh) into dW / dbias.
-template <int BN>
-__host__ __device__ constexpr long long wgrad_slot_f4() { return ((long long)kBM * BN + kBM) / 4; }   // float4s per workspace slot
+// One CTA owns a 128 x 128 tile of dW, two CTAs per SM.  A 256-wide tile (one CTA per SM) measured equal to slower on
+// B200, and so did 2 x 2 clusters that TMA-multicast the shared dY / X boxes (their stages advance in lock step).
+// DET (deterministic mode): instead of red.global, each split CTA writes its fp32 tile and bias column to its workspace
+// slot [tile][split] and the splits of a tile are folded by det_tree_fold (common.cuh) into dW / dbias.
+constexpr int kWgradBN = 128;
+constexpr long long kWgradSlotF4 = ((long long)kBM * kWgradBN + kBM) / 4;   // float4s per workspace slot
 
-template <int STAGES, int BN, bool DET = false>
+template <int STAGES, bool DET = false>
 __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_constant__ CUtensorMap tmY,
                                                                    const __grid_constant__ CUtensorMap tmX, int R,
                                                                    int NO, int KI, float* __restrict__ dW,
                                                                    long long ldw, int rows_per_split,
-                                                                   float* __restrict__ dbias, int cx, int cy,
+                                                                   float* __restrict__ dbias,
                                                                    float4* __restrict__ ws, unsigned int* tickets) {
-  // (cx, cy) = thread-block cluster shape over (KI tiles, NO tiles), 1 or 2 each.  The CTAs of a cluster work on the
-  // same rows: the two KI tiles of a cluster row share their dY boxes, the two NO tiles of a cluster column share their
-  // X boxes, so each CTA loads HALF of what it consumes and TMA-multicasts it to its peer (this kernel is bound by
-  // L2 -> SM traffic: every dY box is needed by all KI tiles and every X box by all NO tiles).
+  constexpr int BN = kWgradBN;
   constexpr uint32_t kBoxBytes = 64 * kBK * 2;  // [64 rows(k) x 64 cols(mn)] bf16 = 8 KB
   constexpr uint32_t kABytes = 2 * kBoxBytes;
   constexpr uint32_t kBBytes = (BN / 64) * kBoxBytes;
@@ -544,23 +518,14 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
   const int r_end = min(R, r_begin + rows_per_split);
   const int nkb = (r_end - r_begin + kBK - 1) / kBK;  // >= 1 by construction of the grid
   const bool do_bias = (dbias != nullptr) && (blockIdx.x == 0);
-  // cluster geometry: rank = x_local + cx * y_local; peers along x share dY, peers along y share X
-  const bool clustered = cx * cy > 1;
-  const uint32_t rank = clustered ? cluster_ctarank() : 0u;
-  const int xl = (int)rank % cx, yl = (int)rank / cx;
-  const uint16_t mask_x = (uint16_t)(cx == 2 ? (3u << (cx * yl)) : (1u << rank));                 // (0,yl) and (1,yl)
-  const uint16_t mask_y = (uint16_t)(cy == 2 ? ((1u << xl) | (1u << (xl + cx))) : (1u << rank));    // (xl,0) and (xl,1)
-  const uint16_t mask_free = (uint16_t)(mask_x | mask_y);      // CTAs whose loads land in this CTA's stages
-  const uint32_t n_free = (uint32_t)(1 + (cx == 2) + (cy == 2));
 
-  pdl_trigger();
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmY);
     tma_prefetch_desc(&tmX);
 #pragma unroll
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], n_free);   // this CTA and the peers it multicasts to have drained the stage
+      mbar_init(&empty_bar[s], 1);
     }
     mbar_init(&accum_bar, 1);
     fence_mbar_init();
@@ -576,10 +541,8 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
   }
   tc_fence_before();
   __syncthreads();
-  if (clustered) cluster_sync_all();   // every CTA's barriers are initialised before a peer's multicast can touch them
   tc_fence_after();
   const uint32_t tmem_base = tmem_slot;
-  pdl_wait();
 
   if (warp == 0) {
     if (elect_one()) {
@@ -597,19 +560,11 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
         const uint32_t a_dst = smem_base + s * kStageBytes;
         const int r0 = r_begin + kb * kBK;
         // rows_per_split is a multiple of kBK, so only the global tail (>= R) is zero-filled by TMA
-        if (cx == 2) {   // this CTA fetches dY box xl for both KI tiles of its cluster row
-          tma_load_2d_mc(a_dst + xl * kBoxBytes, &tmY, &full_bar[s], no0 + 64 * xl, r0, mask_x);
-        } else {
-          tma_load_2d_addr(a_dst, &tmY, &full_bar[s], no0, r0);
-          tma_load_2d_addr(a_dst + kBoxBytes, &tmY, &full_bar[s], no0 + 64, r0);
-        }
-        if (cy == 2) {   // ... and X box yl for both NO tiles of its cluster column
-          tma_load_2d_mc(a_dst + kABytes + yl * kBoxBytes, &tmX, &full_bar[s], ki0 + 64 * yl, r0, mask_y);
-        } else {
+        tma_load_2d_addr(a_dst, &tmY, &full_bar[s], no0, r0);
+        tma_load_2d_addr(a_dst + kBoxBytes, &tmY, &full_bar[s], no0 + 64, r0);
 #pragma unroll
-          for (int bx = 0; bx < BN / 64; ++bx)
-            tma_load_2d_addr(a_dst + kABytes + bx * kBoxBytes, &tmX, &full_bar[s], ki0 + 64 * bx, r0);
-        }
+        for (int bx = 0; bx < BN / 64; ++bx)
+          tma_load_2d_addr(a_dst + kABytes + bx * kBoxBytes, &tmX, &full_bar[s], ki0 + 64 * bx, r0);
       }
     }
   } else if (warp == 1) {
@@ -634,8 +589,7 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
             umma_bf16(tmem_base + BN, da, d1, idesc_b, (kb > 0 || k > 0) ? 1u : 0u);
           }
         }
-        if (clustered) umma_commit_mc(&empty_bar[s], mask_free);   // frees the stage here and tells the peers that feed it
-        else umma_commit(&empty_bar[s]);
+        umma_commit(&empty_bar[s]);
       }
       umma_commit(&accum_bar);
     }
@@ -664,53 +618,49 @@ __global__ void __launch_bounds__(kGemmThreads) gemm_wgrad_kernel(const __grid_c
       tmem_ld_wait();
       if constexpr (DET) {
         float* slot = reinterpret_cast<float*>(ws + (blockIdx.z + (long long)gridDim.z * (blockIdx.y * gridDim.x + blockIdx.x)) *
-                                                        wgrad_slot_f4<BN>());
+                                                        kWgradSlotF4);
         slot[kBM * BN + row_l] = __uint_as_float(bacc[0]);
       } else {
         if (no0 + row_l < NO) atomicAdd(dbias + no0 + row_l, __uint_as_float(bacc[0]));
       }
     }
     __syncwarp();
-    // coalesced accumulation: lane = 4 consecutive columns, one row (128 columns of it) per step
-#pragma unroll 1
-    for (int cp = 0; cp < BN / 128; ++cp) {
-      const int lcol = cp * 128 + lane * 4;
-      const int kcol = ki0 + lcol;
-      const int nvalid = KI - kcol;
-      const bool vec = (ldw % 4 == 0) && nvalid >= 4 && ((reinterpret_cast<uintptr_t>(dW) & 15) == 0);
+    // coalesced accumulation: lane = 4 consecutive columns, one row per step
+    const int lcol = lane * 4;
+    const int kcol = ki0 + lcol;
+    const int nvalid = KI - kcol;
+    const bool vec = (ldw % 4 == 0) && nvalid >= 4 && ((reinterpret_cast<uintptr_t>(dW) & 15) == 0);
 #pragma unroll 4
-      for (int it = 0; it < 32; ++it) {
-        const int rl = quad * 32 + it;
-        const int no = no0 + rl;
-        if (no >= NO || nvalid <= 0) continue;
-        const float4 v = *reinterpret_cast<const float4*>(stage_f + rl * kPitch + lcol);
-        if constexpr (DET) {
-          ws[(blockIdx.z + (long long)gridDim.z * (blockIdx.y * gridDim.x + blockIdx.x)) * wgrad_slot_f4<BN>() +
-             (rl * BN + lcol) / 4] = v;
-          continue;
-        }
-        float* dst = dW + (long long)no * ldw + kcol;
-        if (vec) {
-          asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(v.x), "f"(v.y), "f"(v.z),
-                       "f"(v.w)
-                       : "memory");
-        } else {
-          if (nvalid > 0) atomicAdd(dst, v.x);
-          if (nvalid > 1) atomicAdd(dst + 1, v.y);
-          if (nvalid > 2) atomicAdd(dst + 2, v.z);
-          if (nvalid > 3) atomicAdd(dst + 3, v.w);
-        }
+    for (int it = 0; it < 32; ++it) {
+      const int rl = quad * 32 + it;
+      const int no = no0 + rl;
+      if (no >= NO || nvalid <= 0) continue;
+      const float4 v = *reinterpret_cast<const float4*>(stage_f + rl * kPitch + lcol);
+      if constexpr (DET) {
+        ws[(blockIdx.z + (long long)gridDim.z * (blockIdx.y * gridDim.x + blockIdx.x)) * kWgradSlotF4 +
+           (rl * BN + lcol) / 4] = v;
+        continue;
+      }
+      float* dst = dW + (long long)no * ldw + kcol;
+      if (vec) {
+        asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(v.x), "f"(v.y), "f"(v.z),
+                     "f"(v.w)
+                     : "memory");
+      } else {
+        if (nvalid > 0) atomicAdd(dst, v.x);
+        if (nvalid > 1) atomicAdd(dst + 1, v.y);
+        if (nvalid > 2) atomicAdd(dst + 2, v.z);
+        if (nvalid > 3) atomicAdd(dst + 3, v.w);
       }
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (clustered) cluster_sync_all();   // no CTA leaves while a peer's commit may still arrive on its barriers
   if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
   if constexpr (DET) {
     const long long tile = blockIdx.y * gridDim.x + blockIdx.x;
     const bool vec = (ldw % 4 == 0) && ((reinterpret_cast<uintptr_t>(dW) & 15) == 0);
-    det_tree_fold(ws + tile * gridDim.z * wgrad_slot_f4<BN>(), wgrad_slot_f4<BN>(),
+    det_tree_fold(ws + tile * gridDim.z * kWgradSlotF4, kWgradSlotF4,
                   (kBM * BN + (do_bias ? kBM : 0)) / 4, blockIdx.z, gridDim.z, tickets + tile * gridDim.z,
                   [&](int i, float4 v) {
                     const int e = 4 * i;
@@ -829,27 +779,11 @@ static int launch_tn(const mmfm_gemm_args* a, cudaStream_t st) {
   }
   const int tiles_n = (a->N + BN - 1) / BN, tiles_m = (a->M + kBM - 1) / kBM;
   const int n_tiles = tiles_n * tiles_m;
-  int grid = n_tiles < device_sm_count() ? n_tiles : device_sm_count();
-  // weight-stationary schedule: B's whole K extent fits half of the ring area and the grid can be a multiple of tiles_n
-  // (measured neutral on B200 -- these GEMMs turned out to be bound by epilogue instruction issue, not by L2 -> SM
-  // traffic -- so the streamed-B schedule stays the default; MMFM_GEMM_BSTAT=1 enables it for A/B measurements)
-  static int bstat_env = -1;
-  if (bstat_env < 0) {
-    const char* e = getenv("MMFM_GEMM_BSTAT");
-    bstat_env = (e && e[0] == '1') ? 1 : 0;
-  }
-  const int nkb = (a->K + kBK - 1) / kBK;
-  int bstat = 0;
-  if (bstat_env && (size_t)nkb * BN * kBK * 2 * 2 <= (size_t)STAGES * (kBM * kBK * 2 + BN * kBK * 2) &&
-      tiles_n <= device_sm_count() && tiles_m > 1) {
-    int per_n = device_sm_count() / tiles_n;
-    if (per_n > tiles_m) per_n = tiles_m;
-    grid = per_n * tiles_n;
-    bstat = 1;
-  }
-  set_l2_window(a->D, (size_t)a->M * (size_t)a->ldd * (a->d_fp32 ? 4 : 2));   // the output is the next kernel's input
-  MMFM_CHECK_CUDA(launch_pdl(gemm_tn_kernel<BN, STAGES, EPI>, dim3(grid), dim3(kTnThreads), smem, st, tmA, tmB, *a, tiles_n,
-                             n_tiles, bstat));
+  // B streams through the ring with A: a weight-stationary schedule (B's K extent resident in shared memory) measured
+  // neutral on B200, these GEMMs being bound by epilogue instruction issue rather than by L2 -> SM traffic
+  const int grid = n_tiles < device_sm_count() ? n_tiles : device_sm_count();
+  gemm_tn_kernel<BN, STAGES, EPI><<<grid, kTnThreads, smem, st>>>(tmA, tmB, *a, tiles_n, n_tiles);
+  MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -929,29 +863,22 @@ extern "C" int mmfm_gemm_tn(const mmfm_gemm_args* a, void* stream) {
 }
 
 // split-R arithmetic of the wgrad launch (also the deterministic workspace size: one slot per CTA)
-static int wgrad_splits(int R, int NO, int KI, int BN, int* rows_per_split) {
-  const int tiles = ((NO + kBM - 1) / kBM) * ((KI + BN - 1) / BN);
+static int wgrad_splits(int R, int NO, int KI, int* rows_per_split) {
+  const int tiles = ((NO + kBM - 1) / kBM) * ((KI + kWgradBN - 1) / kWgradBN);
   const int kblocks = (R + kBK - 1) / kBK;
-  static int waves_x2 = -1;   // MMFM_WGRAD_CTAS_X2: target CTA count in half-SM-counts (default 4 = two CTAs per SM)
-  if (waves_x2 < 0) {
-    const char* e = getenv("MMFM_WGRAD_CTAS_X2");
-    waves_x2 = e ? atoi(e) : 4;
-    if (waves_x2 < 1) waves_x2 = 4;
-  }
   // all CTAs must be resident at once (two per SM): a split count rounded UP spills a few CTAs into a second wave that
   // costs as much as the first (measured 43 us vs 34 us on the QKV shape), so round down
-  // BN 256: one CTA per SM (144 KB of stages, 512 TMEM columns); BN 128: two
-  int splits = ((BN == 256 ? 2 : waves_x2) * device_sm_count() / 2) / tiles;
+  int splits = 2 * device_sm_count() / tiles;
   if (splits > kblocks) splits = kblocks;
   if (splits < 1) splits = 1;
   *rows_per_split = ((kblocks + splits - 1) / splits) * kBK;
   return (R + *rows_per_split - 1) / *rows_per_split;
 }
 
-template <int BN>
+template <bool DET>
 static int launch_wgrad(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI, float* dW,
-                        long long ldw, float* dbias, void* stream) {
-  constexpr int STAGES = 3;
+                        long long ldw, float* dbias, float4* ws, unsigned int* tickets, cudaStream_t st) {
+  constexpr int STAGES = 3, BN = kWgradBN;
   CUtensorMap tmY, tmX;
   int rc = make_tmap_bf16_2d(&tmY, dY, (uint64_t)R, (uint64_t)NO, (uint64_t)lddy, 64, kBK, TMA_SW_128);
   if (rc) return rc;
@@ -960,71 +887,24 @@ static int launch_wgrad(const void* dY, long long lddy, const void* X, long long
   constexpr size_t smem = (size_t)STAGES * ((2 + BN / 64) * 64 * kBK * 2) + 2048 + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    MMFM_CHECK_CUDA(cudaFuncSetAttribute(gemm_wgrad_kernel<STAGES, BN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    MMFM_CHECK_CUDA(cudaFuncSetAttribute(gemm_wgrad_kernel<STAGES, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem));
     attr_set = true;
   }
   int rows_per_split = 0;
-  const int splits = wgrad_splits(R, NO, KI, BN, &rows_per_split);
-  dim3 grid((KI + BN - 1) / BN, (NO + kBM - 1) / kBM, splits);
-  static int mc_env = -1;   // MMFM_WGRAD_MULTICAST=1: 2x2 clusters, each CTA loads half of its boxes and multicasts them
-  if (mc_env < 0) {
-    const char* e = getenv("MMFM_WGRAD_MULTICAST");
-    mc_env = (e && e[0] == '1') ? 1 : 0;   // measured slower than independent CTAs (lock-step stages): off by default
-  }
-  const int cx = (mc_env && BN == 128 && grid.x % 2 == 0) ? 2 : 1, cy = (mc_env && BN == 128 && grid.y % 2 == 0) ? 2 : 1;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(kGemmThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = (cudaStream_t)stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = cx;
-  attr[0].val.clusterDim.y = cy;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  MMFM_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_wgrad_kernel<STAGES, BN>, tmY, tmX, R, NO, KI, dW, ldw, rows_per_split, dbias,
-                                     cx, cy, (float4*)nullptr, (unsigned int*)nullptr));
+  const int splits = wgrad_splits(R, NO, KI, &rows_per_split);
+  const dim3 grid((KI + BN - 1) / BN, (NO + kBM - 1) / kBM, splits);
+  gemm_wgrad_kernel<STAGES, DET><<<grid, kGemmThreads, smem, st>>>(tmY, tmX, R, NO, KI, dW, ldw, rows_per_split, dbias,
+                                                                  ws, tickets);
+  MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
-// deterministic twin: always the 128-wide tile without clusters (MMFM_WGRAD_BN / MMFM_WGRAD_MULTICAST do not apply)
 static DetNeed wgrad_det_need(int R, int NO, int KI) {
   int rows_per_split = 0;
-  const int splits = wgrad_splits(R, NO, KI, 128, &rows_per_split);
-  const long long ctas = (long long)((NO + kBM - 1) / kBM) * ((KI + 127) / 128) * splits;
-  return DetNeed{ctas * wgrad_slot_f4<128>() * 16, (int)ctas};
-}
-
-static int launch_wgrad_det(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI,
-                            float* dW, long long ldw, float* dbias, const mmfm_det_ws* ws, cudaStream_t st) {
-  constexpr int STAGES = 3, BN = 128;
-  MMFM_REQUIRE(ws != nullptr, "mmfm_gemm_wgrad_det: null workspace");
-  if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, wgrad_det_need(R, NO, KI),
-                            "mmfm_gemm_wgrad_det"))
-    return rc;
-  CUtensorMap tmY, tmX;
-  int rc = make_tmap_bf16_2d(&tmY, dY, (uint64_t)R, (uint64_t)NO, (uint64_t)lddy, 64, kBK, TMA_SW_128);
-  if (rc) return rc;
-  rc = make_tmap_bf16_2d(&tmX, X, (uint64_t)R, (uint64_t)KI, (uint64_t)ldx, 64, kBK, TMA_SW_128);
-  if (rc) return rc;
-  constexpr size_t smem = (size_t)STAGES * ((2 + BN / 64) * 64 * kBK * 2) + 2048 + 1024;
-  static bool attr_set = false;
-  if (!attr_set) {
-    MMFM_CHECK_CUDA(cudaFuncSetAttribute(gemm_wgrad_kernel<STAGES, BN, true>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
-  int rows_per_split = 0;
-  const int splits = wgrad_splits(R, NO, KI, BN, &rows_per_split);
-  MMFM_CHECK_CUDA(launch_pdl(gemm_wgrad_kernel<STAGES, BN, true>, dim3((KI + BN - 1) / BN, (NO + kBM - 1) / kBM, splits),
-                             dim3(kGemmThreads), smem, st, tmY, tmX, R, NO, KI, dW, ldw, rows_per_split, dbias, 1, 1,
-                             (float4*)ws->buf, ws->tickets));
-  return 0;
+  const int splits = wgrad_splits(R, NO, KI, &rows_per_split);
+  const long long ctas = (long long)((NO + kBM - 1) / kBM) * ((KI + kWgradBN - 1) / kWgradBN) * splits;
+  return DetNeed{ctas * kWgradSlotF4 * 16, (int)ctas};
 }
 
 static DetNeed colsum_det_need(int R, int NO) {
@@ -1046,20 +926,19 @@ extern "C" int mmfm_gemm_wgrad(const void* dY, long long lddy, const void* X, lo
                                float* dW, long long ldw, float* dbias, void* stream) {
   MMFM_REQUIRE(dY && X && dW, "mmfm_gemm_wgrad: null operand");
   MMFM_REQUIRE(R > 0 && NO > 0 && KI > 0, "mmfm_gemm_wgrad: bad shape R=%d NO=%d KI=%d", R, NO, KI);
-  static int bn_env = -1;   // MMFM_WGRAD_BN=128 pins the 128-wide dW tile (A/B measurements)
-  if (bn_env < 0) {
-    const char* e = getenv("MMFM_WGRAD_BN");
-    bn_env = e ? atoi(e) : 128;   // the 256-wide tile measured equal (QKV 29.4 vs 29.8 us) to slower (down 25.7 vs 23.4 us)
-  }
-  if (bn_env == 256 && KI % 256 == 0) return launch_wgrad<256>(dY, lddy, X, ldx, R, NO, KI, dW, ldw, dbias, stream);
-  return launch_wgrad<128>(dY, lddy, X, ldx, R, NO, KI, dW, ldw, dbias, stream);
+  return launch_wgrad<false>(dY, lddy, X, ldx, R, NO, KI, dW, ldw, dbias, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int mmfm_gemm_wgrad_det(const void* dY, long long lddy, const void* X, long long ldx, int R, int NO, int KI,
                                    float* dW, long long ldw, float* dbias, const mmfm_det_ws* ws, void* stream) {
   MMFM_REQUIRE(dY && X && dW, "mmfm_gemm_wgrad_det: null operand");
   MMFM_REQUIRE(R > 0 && NO > 0 && KI > 0, "mmfm_gemm_wgrad_det: bad shape R=%d NO=%d KI=%d", R, NO, KI);
-  return launch_wgrad_det(dY, lddy, X, ldx, R, NO, KI, dW, ldw, dbias, ws, (cudaStream_t)stream);
+  MMFM_REQUIRE(ws != nullptr, "mmfm_gemm_wgrad_det: null workspace");
+  if (int rc = det_ws_check(ws->buf, ws->bytes, ws->tickets, ws->n_tickets, wgrad_det_need(R, NO, KI),
+                            "mmfm_gemm_wgrad_det"))
+    return rc;
+  return launch_wgrad<true>(dY, lddy, X, ldx, R, NO, KI, dW, ldw, dbias, (float4*)ws->buf, ws->tickets,
+                            (cudaStream_t)stream);
 }
 
 extern "C" int mmfm_colsum_bf16(const void* dY, long long ld, int R, int NO, float* out, void* stream) {

@@ -11,21 +11,16 @@
 //     row-per-thread accesses) -> fence.proxy.async -> mbarrier arrive.  No global memory instruction at all.
 //   * warp 2 (store): one elected lane issues cp.async.bulk.tensor stores of the tile's four [128 x 32] boxes (UTMASTG)
 //     and recycles the staging buffer when the TMA unit has read it.  Edge tiles are clipped by the tensor map.
-//   * warp 3 (input): residual (fp32) or saved-tensor (bf16) boxes of a tile are TMA-loaded INTO the staging buffer
+//   * warp 3 (input): saved-tensor (bf16) boxes of a tile are TMA-loaded INTO the staging buffer
 //     two tiles ahead; the epilogue combines them in place, so they cost neither registers nor extra shared memory.
 //   * warp 0 (A/B ring producer) and warp 1 (TMEM allocation + tcgen05.mma issue, double-buffered accumulator) as in
 //     gemm_tn_kernel.
 // Staging is double-buffered, so the MMA of tile i+1, the epilogue of tile i and the store of tile i-1 overlap.
 //
-// Weight-stationary schedule (`bstat`): these skinny-K GEMMs are bound by the chip-wide L2 -> SM throughput (~6300 B/clk
-// = 12 TB/s; B300_MICROARCH.md "LTS throughput cap"): ncu shows 315 MB of TMA loads for the 26 MB activation of the QKV
-// call (every 128 x 128 tile re-reads its 64 KB slab of the weight) and the duration equals (loads + stores) / 12 TB/s.
-// When the weight slab of a column tile ([128 x K] bf16, K <= 256; K <= 512 for single bf16 outputs) fits beside the
-// staging buffers, the grid is rounded to a multiple of the column-tile count, every CTA keeps ITS slab resident for
-// the whole kernel and the ring carries activation k-blocks only: the QKV call drops from 393 MB to 236 MB of L2
-// traffic.  MMFM_GEMM_TS_BSTAT=0 switches it off.
+// A and B stream through the ring together.  A weight-stationary schedule (each CTA keeping its column tile's [BN x K]
+// weight slab resident, the ring carrying activation k-blocks only) cut the QKV call's L2 -> SM traffic from 393 MB to
+// 236 MB but measured neutral to slower on B200: the A-only ring it leaves room for is too shallow.
 #include "common.cuh"
-#include <stdlib.h>
 #include "host_util.h"
 #include "../../include/mmfm_b200.h"
 
@@ -59,7 +54,6 @@ enum TsEpi : int {
   TS_BF16 = 0,       // D(bf16) = v
   TS_SOFTSIGN = 1,   // D(bf16) = softsign(v) * s
   TS_F32 = 2,        // D(f32)  = v
-  TS_RES = 3,        // D(f32)  = res + dropout(v)
   TS_GELU_DG = 4,    // D(bf16) = gelu(v) ; D2(bf16) = gelu'(v)
   TS_MULAUX = 5,     // D(bf16) = v * aux
   TS_DSOFTSIGN = 6,  // D(bf16) = v * s * (1 - |aux / s|)^2
@@ -68,15 +62,15 @@ enum TsEpi : int {
 
 template <int EPI>
 struct TsCfg {
-  static constexpr bool kF32 = EPI == TS_F32 || EPI == TS_RES;
-  static constexpr bool kHasIn = EPI == TS_RES || EPI == TS_MULAUX || EPI == TS_DSOFTSIGN || EPI == TS_ROWDOT;
+  static constexpr bool kF32 = EPI == TS_F32;
+  static constexpr bool kHasIn = EPI == TS_MULAUX || EPI == TS_DSOFTSIGN || EPI == TS_ROWDOT;
   static constexpr bool kTwoOut = EPI == TS_GELU_DG;
   static constexpr uint32_t kRowBytes = kF32 ? 128u : 64u;          // one box row: 32 columns
   static constexpr uint32_t kSlice = 128u * kRowBytes;              // one [128 x 32] box
   static constexpr uint32_t kOut = 4u * kSlice;                     // one output tile
   static constexpr uint32_t kBuf = kOut * (kTwoOut ? 2u : 1u);      // one staging buffer
 };
-constexpr int kTsMaxStages = 6;
+constexpr int kTsMaxStages = 4;
 constexpr size_t kTsMaxSmem = 230400;   // 225 KB dynamic (+ static barriers) of the 227 KB a CTA may own
 
 // BN = 256: the tile is 128 x 256 (fp32 accumulator 2 x 256 TMEM columns).  Every byte of an A / B tile is read from
@@ -92,7 +86,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
                                                                     const __grid_constant__ CUtensorMap tmD2,
                                                                     const __grid_constant__ CUtensorMap tmIn,
                                                                     const mmfm_gemm_args p, int tiles_n, int n_tiles,
-                                                                    int bstat, int nst) {
+                                                                    int nst) {
   using Cfg = TsCfg<EPI>;
   constexpr int STAGES = kTsMaxStages;
   constexpr uint32_t kABytes = kTsBM * kTsBK * 2, kBBytes = BN * kTsBK * 2;
@@ -101,7 +95,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
   constexpr int kTsBN = BN;
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[STAGES], empty_bar[STAGES];
-  __shared__ __align__(8) uint64_t acc_full[2], acc_empty[2], in_full[2], stg_full[2], stg_free[2], b_full;
+  __shared__ __align__(8) uint64_t acc_full[2], acc_empty[2], in_full[2], stg_full[2], stg_free[2];
   __shared__ uint32_t tmem_slot;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -110,17 +104,13 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
 #ifdef MMFM_DBG_TIMING
   if (threadIdx.x == 0 && blockIdx.x < 160) g_dbg_cta[blockIdx.x][0] = dbg_now();
 #endif
-  // shared memory: [resident weight slab (bstat)] [ring: nst stages of A (+ B when streamed)] [2 staging buffers]
+  // shared memory: [ring: nst stages of A + B] [2 staging buffers]
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem_al = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t b_res = bstat ? (uint32_t)nkb * kBBytes : 0u;
-  const uint32_t st_bytes = bstat ? kABytes : kTsStageBytes;
-  const uint32_t ring_base = smem_base + b_res;
-  const uint32_t stg_off = b_res + (uint32_t)nst * st_bytes;
+  const uint32_t stg_off = (uint32_t)nst * kTsStageBytes;
   const uint32_t stg_base = smem_base + stg_off;                      // staging buffers (1024-aligned)
   uint8_t* stg_ptr = smem_al + stg_off;
 
-  pdl_trigger();
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
@@ -140,7 +130,6 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
       mbar_init(&stg_full[i], kTsEpiWarps);
       mbar_init(&stg_free[i], 1);
     }
-    mbar_init(&b_full, 1);
     fence_mbar_init();
   }
   if (warp == 1) {
@@ -151,27 +140,21 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = tmem_slot;
-  pdl_wait();      // barriers / TMEM are set up; from here on global memory of the preceding kernels is touched
 
   if (warp == 0) {
     // ------------------------------------------------ A / B ring producer ------------------------------------------
     if (elect_one()) {
       uint32_t it = 0;
       const uint32_t ns = (uint32_t)nst;
-      if (bstat) {   // the grid is a multiple of tiles_n: every tile of this CTA has the same column block
-        const int n0 = ((int)blockIdx.x % tiles_n) * kTsBN;
-        mbar_arrive_expect_tx(&b_full, b_res);
-        for (int kb = 0; kb < nkb; ++kb) tma_load_2d_addr(smem_base + kb * kBBytes, &tmB, &b_full, kb * kTsBK, n0);
-      }
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int m0 = (tile / tiles_n) * kTsBM, n0 = (tile % tiles_n) * kTsBN;
         for (int kb = 0; kb < nkb; ++kb, ++it) {
           const uint32_t s = it % ns;
           if (it >= ns) mbar_wait(&empty_bar[s], ((it / ns) - 1) & 1);
-          mbar_arrive_expect_tx(&full_bar[s], st_bytes);
-          const uint32_t a_dst = ring_base + s * st_bytes;
+          mbar_arrive_expect_tx(&full_bar[s], kTsStageBytes);
+          const uint32_t a_dst = smem_base + s * kTsStageBytes;
           tma_load_2d_addr(a_dst, &tmA, &full_bar[s], kb * kTsBK, m0);
-          if (!bstat) tma_load_2d_addr(a_dst + kABytes, &tmB, &full_bar[s], kb * kTsBK, n0);
+          tma_load_2d_addr(a_dst + kABytes, &tmB, &full_bar[s], kb * kTsBK, n0);
         }
         DBG_TS(0, (int)(it / (uint32_t)nkb) - 1);      // all k-blocks of the tile issued
       }
@@ -182,7 +165,6 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
       const uint32_t idesc = make_idesc_bf16(kTsBM, kTsBN, 0, 0);
       uint32_t it = 0, t = 0;
       const uint32_t ns = (uint32_t)nst;
-      if (bstat) mbar_wait(&b_full, 0);
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++t) {
         const uint32_t buf = t & 1u;
         if (t >= 2) mbar_wait(&acc_empty[buf], ((t >> 1) - 1) & 1);
@@ -192,8 +174,8 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
           const uint32_t s = it % ns;
           mbar_wait(&full_bar[s], (it / ns) & 1);
           tc_fence_after();
-          const uint32_t a_addr = ring_base + s * st_bytes;
-          const uint32_t b_addr = bstat ? smem_base + kb * kBBytes : a_addr + kABytes;
+          const uint32_t a_addr = smem_base + s * kTsStageBytes;
+          const uint32_t b_addr = a_addr + kABytes;
 #pragma unroll
           for (int k = 0; k < kTsBK / 16; ++k)
             umma_bf16(d_tmem, make_smem_desc(a_addr + k * 32, 16, 1024, 2), make_smem_desc(b_addr + k * 32, 16, 1024, 2),
@@ -234,7 +216,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
       bulk_wait_group<0>();
     }
   } else if (warp == 3) {
-    // ------------------------------------------------ input warp: residual / saved-tensor boxes ---------------------
+    // ------------------------------------------------ input warp: saved-tensor boxes ------------------------------
     if (Cfg::kHasIn && elect_one()) {
       uint32_t u = 0;
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -266,7 +248,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
     const int row = quad * 32 + lane;
     bool drop = false;
     unsigned long long seed = 0ull;
-    if (EPI == TS_RES || EPI == TS_ROWDOT) {
+    if (EPI == TS_ROWDOT) {
       drop = p.drop.thresh != 0u;
       if (drop) seed = *p.drop.seed;
     }
@@ -320,19 +302,7 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
 #pragma unroll
             for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(acc[j]);
           }
-          if (EPI == TS_RES) {
-            if (drop) {
-              const uint4 w = drop_bytes16(seed, p.drop.site, (uint64_t)r, drop_gpr, (uint32_t)((nb + c0) >> 4));
-#pragma unroll
-              for (int j = 0; j < 16; ++j) v[j] = (drop_byte(w, j) < p.drop.thresh) ? 0.f : v[j] * p.drop.scale;
-            }
-#pragma unroll
-            for (int j4 = 0; j4 < 4; ++j4) {      // residual box is in place: combine and write back
-              float4* q = reinterpret_cast<float4*>(box + ((((uint32_t)(c0 >> 2) + j4) ^ swz) << 4));
-              const float4 rv = *q;
-              *q = make_float4(v[4 * j4] + rv.x, v[4 * j4 + 1] + rv.y, v[4 * j4 + 2] + rv.z, v[4 * j4 + 3] + rv.w);
-            }
-          } else if (EPI == TS_F32) {
+          if (EPI == TS_F32) {
 #pragma unroll
             for (int j4 = 0; j4 < 4; ++j4)
               *reinterpret_cast<float4*>(box + ((((uint32_t)(c0 >> 2) + j4) ^ swz) << 4)) =
@@ -442,8 +412,7 @@ static int launch_ts_bn(const mmfm_gemm_args* a, cudaStream_t st) {
     rc = make_tmap_bf16_2d(&tmD2, a->D2, (uint64_t)a->M, (uint64_t)a->N, (uint64_t)a->ldd, 32, 128, TMA_SW_64);
     if (rc) return rc;
   }
-  if (EPI == TS_RES) rc = make_tmap_f32_2d(&tmIn, a->res, (uint64_t)a->M, (uint64_t)a->N, (uint64_t)a->ldr, 32, 128, TMA_SW_128);
-  else if (Cfg::kHasIn) rc = make_tmap_bf16_2d(&tmIn, a->aux, (uint64_t)a->M, (uint64_t)a->N, (uint64_t)a->ldaux, 32, 128, TMA_SW_64);
+  if (Cfg::kHasIn) rc = make_tmap_bf16_2d(&tmIn, a->aux, (uint64_t)a->M, (uint64_t)a->N, (uint64_t)a->ldaux, 32, 128, TMA_SW_64);
   if (rc) return rc;
   static bool attr_set = false;
   if (!attr_set) {
@@ -452,45 +421,21 @@ static int launch_ts_bn(const mmfm_gemm_args* a, cudaStream_t st) {
   }
   const int tiles_n = (a->N + BN - 1) / BN, tiles_m = (a->M + kTsBM - 1) / kTsBM;
   const int n_tiles = tiles_n * tiles_m;
-  const int sms = device_sm_count();
-  int grid = n_tiles < sms ? n_tiles : sms;
-  const size_t a_stage = (size_t)kTsBM * kTsBK * 2, b_stage = (size_t)BN * kTsBK * 2;
-  // streamed schedule: as many A + B stages as fit beside the two staging buffers (at most 4)
-  size_t room = (kTsMaxSmem - 1024 - 2 * (size_t)Cfg::kBuf) / (a_stage + b_stage);
-  int nst = room > 4 ? 4 : (int)room, bstat = 0;
-  size_t smem = 1024 + (size_t)nst * (a_stage + b_stage) + 2 * (size_t)Cfg::kBuf;
-  static int bstat_env = -1;
-  if (bstat_env < 0) {
-    const char* e = getenv("MMFM_GEMM_TS_BSTAT");
-    bstat_env = (e && e[0] == '1') ? 1 : 0;     // measured neutral to slower (the A-only ring is too shallow): opt-in
-  }
-  // weight-stationary schedule: the column tile's whole K extent of B stays resident, the ring carries A only
-  const int nkb = (a->K + kTsBK - 1) / kTsBK;
-  const size_t b_res = (size_t)nkb * b_stage;
-  if (bstat_env && tiles_n <= sms && tiles_m >= 2 * (sms / tiles_n) &&
-      1024 + b_res + 2 * a_stage + 2 * (size_t)Cfg::kBuf <= kTsMaxSmem) {
-    room = (kTsMaxSmem - 1024 - b_res - 2 * (size_t)Cfg::kBuf) / a_stage;
-    nst = room > (size_t)kTsMaxStages ? kTsMaxStages : (int)room;
-    bstat = 1;
-    grid = (sms / tiles_n) * tiles_n;
-    smem = 1024 + b_res + (size_t)nst * a_stage + 2 * (size_t)Cfg::kBuf;
-  }
-  set_l2_window(a->D, (size_t)a->M * (size_t)a->ldd * (a->d_fp32 ? 4 : 2));   // the output is the next kernel's input
-  MMFM_CHECK_CUDA(launch_pdl(gemm_tn_ts_kernel<EPI, BN>, dim3(grid), dim3(kTsThreads), smem, st, tmA, tmB, tmD, tmD2, tmIn, *a,
-                             tiles_n, n_tiles, bstat, nst));
+  const int grid = n_tiles < device_sm_count() ? n_tiles : device_sm_count();
+  // as many A + B stages as fit beside the two staging buffers (at most kTsMaxStages)
+  const size_t stage = (size_t)(kTsBM + BN) * kTsBK * 2;
+  const size_t room = (kTsMaxSmem - 1024 - 2 * (size_t)Cfg::kBuf) / stage;
+  const int nst = room > (size_t)kTsMaxStages ? kTsMaxStages : (int)room;
+  const size_t smem = 1024 + (size_t)nst * stage + 2 * (size_t)Cfg::kBuf;
+  gemm_tn_ts_kernel<EPI, BN><<<grid, kTsThreads, smem, st>>>(tmA, tmB, tmD, tmD2, tmIn, *a, tiles_n, n_tiles, nst);
+  MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
-// 256-wide tiles when N is a multiple of 256 (the model's 256 / 512 / 768-column projections); MMFM_GEMM_TS_BN=128 pins
-// the 128-wide tile (A/B measurements)
+// 256-wide tiles when N is a multiple of 256 (the model's 256 / 512 / 768-column projections)
 template <int EPI>
 static int launch_ts(const mmfm_gemm_args* a, cudaStream_t st) {
-  static int bn_env = -1;
-  if (bn_env < 0) {
-    const char* e = getenv("MMFM_GEMM_TS_BN");
-    bn_env = e ? atoi(e) : 256;
-  }
-  if (bn_env == 256 && a->N % 256 == 0) return launch_ts_bn<EPI, 256>(a, st);
+  if (a->N % 256 == 0) return launch_ts_bn<EPI, 256>(a, st);
   return launch_ts_bn<EPI, 128>(a, st);
 }
 
@@ -499,69 +444,51 @@ namespace mmfm {
 static bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 // Returns 1 when the call was taken by the TMA-store kernel, 0 when it does not fit (the caller falls back to
-// gemm_tn_kernel), < 0 on error.  MMFM_GEMM_TS=0 disables the path (A/B measurements).
+// gemm_tn_kernel), < 0 on error.
 int try_launch_gemm_ts(const mmfm_gemm_args* a, cudaStream_t st) {
-  static int enabled = -1;
-  if (enabled < 0) {
-    const char* e = getenv("MMFM_GEMM_TS");
-    enabled = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (!enabled) return 0;
   if (a->N <= 64 || a->N % 4 != 0 || a->remap_T > 0 || a->row_zero != nullptr) return 0;
   const bool f32 = a->d_fp32 != 0;
   const int esz = f32 ? 4 : 2;
   if (!al16(a->D) || (a->ldd * esz) % 16 != 0) return 0;
   if (a->bias && !al16(a->bias)) return 0;
   const bool drop = a->drop.thresh != 0;
+  // fp32 + residual stays on gemm_tn_kernel: here it measured 2-3 us SLOWER (28.1 vs 26.4 us out-proj, 37.3 vs 34.4 us
+  // down-proj, graph-timed): the residual box travels TMA -> shared memory -> registers -> shared memory -> TMA, twice
+  // the shared-memory bytes of the staged epilogue, and shared-memory bandwidth is what the main loop competes for.
+  if (a->res) return 0;
+  if (drop && a->act != MMFM_ACT_ROWDOT_DROP) return 0;
   int epi = -1;
-  if (a->res) {
-    // fp32 + residual: measured 2-3 us SLOWER here than in gemm_tn_kernel (28.1 vs 26.4 us out-proj, 37.3 vs 34.4 us
-    // down-proj, graph-timed): the residual box travels TMA -> shared memory -> registers -> shared memory -> TMA, twice
-    // the shared-memory bytes of the staged epilogue, and shared-memory bandwidth is what the main loop competes for.
-    // MMFM_GEMM_TS_RES=1 routes it here anyway (A/B measurements).
-    static int res_env = -1;
-    if (res_env < 0) {
-      const char* e = getenv("MMFM_GEMM_TS_RES");
-      res_env = (e && e[0] == '1') ? 1 : 0;
-    }
-    if (!res_env) return 0;
-    if (a->act != MMFM_ACT_NONE || !f32 || a->D2 || !al16(a->res) || (a->ldr * 4) % 16 != 0) return 0;
-    epi = TS_RES;
-  } else {
-    if (drop && a->act != MMFM_ACT_ROWDOT_DROP) return 0;
-    switch (a->act) {
-      case MMFM_ACT_NONE:
-        if (a->D2) return 0;
-        epi = f32 ? TS_F32 : TS_BF16;
-        break;
-      case MMFM_ACT_SOFTSIGN:
-        if (f32 || a->D2) return 0;
-        epi = TS_SOFTSIGN;
-        break;
-      case MMFM_ACT_GELU_DG:
-        if (f32 || !a->D2 || !al16(a->D2)) return 0;
-        epi = TS_GELU_DG;
-        break;
-      case MMFM_ACT_MULAUX:
-      case MMFM_ACT_DSOFTSIGN:
-        if (f32 || a->D2 || !a->aux || !al16(a->aux) || (a->ldaux * 2) % 16 != 0) return 0;
-        epi = a->act == MMFM_ACT_MULAUX ? TS_MULAUX : TS_DSOFTSIGN;
-        break;
-      case MMFM_ACT_ROWDOT_DROP:
-        if (f32 || a->D2 || a->bias || !a->aux || !al16(a->aux) || (a->ldaux * 2) % 16 != 0 || a->N % 32 != 0 || !a->rowdot)
-          return 0;
-        epi = TS_ROWDOT;
-        break;
-      default:
+  switch (a->act) {
+    case MMFM_ACT_NONE:
+      if (a->D2) return 0;
+      epi = f32 ? TS_F32 : TS_BF16;
+      break;
+    case MMFM_ACT_SOFTSIGN:
+      if (f32 || a->D2) return 0;
+      epi = TS_SOFTSIGN;
+      break;
+    case MMFM_ACT_GELU_DG:
+      if (f32 || !a->D2 || !al16(a->D2)) return 0;
+      epi = TS_GELU_DG;
+      break;
+    case MMFM_ACT_MULAUX:
+    case MMFM_ACT_DSOFTSIGN:
+      if (f32 || a->D2 || !a->aux || !al16(a->aux) || (a->ldaux * 2) % 16 != 0) return 0;
+      epi = a->act == MMFM_ACT_MULAUX ? TS_MULAUX : TS_DSOFTSIGN;
+      break;
+    case MMFM_ACT_ROWDOT_DROP:
+      if (f32 || a->D2 || a->bias || !a->aux || !al16(a->aux) || (a->ldaux * 2) % 16 != 0 || a->N % 32 != 0 || !a->rowdot)
         return 0;
-    }
+      epi = TS_ROWDOT;
+      break;
+    default:
+      return 0;
   }
   int rc = 0;
   switch (epi) {
     case TS_BF16: rc = launch_ts<TS_BF16>(a, st); break;
     case TS_SOFTSIGN: rc = launch_ts<TS_SOFTSIGN>(a, st); break;
     case TS_F32: rc = launch_ts<TS_F32>(a, st); break;
-    case TS_RES: rc = launch_ts<TS_RES>(a, st); break;
     case TS_GELU_DG: rc = launch_ts<TS_GELU_DG>(a, st); break;
     case TS_MULAUX: rc = launch_ts<TS_MULAUX>(a, st); break;
     case TS_DSOFTSIGN: rc = launch_ts<TS_DSOFTSIGN>(a, st); break;

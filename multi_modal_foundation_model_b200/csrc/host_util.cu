@@ -2,7 +2,6 @@
 #include "../../include/mmfm_b200.h"
 
 #include <stdarg.h>
-#include <stdlib.h>
 
 #include <mutex>
 
@@ -94,62 +93,6 @@ int make_tmap_bf16_3d(CUtensorMap* out, const void* base, uint64_t batch, uint64
                (int)r, (unsigned long long)batch, (unsigned long long)rows, (unsigned long long)cols,
                (unsigned long long)ld, box_cols, box_rows);
   return 0;
-}
-
-bool pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("MMFM_PDL");
-    on = (e && e[0] == '1') ? 1 : 0;   // measured neutral on the default step (23 181 vs 23 319 trials/s): opt-in
-  }
-  return on != 0;
-}
-
-static thread_local const void* g_win_ptr = nullptr;
-static thread_local size_t g_win_bytes = 0;
-
-static int l2_persist_state() {   // -1 off, else the maximum window size in MB
-  static int state = -2;
-  if (state == -2) {
-    const char* e = getenv("MMFM_L2_PERSIST");
-    state = -1;
-    if (e && e[0] == '1') {
-      int dev = 0, max_persist = 0, max_win = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev);
-      cudaDeviceGetAttribute(&max_win, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-      const char* mb = getenv("MMFM_L2_PERSIST_MB");       // set-aside = largest window taken (default: the device maximum)
-      if (mb && atoi(mb) > 0 && ((size_t)atoi(mb) << 20) < (size_t)max_persist) max_persist = atoi(mb) << 20;
-      if (max_persist > 0 && max_win > 0 &&
-          cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist) == cudaSuccess) {
-        state = max_persist >> 20;
-        if (getenv("MMFM_L2_PERSIST_VERBOSE"))
-          fprintf(stderr, "mmfm: persisting L2 set-aside %d MB, window limit %d MB\n", max_persist >> 20, max_win >> 20);
-      }
-    }
-  }
-  return state;
-}
-
-void set_l2_window(const void* ptr, size_t bytes) {
-  g_win_ptr = ptr;
-  g_win_bytes = bytes;
-}
-
-bool take_l2_window(cudaAccessPolicyWindow* w) {
-  const void* ptr = g_win_ptr;
-  const size_t bytes = g_win_bytes;
-  g_win_ptr = nullptr;
-  g_win_bytes = 0;
-  const int lim = l2_persist_state();
-  if (lim < 0 || ptr == nullptr || bytes == 0) return false;
-  if (bytes > ((size_t)lim << 20)) return false;   // an output larger than the set-aside would only thrash it
-  w->base_ptr = const_cast<void*>(ptr);
-  w->num_bytes = bytes;
-  w->hitRatio = 1.0f;
-  w->hitProp = cudaAccessPropertyPersisting;
-  w->missProp = cudaAccessPropertyStreaming;
-  return true;
 }
 
 int device_sm_count() {

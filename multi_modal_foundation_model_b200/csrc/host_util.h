@@ -60,37 +60,4 @@ bool det_need_glue(int kind, long long d0, long long d1, long long d2, DetNeed* 
 int det_ws_check(const void* buf, long long bytes, const unsigned int* tickets, int n_tickets, const DetNeed& need,
                  const char* who);
 
-// MMFM_PDL=1 (default 0: measured neutral): launch the hot kernels with programmatic stream serialization (see
-// common.cuh: pdl_enter)
-bool pdl_enabled();
-
-// L2 residency between producer and consumer kernels (MMFM_L2_PERSIST=1; off: measured neutral at a 27 MB set-aside and
-// slower above it, DESIGN.md section 3.6): a launcher
-// names the tensor its kernel PRODUCES for the next kernel (set_l2_window) and launch_pdl attaches it to the launch as
-// an access-policy window with the persisting property, so that the 126 MB L2 keeps the freshly written activations
-// (26-79 MB) instead of streaming them to HBM and back.  The set-aside is configured once per device.
-void set_l2_window(const void* ptr, size_t bytes);
-bool take_l2_window(cudaAccessPolicyWindow* w);
-
-// <<<grid, block, smem, stream>>> with the programmatic-dependent-launch attribute; the kernel must call pdl_enter()
-// before it touches global memory
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (take_l2_window(&attr[1].val.accessPolicyWindow)) {
-    attr[1].id = cudaLaunchAttributeAccessPolicyWindow;
-    cfg.numAttrs = 2;
-  }
-  return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-
 }  // namespace mmfm

@@ -32,7 +32,6 @@ __global__ void __launch_bounds__(kLnWarps * 32) layernorm_fwd_kernel(const floa
                                                                        bf16* __restrict__ y, float* __restrict__ mean,
                                                                        float* __restrict__ rstd, int R, int H,
                                                                        float eps, int modmajor_T, int S) {
-  pdl_enter();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long BT = modmajor_T > 0 ? (long long)(R / S) * modmajor_T : 0;
   const float invH = 1.0f / (float)H;
@@ -161,7 +160,6 @@ __global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_kernel(
     bf16* __restrict__ dxb, DropCfg drop, float* __restrict__ dgamma, float* __restrict__ dbeta, int R, int H,
     int modmajor_T, int S, float* __restrict__ ws, unsigned int* tickets) {
   static_assert(NV > 0, "register path only");
-  pdl_enter();
   __shared__ float red[kLnWarps][NV * 128 + 4];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long BT = modmajor_T > 0 ? (long long)(R / S) * modmajor_T : 0;
@@ -263,7 +261,6 @@ __global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_kernel(
 // ------------------------------------------------------------------------------------------------------------
 template <int NV>
 __global__ void __launch_bounds__(kLnWarps * 32) layernorm_fwd_multi_kernel(const mmfm_ln_multi_args a) {
-  pdl_enter();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int R = a.R, H = a.H;
   const float invH = 1.0f / (float)H;
@@ -323,7 +320,6 @@ template <int NV, int NL, bool DET = false>
 __global__ void __launch_bounds__(kLnWarps * 32) layernorm_bwd_multi_kernel(const mmfm_ln_multi_args a,
                                                                             float* __restrict__ ws,
                                                                             unsigned int* tickets) {
-  pdl_enter();
   __shared__ float red[kLnWarps][128 * NV + 4];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int R = a.R, H = a.H;
@@ -576,9 +572,8 @@ extern "C" int mmfm_layernorm_fwd(const float* x, const float* gamma, const floa
                "mmfm_layernorm_fwd: modality-major remap needs S %% T == 0 and R %% S == 0");
   cudaStream_t st = (cudaStream_t)stream;
   const int grid = ln_grid_fwd(R, H);
-  set_l2_window(y, (size_t)R * H * 2);   // read next by the projection GEMM
 #define LN_FWD(NV) \
-  MMFM_CHECK_CUDA(launch_pdl(layernorm_fwd_kernel<NV>, dim3(grid), dim3(kLnWarps * 32), 0, st, x, gamma, beta, (bf16*)y, mean, rstd, R, H, eps, modmajor_T, S))
+  layernorm_fwd_kernel<NV><<<grid, kLnWarps * 32, 0, st>>>(x, gamma, beta, (bf16*)y, mean, rstd, R, H, eps, modmajor_T, S)
   switch (H) {
     case 128: LN_FWD(1); break;
     case 256: LN_FWD(2); break;
@@ -609,14 +604,14 @@ extern "C" int mmfm_layernorm_bwd(const void* dy, const float* x, const float* m
   cudaStream_t st = (cudaStream_t)stream;
   // fewer, fatter CTAs than the forward (every CTA ends with 2*H atomics); exactly one resident wave
   const int want = (R + kLnWarps * 4 - 1) / (kLnWarps * 4);
-  if (dxb) set_l2_window(dxb, (size_t)R * H * 2);   // read next by a dgrad GEMM
 #define LN_BWD(NV)                                                                                                \
   do {                                                                                                            \
     static int cap = 0;                                                                                           \
     if (cap == 0) cap = resident_ctas(layernorm_bwd_kernel<NV>, kLnWarps * 32);                                   \
     const int grid = want < cap ? (want < 1 ? 1 : want) : cap;                                                    \
-    MMFM_CHECK_CUDA(launch_pdl(layernorm_bwd_kernel<NV>, dim3(grid), dim3(kLnWarps * 32), 0, st, (const bf16*)dy, x, mean,  \
-                               rstd, gamma, dres, dx, (bf16*)dxb, dc, dgamma, dbeta, R, H, modmajor_T, S, nullptr, nullptr)); \
+    layernorm_bwd_kernel<NV><<<grid, kLnWarps * 32, 0, st>>>((const bf16*)dy, x, mean, rstd, gamma, dres, dx,     \
+                                                             (bf16*)dxb, dc, dgamma, dbeta, R, H, modmajor_T, S,  \
+                                                             nullptr, nullptr);                                   \
   } while (0)
   switch (H) {
     case 128: LN_BWD(1); break;
@@ -652,9 +647,9 @@ extern "C" int mmfm_layernorm_fwd_multi(const mmfm_ln_multi_args* a, void* strea
   cudaStream_t st = (cudaStream_t)stream;
   const int grid = ln_grid_fwd(a->R, a->H);
   switch (a->H) {
-    case 128: MMFM_CHECK_CUDA(launch_pdl(layernorm_fwd_multi_kernel<1>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a)); break;
-    case 256: MMFM_CHECK_CUDA(launch_pdl(layernorm_fwd_multi_kernel<2>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a)); break;
-    default: MMFM_CHECK_CUDA(launch_pdl(layernorm_fwd_multi_kernel<4>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a)); break;
+    case 128: layernorm_fwd_multi_kernel<1><<<grid, kLnWarps * 32, 0, st>>>(*a); break;
+    case 256: layernorm_fwd_multi_kernel<2><<<grid, kLnWarps * 32, 0, st>>>(*a); break;
+    default: layernorm_fwd_multi_kernel<4><<<grid, kLnWarps * 32, 0, st>>>(*a); break;
   }
   MMFM_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -671,10 +666,8 @@ template <int NV, bool DET>
 static int ln_bwd_multi_launch(const mmfm_ln_multi_args* a, cudaStream_t st, float* ws_buf, unsigned int* tickets) {
   const int grid = ln_bwd_multi_grid(a->R, a->H, a->n);
 #define LNB(NL)                                                                                                  \
-  MMFM_CHECK_CUDA(DET ? launch_pdl(layernorm_bwd_multi_kernel<NV, NL, true>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a, \
-                                   ws_buf, tickets)                                                               \
-                      : launch_pdl(layernorm_bwd_multi_kernel<NV, NL>, dim3(grid), dim3(kLnWarps * 32), 0, st, *a,   \
-                                   (float*)nullptr, (unsigned int*)nullptr))
+  if constexpr (DET) layernorm_bwd_multi_kernel<NV, NL, true><<<grid, kLnWarps * 32, 0, st>>>(*a, ws_buf, tickets); \
+  else layernorm_bwd_multi_kernel<NV, NL><<<grid, kLnWarps * 32, 0, st>>>(*a, nullptr, nullptr)
   switch (a->n) {
     case 1: LNB(1); break;
     case 2: LNB(2); break;
@@ -751,11 +744,10 @@ extern "C" int mmfm_layernorm_bwd_det(const void* dy, const float* x, const floa
   }
   cudaStream_t st = (cudaStream_t)stream;
   const int grid = ln_bwd_det_grid(R);
-  if (dxb) set_l2_window(dxb, (size_t)R * H * 2);
 #define LN_BWD_DET(NV)                                                                                            \
-  MMFM_CHECK_CUDA(launch_pdl(layernorm_bwd_kernel<NV, true>, dim3(grid), dim3(kLnWarps * 32), 0, st, (const bf16*)dy, x, \
-                             mean, rstd, gamma, dres, dx, (bf16*)dxb, dc, dgamma, dbeta, R, H, modmajor_T, S,      \
-                             (float*)ws->buf, ws->tickets))
+  layernorm_bwd_kernel<NV, true><<<grid, kLnWarps * 32, 0, st>>>((const bf16*)dy, x, mean, rstd, gamma, dres, dx,  \
+                                                                 (bf16*)dxb, dc, dgamma, dbeta, R, H, modmajor_T, S, \
+                                                                 (float*)ws->buf, ws->tickets)
   switch (H) {
     case 128: LN_BWD_DET(1); break;
     case 256: LN_BWD_DET(2); break;

@@ -24,8 +24,8 @@ import torch
 from torch.autograd.function import once_differentiable
 
 from . import adapter, masker as _masker, ops
-from ._lib import (ACT_DGELU, ACT_DSOFTSIGN, ACT_GELU, ACT_GELU_DG, ACT_MULAUX, ACT_NONE, ACT_ROWDOT_DROP, ACT_SOFTSIGN, LOSS_CE, LOSS_MSE, LOSS_POISSON, MASK_CAUSAL,
-                   MASK_KEY, MASK_KEY_OR_DIAG, CastItem, MmfmError, lib)
+from ._lib import (ACT_DSOFTSIGN, ACT_GELU_DG, ACT_MULAUX, ACT_NONE, ACT_ROWDOT_DROP, ACT_SOFTSIGN, LOSS_CE, LOSS_MSE, LOSS_POISSON, MASK_CAUSAL,
+                   MASK_KEY, MASK_KEY_OR_DIAG, MAX_LN, CastItem, MmfmError, lib)
 from .ops import NO_DROP, DropSpec
 
 bf16 = torch.bfloat16
@@ -76,8 +76,8 @@ def fuse_context_norms(named, n_dec: int) -> bool:
     normalises the gamma-weighted sum of their upstream gradients (mmfm_layernorm_bwd_multi) instead of n passes over the
     context with n read-modify-writes of its gradient.  Their gamma / beta gradients then become final after the LAST
     decoder layer of the backward, so they move behind the decoder layers in the flat gradient order.
-    MMFM_FUSE_CTX_LN=0 keeps the per-layer kernels (ScaleNorm and widths the fused kernels do not take always do)."""
-    if os.environ.get("MMFM_FUSE_CTX_LN", "1") == "0" or n_dec < 2:
+    ScaleNorm, widths the fused kernels do not take and more than MAX_LN decoder layers keep the per-layer kernels."""
+    if n_dec < 2 or n_dec > MAX_LN:
         return False
     w = named.get("decoder.0.context_norm.weight")
     if w is None:
@@ -598,7 +598,7 @@ class Plan:
             # instead of the pre-activation, so the backward epilogue is a single multiply
             A[pre + ".dg"], A[pre + ".g"] = b16(R, inter), b16(R, inter)
             ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=self._bias([pre + ".up_proj.bias"]),
-                        act=ACT_GELU_DG if eng.save_gelu_grad else ACT_GELU, D2=A[pre + ".dg"])
+                        act=ACT_GELU_DG, D2=A[pre + ".dg"])
             ops.gemm_tn(A[pre + ".g"], sh.nat[pre + ".down_proj"], x_out, bias=self._bias([pre + ".down_proj.bias"]),
                         drop=self._drop(SITE_MLP, layer, side, p_drop), res=x_in)
 
@@ -709,15 +709,16 @@ class Plan:
         def mlp_bwd(pre, x_in, ln_name, Gs, inter, dxb, drop_prev):
             duv = du[:, :inter]
             lin_bwd(Gb, A[pre + ".g"], pre + ".down_proj", pre + ".down_proj", duv,
-                    act=ACT_MULAUX if eng.save_gelu_grad else ACT_DGELU, aux=A[pre + ".dg"])
+                    act=ACT_MULAUX, aux=A[pre + ".dg"])
             lin_bwd(duv, A[ln_name], pre + ".up_proj", pre + ".up_proj", dh)
             self._ln_bwd(dh, x_in, ln_name, Gs, Gs, dxb, drop_prev)
 
         def out_proj_bwd(pre, nh, p_drop, kind_o, layer, side):
             """out-projection dgrad (+ wgrad).  At d_head 32 its epilogue also does the attention-backward preparation
             (delta = rowsum(dO * O) per head, output-dropout mask on dO): one launch and one pass over dO / O less per
-            attention call.  Returns True when the attention kernel may skip its own preparation."""
-            fuse = eng.fuse_attn_prep and H // nh == 32
+            attention call.  Returns True when the attention kernel may skip its own preparation.  The TMA-store GEMM,
+            the only one with this epilogue, takes it for H > 64."""
+            fuse = H > 64 and H % 32 == 0 and H // nh == 32
             if fuse:
                 lin_bwd(Gb, A[pre + ".ao"], pre + ".out_proj", pre + ".out_proj", d_ao, act=ACT_ROWDOT_DROP,
                         aux=A[pre + ".ao"], rowdot=self.delta, rowdot_S=S, drop=self._drop(kind_o, layer, side, p_drop))
@@ -1039,14 +1040,7 @@ class Engine:
         self.plans: Dict[Tuple[int, bool, Any, Tuple[str, ...], bool], Plan] = {}
         self.arenas: Dict[Tuple[int, bool], Arena] = {}
         self.ddp = None          # set by parallel.DataParallel
-        import os as _os
-        self.use_graphs = _os.environ.get("MMFM_CUDA_GRAPHS", "1") != "0"
-        # MLP forward saves gelu'(u) (default) or the pre-activation u (MMFM_GELU_SAVE=u: A/B of the two backward epilogues)
-        self.save_gelu_grad = _os.environ.get("MMFM_GELU_SAVE", "dg") != "u"
-        # attention-backward preparation inside the out-projection dgrad epilogue (MMFM_FUSE_ATTN_PREP=0: separate kernel);
-        # needs the TMA-store GEMM, i.e. H > 64
-        self.fuse_attn_prep = (_os.environ.get("MMFM_FUSE_ATTN_PREP", "1") != "0" and self.H > 64 and self.H % 32 == 0
-                               and _os.environ.get("MMFM_GEMM_TS", "1") != "0")
+        self.use_graphs = os.environ.get("MMFM_CUDA_GRAPHS", "1") != "0"
         self.last_plan: Optional[Plan] = None
         from .model import MultiModalOutput
         self.output_cls = MultiModalOutput      # dropin.install() swaps in the reference's own dataclass

@@ -74,7 +74,6 @@ def _wgrad_restated(R, NO, KI, sm):
     return tiles * splits * (kBM * BN + kBM) * 4, tiles * splits
 
 
-@pytest.mark.skipif("MMFM_WGRAD_CTAS_X2" in os.environ, reason="restatement assumes the default split target")
 @pytest.mark.parametrize("R,NO,KI", [
     (51200, 768, 256), (51200, 256, 256), (51200, 512, 256), (51200, 256, 512), (51200, 668, 256), (25600, 256, 1336),
     (25600, 1336, 668), (25600, 256, 4), (3200, 256, 256), (130, 200, 72), (64, 8, 8),

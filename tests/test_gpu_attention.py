@@ -54,6 +54,7 @@ def _ref(q, k, v, allowed, nh, d, keep_p=None, keep_o=None):
     (2, 4, 32, 100, 100, 1, False, 10),       # one key half, one query tile (persistent fused backward, smallest form)
     (1, 4, 32, 256, 256, 0, False, 0),        # the largest shape the fused kernels take: two full halves / tiles
     (2, 4, 32, 200, 120, 2, False, 0),        # two query tiles over a single key half, causal
+    (2, 4, 32, 150, 150, 1, False, 10),       # Sq % 4 != 0: the fused backward refuses it, the streamed pair takes it
 ])
 @pytest.mark.parametrize("dropout", [False, True])
 def test_attention_fwd_bwd(B, nh, d, Sq, Sk, mode, sep, pad, dropout):

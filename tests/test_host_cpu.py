@@ -212,21 +212,22 @@ def test_heldout_mask_compact_form_equals_reference():
         assert r["eval_mask"].dtype == torch.int64 and np.array_equal(r["eval_mask"].numpy(), dense[:, :, 0]), (mode, i)
 
 
-def test_flat_gradient_order_with_fused_context_norms(monkeypatch):
+def test_flat_gradient_order_with_and_without_fused_context_norms():
     """The decoder layers' context_norm gradients come out of ONE launch after the last decoder layer of the backward
     (engine.fuse_context_norms), so in the flat gradient order -- reverse execution order, the data-parallel bucket
     order -- they sit behind every decoder-layer parameter and in front of decoder_proj_context; with the fusion off they
-    stay inside their layers.  Either way the order is a permutation of all parameters."""
+    stay inside their layers.  Either way the order is a permutation of all parameters.  The fused LayerNorm kernels take
+    at most MAX_LN layers, so 9 decoder layers at H = 128 are not fused."""
     from multi_modal_foundation_model_b200 import engine
     from multi_modal_foundation_model_b200.model import build_model
-    m = build_model(40, 2, default_model_config(n_layers=3))
-    named = dict(m.named_parameters(remove_duplicate=False))
-    for fused in (True, False):
-        monkeypatch.setenv("MMFM_FUSE_CTX_LN", "1" if fused else "0")
-        assert engine.fuse_context_norms(named, 3) is fused
+    for n_dec, fused, cfg in ((3, True, default_model_config(n_layers=3)),
+                              (9, False, default_model_config(n_layers=9, hidden_size=128, n_heads=4))):
+        m = build_model(40, 2, cfg)
+        named = dict(m.named_parameters(remove_duplicate=False))
+        assert engine.fuse_context_norms(named, n_dec) is fused
         order = engine.ParamStore._execution_reverse_order(m, named)
         assert sorted(order) == sorted(named)
-        ctx = [order.index(f"decoder.{i}.context_norm.weight") for i in range(3)]
+        ctx = [order.index(f"decoder.{i}.context_norm.weight") for i in range(n_dec)]
         last_layer_param = max(order.index(n) for n in order if n.startswith("decoder.") and ".context_norm." not in n)
         if fused:
             assert min(ctx) > last_layer_param and max(ctx) < order.index("decoder_proj_context.weight")
