@@ -54,6 +54,7 @@ enum TsEpi : int {
   TS_BF16 = 0,       // D(bf16) = v
   TS_SOFTSIGN = 1,   // D(bf16) = softsign(v) * s
   TS_F32 = 2,        // D(f32)  = v
+  TS_GELU = 3,       // D(bf16) = gelu(v)                       (forward-only MLP-up: no derivative stored)
   TS_GELU_DG = 4,    // D(bf16) = gelu(v) ; D2(bf16) = gelu'(v)
   TS_MULAUX = 5,     // D(bf16) = v * aux
   TS_DSOFTSIGN = 6,  // D(bf16) = v * s * (1 - |aux / s|)^2
@@ -318,6 +319,14 @@ __global__ void __launch_bounds__(kTsThreads, 1) gemm_tn_ts_kernel(const __grid_
 #pragma unroll
               for (int j = 0; j < 16; j += 2) gelu_erf_both2(v[j], v[j + 1], v[j], v[j + 1], d2[j], d2[j + 1]);
             }
+            if (EPI == TS_GELU) {
+              // the same evaluation as TS_GELU_DG, so D is bit for bit what that flavour writes; the derivative is dead
+#pragma unroll
+              for (int j = 0; j < 16; j += 2) {
+                float g0, g1;
+                gelu_erf_both2(v[j], v[j + 1], v[j], v[j + 1], g0, g1);
+              }
+            }
             uint4 wdrop = make_uint4(0u, 0u, 0u, 0u);
             if (EPI == TS_ROWDOT && drop)
               wdrop = drop_bytes16(seed, p.drop.site, (uint64_t)r, drop_gpr, (uint32_t)((nb + c0) >> 4));
@@ -467,6 +476,10 @@ int try_launch_gemm_ts(const mmfm_gemm_args* a, cudaStream_t st) {
       if (f32 || a->D2) return 0;
       epi = TS_SOFTSIGN;
       break;
+    case MMFM_ACT_GELU:
+      if (f32 || a->D2) return 0;        // with D2 (the pre-activation) it stays on gemm_tn_kernel
+      epi = TS_GELU;
+      break;
     case MMFM_ACT_GELU_DG:
       if (f32 || !a->D2 || !al16(a->D2)) return 0;
       epi = TS_GELU_DG;
@@ -489,6 +502,7 @@ int try_launch_gemm_ts(const mmfm_gemm_args* a, cudaStream_t st) {
     case TS_BF16: rc = launch_ts<TS_BF16>(a, st); break;
     case TS_SOFTSIGN: rc = launch_ts<TS_SOFTSIGN>(a, st); break;
     case TS_F32: rc = launch_ts<TS_F32>(a, st); break;
+    case TS_GELU: rc = launch_ts<TS_GELU>(a, st); break;
     case TS_GELU_DG: rc = launch_ts<TS_GELU_DG>(a, st); break;
     case TS_MULAUX: rc = launch_ts<TS_MULAUX>(a, st); break;
     case TS_DSOFTSIGN: rc = launch_ts<TS_DSOFTSIGN>(a, st); break;

@@ -24,7 +24,7 @@ import torch
 from torch.autograd.function import once_differentiable
 
 from . import adapter, masker as _masker, ops
-from ._lib import (ACT_DSOFTSIGN, ACT_GELU_DG, ACT_MULAUX, ACT_NONE, ACT_ROWDOT_DROP, ACT_SOFTSIGN, LOSS_CE, LOSS_MSE, LOSS_POISSON, MASK_CAUSAL,
+from ._lib import (ACT_DSOFTSIGN, ACT_GELU, ACT_GELU_DG, ACT_MULAUX, ACT_NONE, ACT_ROWDOT_DROP, ACT_SOFTSIGN, LOSS_CE, LOSS_MSE, LOSS_POISSON, MASK_CAUSAL,
                    MASK_KEY, MASK_KEY_OR_DIAG, MAX_LN, CastItem, MmfmError, lib)
 from .ops import NO_DROP, DropSpec
 
@@ -246,6 +246,7 @@ class ParamStore:
                 return False
         return True
 
+    @torch.inference_mode(False)
     @torch.no_grad()
     def adopt(self) -> None:
         """Re-home every Parameter's storage into the flat buffer (values preserved)."""
@@ -349,9 +350,27 @@ class Arena:
         return t
 
 
+class PinnedStage:
+    """Pinned host buffer feeding an asynchronous H2D copy (a pageable source would make the copy a sync point).  The
+    DMA reads the buffer when the copy executes, not when it is enqueued, so a host running steps ahead of the device
+    would ship a later step's values; a rewrite therefore waits for the event recorded after the previous copy."""
+
+    def __init__(self, shape, dtype):
+        self.host = torch.zeros(*shape, dtype=dtype).pin_memory()
+        self.copied = torch.cuda.Event()
+
+    def copy_to(self, dst: torch.Tensor, src: torch.Tensor) -> None:
+        self.copied.synchronize()
+        self.host.copy_(src)
+        dst.copy_(self.host, non_blocking=True)
+        self.copied.record()
+
+
 # ------------------------------------------------------------------------------------------------------------
 class Plan:
     """All buffers + the recorded forward / backward launch lists for one (batch size, train/eval) shape."""
+
+    fwd_only = False
 
     def __init__(self, eng: "Engine", B: int, training: bool, session=None, arena: Optional[Arena] = None,
                  u8_mods: Tuple[str, ...] = (), grad_inputs: Tuple[str, ...] = ()):
@@ -375,7 +394,8 @@ class Plan:
         self._keep: List[Any] = []
         # deterministic mode (torch.use_deterministic_algorithms): the cross-CTA reductions of the backward go through
         # the *_det kernels on this one workspace, sized after recording to the largest call (one stream: shared)
-        self.det_ws = ops.DetWorkspace() if ops.deterministic() else None
+        self.det_ws = ops.DetWorkspace() if ops.deterministic() and not self.fwd_only else None
+        self._bufs: Dict[Any, torch.Tensor] = {}     # forward-only plan: the scratch buffers every layer reuses (_scratch)
 
         def raw(shape, dtype, esize):
             n = int(np.prod(shape)) * esize
@@ -416,9 +436,9 @@ class Plan:
         # per-modality 32-bit Bernoulli thresholds of the device-side mask sampler (0 = read the mask buffer); a device
         # array so that the captured graph sees per-step changes, staged through pinned host memory
         self.sample_thresh = torch.zeros(len(mods), device=dev, dtype=torch.int32)
-        self._thresh_host = torch.zeros(len(mods), dtype=torch.int32).pin_memory()
+        self._thresh_stage = PinnedStage((len(mods),), torch.int32)
         self._thresh_cur = [0] * len(mods)
-        self._mask_host = {m.name: torch.zeros(B, T, dtype=torch.int64).pin_memory() for m in mods}
+        self._mask_stage = {m.name: PinnedStage((B, T), torch.int64) for m in mods}
         # ---- mask products -------------------------------------------------------------------------------
         self.zero, self.kvalid, self.tmask = u8(S), u8(B, S), u8(B, S)
         self.nex, self.inv_n = i64(len(mods)), f32(1)
@@ -429,12 +449,14 @@ class Plan:
         self.partials = torch.zeros(len(mods) * self.n_partials, device=dev)
         self.mod_loss, self.loss = f32(len(mods)), f32(1)
 
+        self.wgrad_writes: List[Tuple[int, Tuple[str, ...]]] = []   # (wgrad call index, parameters it writes)
         rec_f, rec_b = ops.Recorder(), ops.Recorder()
         ops.set_recorder(rec_f)
         try:
             self._build_forward(f32, b16)
-            ops.set_recorder(rec_b)
-            self._build_backward(f32, b16)
+            if not self.fwd_only:
+                ops.set_recorder(rec_b)
+                self._build_backward(f32, b16)
         finally:
             ops.set_recorder(None)
         self._g_fwd = self._g_bwd = None
@@ -457,9 +479,21 @@ class Plan:
             return NO_DROP
         return DropSpec(self.seed, site_id(kind, layer, side), p)
 
+    def _scratch(self, key, make):
+        """A buffer the forward writes.  The training plan takes a new one per call: the backward reads each.  The
+        forward-only plan takes one per key and reuses it in every layer: the next layer overwrites it after its last
+        reader has run."""
+        if not self.fwd_only:
+            return make()
+        t = self._bufs.get(key)
+        if t is None:
+            t = self._bufs[key] = make()
+        return t
+
     def _ln_fwd(self, x, name, y, stats, modmajor=False):
         st = self.eng.store
-        mean, rstd = torch.empty(self.R, device=x.device), torch.empty(self.R, device=x.device)
+        new = lambda: torch.empty(self.R, device=x.device)
+        mean, rstd = self._scratch("ln_mean", new), self._scratch("ln_rstd", new)
         self._keep += [mean, rstd]
         stats[name] = (mean, rstd)
         if st.has(name + ".scale"):       # ScaleNorm: `mean` unused, `rstd` holds 1 / max(||x||, eps)
@@ -511,10 +545,11 @@ class Plan:
         B, S, H = self.B, self.S, self.eng.H
         d = H // nh
         if fwd:
-            self.lse[tag] = torch.empty(B, nh, S, device=q.device)
+            self.lse[tag] = self._scratch(("lse", nh), lambda: torch.empty(B, nh, S, device=q.device))
             dp = self._drop(kind_p, layer, side, p_drop)
             if dp.thresh:
-                self.pkeep[tag] = torch.zeros(B * nh * S * ((S + 63) // 64) * 4, device=q.device, dtype=torch.int16)
+                self.pkeep[tag] = self._scratch(("pkeep", nh), lambda: torch.zeros(B * nh * S * ((S + 63) // 64) * 4,
+                                                                                   device=q.device, dtype=torch.int16))
         dp = self._drop(kind_p, layer, side, p_drop)
         do = self._drop(kind_o, layer, side, p_drop)
         kw = dict(B=B, n_heads=nh, Sq=S, Sk=S, d_head=d, mask_mode=mode, mod_q=self.mod_ids if sep else None,
@@ -536,6 +571,17 @@ class Plan:
         self.pkeep: Dict[str, torch.Tensor] = {}
         self.act: Dict[str, torch.Tensor] = {}   # saved bf16 activations by name
         A = self.act
+        fo = self.fwd_only
+
+        def act(key, r, c):
+            return self._scratch((key, c), lambda: b16(r, c))
+
+        def resid(prev, pair):
+            """Output of a residual sub-layer whose input is `prev`: a buffer of its own in the training plan (the backward
+            reads every one); in the forward-only plan the other buffer of `pair` (the residual GEMM never runs in place)."""
+            if not fo:
+                return f32(R, H)
+            return pair[1] if prev is pair[0] else pair[0]
 
         sh.refresh()
         ops.mask_prep([self.mask[m.name] for m in mods], [self.attn[m.name] for m in mods], [m.C for m in mods],
@@ -579,39 +625,50 @@ class Plan:
                                 drop=drop, remap=(T, S, off), row_zero=self.zero, res=self.emb[side])
 
         def attn_block(pre, x_in, x_out, ln_name, mode, nh, p_drop, layer, side, sep):
-            A[ln_name] = b16(R, H)
+            A[ln_name] = act("ln", R, H)
             self._ln_fwd(x_in, ln_name, A[ln_name], self.stats)
-            A[pre + ".qkv"] = b16(R, 3 * H)
+            A[pre + ".qkv"] = act("qkv", R, 3 * H)
             ops.gemm_tn(A[ln_name], sh.nat[pre + ".qkv"], A[pre + ".qkv"],
                         bias=self._bias([f"{pre}.{k}.bias" for k in ("query", "key", "value")]))
             qkv = A[pre + ".qkv"]
-            A[pre + ".ao"] = b16(R, H)
+            A[pre + ".ao"] = act("ao", R, H)
             self._attention(True, pre, qkv[:, :H], qkv[:, H:2 * H], qkv[:, 2 * H:], A[pre + ".ao"], mode, nh, p_drop,
                             SITE_ATTN_PROB, SITE_ATTN_OUT, layer, side, sep)
             ops.gemm_tn(A[pre + ".ao"], sh.nat[pre + ".out_proj"], x_out, bias=self._bias([pre + ".out_proj.bias"]),
                         res=x_in)
 
         def mlp_block(pre, x_in, x_out, ln_name, p_drop, layer, side, inter):
-            A[ln_name] = b16(R, H)
+            A[ln_name] = act("ln", R, H)
             self._ln_fwd(x_in, ln_name, A[ln_name], self.stats)
-            # saved for backward: gelu(u) (operand of the down projection and of its wgrad) and gelu'(u) -- the derivative
-            # instead of the pre-activation, so the backward epilogue is a single multiply
-            A[pre + ".dg"], A[pre + ".g"] = b16(R, inter), b16(R, inter)
-            ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=self._bias([pre + ".up_proj.bias"]),
-                        act=ACT_GELU_DG, D2=A[pre + ".dg"])
+            up_bias = self._bias([pre + ".up_proj.bias"])
+            if fo and inter > 64 and inter % 4 == 0:
+                # no backward to feed: gelu(u) alone, from the TMA-store kernel's TS_GELU epilogue (the evaluation of its
+                # TS_GELU_DG flavour, which the training plan's call below takes at these widths: the same bits)
+                A[pre + ".g"] = act("g", R, inter)
+                ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=up_bias, act=ACT_GELU)
+            else:
+                # saved for backward: gelu(u) (operand of the down projection and of its wgrad) and gelu'(u) -- the
+                # derivative instead of the pre-activation, so the backward epilogue is a single multiply
+                A[pre + ".dg"], A[pre + ".g"] = act("dg", R, inter), act("g", R, inter)
+                ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=up_bias, act=ACT_GELU_DG,
+                            D2=A[pre + ".dg"])
             ops.gemm_tn(A[pre + ".g"], sh.nat[pre + ".down_proj"], x_out, bias=self._bias([pre + ".down_proj.bias"]),
                         drop=self._drop(SITE_MLP, layer, side, p_drop), res=x_in)
 
         # ---- encoder (encoder_embeddings.py:106-116; mm.py:197-204) ----------------------------------------
         hp = eng.hp
+        # forward-only: the encoder alternates between its embedding output and the decoder's embedding sum (dead once
+        # the embedders have run); it ends where it started, so the decoder then alternates with that buffer
+        pair = (self.xs[0], self.emb[SIDE_DEC])
         for i in range(eng.Le):
             pre = f"encoder.{i}"
-            self.xs += [f32(R, H), f32(R, H)]
+            for _ in range(2):
+                self.xs.append(resid(self.xs[-1], pair))
             attn_block(pre + ".attn", self.xs[2 * i], self.xs[2 * i + 1], pre + ".ln1", MASK_KEY_OR_DIAG,
                        hp["enc_heads"], hp["enc_dropout"], i, SIDE_ENC, False)
             mlp_block(pre + ".mlp", self.xs[2 * i + 1], self.xs[2 * i + 2], pre + ".ln2", hp["enc_dropout"], i,
                       SIDE_ENC, eng.enc_inter)
-        A["encoder_norm"] = b16(R, H)
+        A["encoder_norm"] = act("ln", R, H)
         self._ln_fwd(self.xs[-1], "encoder_norm", A["encoder_norm"], self.stats)
         # context = decoder_proj_context(x) + encoder_emb (mm.py:292)
         self.ctx = f32(R, H)
@@ -630,31 +687,33 @@ class Plan:
                 self.stats[n] = (cmean, crstd)
             ops.layernorm_fwd_multi(self.ctx, [st.p(n + ".weight") for n in names], [st.p(n + ".bias") for n in names],
                                     [A[n] for n in names], cmean, crstd, R=R, H=H)
+        pair = (self.ys[0], self.xs[-1])
         for i in range(eng.Ld):
             pre = f"decoder.{i}"
-            self.ys += [f32(R, H), f32(R, H), f32(R, H)]
+            for _ in range(3):
+                self.ys.append(resid(self.ys[-1], pair))
             y0, y1, y2, y3 = self.ys[3 * i: 3 * i + 4]
             attn_block(pre + ".attn", y0, y1, pre + ".ln1", dec_mode, hp["dec_heads"], hp["dec_dropout"], i, SIDE_DEC,
                        eng.sep)
             # cross attention: q from query_norm(y), k/v from context_norm(context), mask = ENCODER mask
             xa = pre + ".cross_attn"
-            A[pre + ".query_norm"] = b16(R, H)
+            A[pre + ".query_norm"] = act("ln", R, H)
             self._ln_fwd(y1, pre + ".query_norm", A[pre + ".query_norm"], self.stats)
             if not eng.fuse_ctx:
-                A[pre + ".context_norm"] = b16(R, H)
+                A[pre + ".context_norm"] = act("context_norm", R, H)
                 self._ln_fwd(self.ctx, pre + ".context_norm", A[pre + ".context_norm"], self.stats)
-            A[xa + ".q"], A[xa + ".kv"] = b16(R, H), b16(R, 2 * H)
+            A[xa + ".q"], A[xa + ".kv"] = act("xq", R, H), act("xkv", R, 2 * H)
             ops.gemm_tn(A[pre + ".query_norm"], sh.nat[xa + ".query"], A[xa + ".q"], bias=self._bias([xa + ".query.bias"]))
             ops.gemm_tn(A[pre + ".context_norm"], sh.nat[xa + ".kv"], A[xa + ".kv"],
                         bias=self._bias([xa + ".key.bias", xa + ".value.bias"]))
-            A[xa + ".ao"] = b16(R, H)
+            A[xa + ".ao"] = act("ao", R, H)
             self._attention(True, xa, A[xa + ".q"], A[xa + ".kv"][:, :H], A[xa + ".kv"][:, H:], A[xa + ".ao"],
                             MASK_KEY_OR_DIAG, hp["dec_heads"], hp["dec_dropout"], SITE_XATTN_PROB, SITE_XATTN_OUT, i,
                             SIDE_DEC, False)
             ops.gemm_tn(A[xa + ".ao"], sh.nat[xa + ".out_proj"], y2, bias=self._bias([xa + ".out_proj.bias"]), res=y1)
             mlp_block(pre + ".mlp", y2, y3, pre + ".ln2", hp["dec_dropout"], i, SIDE_DEC, eng.dec_inter)
         # decoder_norm, written modality-major so that every head reads a contiguous [B*T, H] block
-        A["decoder_norm"] = b16(R, H)
+        A["decoder_norm"] = act("ln", R, H)
         self._ln_fwd(self.ys[-1], "decoder_norm", A["decoder_norm"], self.stats, modmajor=True)
 
         # ---- heads + fused masked loss / gradient (decoder_embeddings.py:95-109; mm.py:217-239) -------------
@@ -667,7 +726,7 @@ class Plan:
                 ops.smallc_head_fwd(ym, st.p(pre + ".weight"), st.p(pre + ".bias"), pr, R=BT, H=H, Cc=m.C)
             else:
                 ops.gemm_tn(ym, sh.nat[pre], pr, bias=st.p(pre + ".bias"))
-            self.dpreds[m.name] = b16(BT, m.C)
+            self.dpreds[m.name] = act("dpreds", BT, m.C)      # forward-only: written, never read
             ops.loss_fwd_bwd(pr, self.tgt[m.name].view(BT, m.C), self.tmask, self.inv_n, m.loss_kind,
                              self.partials[k * self.n_partials:(k + 1) * self.n_partials], self.dpreds[m.name], B=B,
                              T=T, Cc=m.C, S=S, off=k * T)
@@ -687,7 +746,6 @@ class Plan:
         self.delta = f32(B, max(hp["enc_heads"], hp["dec_heads"]), S)
         ddec = b16(R, H)                                       # gradient wrt decoder_norm output (modality-major)
         self.grad_marks: List[Tuple[int, int]] = []           # (calls issued, flat-gradient offset that is final)
-        self.wgrad_writes: List[Tuple[int, Tuple[str, ...]]] = []   # (wgrad call index, parameters it writes)
 
         def mark(next_param: Optional[str]):
             rec = ops._REC
@@ -884,9 +942,8 @@ class Plan:
 
     def set_sample_thresh(self, thresh: List[int]) -> None:
         if thresh != self._thresh_cur:
-            for k, v in enumerate(thresh):
-                self._thresh_host[k] = v - (1 << 32) if v >= (1 << 31) else v      # uint32 bit pattern in an int32
-            self.sample_thresh.copy_(self._thresh_host, non_blocking=True)
+            bits = [v - (1 << 32) if v >= (1 << 31) else v for v in thresh]       # uint32 bit pattern in an int32
+            self._thresh_stage.copy_to(self.sample_thresh, torch.tensor(bits, dtype=torch.int32))
             self._thresh_cur = list(thresh)
 
     def backward_schedule(self) -> Tuple[Tuple[int, ...], List[Any], List[Tuple[int, int]]]:
@@ -953,6 +1010,17 @@ class Plan:
             self._bwd_body()
 
 
+class ForwardPlan(Plan):
+    """The forward schedule alone, for steps that run with gradients disabled (torch.no_grad / inference_mode): no
+    backward launches, nothing saved for one.  Buffers are allocated by liveness: two fp32 residual-stream buffers used
+    in turn (plus the two embedding sums and the context), one bf16 buffer per activation role reused by every layer,
+    and one LN-statistics / LSE / dropout-keep / head-gradient buffer that the kernels write and nothing reads.  The
+    footprint does not grow with depth, and the MLP-up epilogue stores gelu(u) without its derivative.  Launch for
+    launch the training plan's forward otherwise: same kernels, seed advance, masks and dropout sites, same results."""
+
+    fwd_only = True
+
+
 # ------------------------------------------------------------------------------------------------------------
 class _StepFn(torch.autograd.Function):
     """Autograd node of one step: forward = the plan's forward schedule; backward = its backward schedule, writing
@@ -986,6 +1054,9 @@ class _StepFn(torch.autograd.Function):
 class Engine:
     _created = 0
 
+    # the engine's buffers (flat parameters, seed, plans) are never inference tensors, even when the first step runs
+    # under torch.inference_mode(): training steps write them in place afterwards
+    @torch.inference_mode(False)
     def __init__(self, model):
         self.model = model
         p0 = next(model.parameters())
@@ -1039,6 +1110,9 @@ class Engine:
         self.shadows = Shadows(self.store, model, self.sessions)
         self.plans: Dict[Tuple[int, bool, Any, Tuple[str, ...], bool], Plan] = {}
         self.arenas: Dict[Tuple[int, bool], Arena] = {}
+        # steps with gradients disabled: forward-only plans, and the arenas they share across sessions
+        self.fwd_plans: Dict[Tuple[int, bool, Any, Tuple[str, ...], bool], ForwardPlan] = {}
+        self.fwd_arenas: Dict[Tuple[int, bool], Arena] = {}
         self.ddp = None          # set by parallel.DataParallel
         self.use_graphs = os.environ.get("MMFM_CUDA_GRAPHS", "1") != "0"
         self.last_plan: Optional[Plan] = None
@@ -1046,34 +1120,36 @@ class Engine:
         self.output_cls = MultiModalOutput      # dropin.install() swaps in the reference's own dataclass
 
     # ---------------------------------------------------------------------------------------------------
+    @torch.inference_mode(False)
     def _plan(self, B: int, T: int, training: bool, session=None, u8_mods: Tuple[str, ...] = (),
-              grad_inputs: Tuple[str, ...] = ()) -> Plan:
+              grad_inputs: Tuple[str, ...] = (), fwd_only: bool = False) -> Plan:
         if self.T is None:
             self.T = T
         elif self.T != T:
-            self.plans.clear()
-            self.arenas.clear()
+            for d in (self.plans, self.arenas, self.fwd_plans, self.fwd_arenas):
+                d.clear()
             self.T = T
+        plans, arenas, cls = (self.fwd_plans, self.fwd_arenas, ForwardPlan) if fwd_only else (self.plans, self.arenas, Plan)
         # deterministic mode selects other kernels: its own plan (and graphs), never a change to a captured one
         # input-gradient plans record extra launches after the default schedule: their own plan, like the two above
         key = (B, training, session, u8_mods, ops.deterministic(), grad_inputs)
-        pl = self.plans.get(key)
+        pl = plans.get(key)
         if pl is None:
             arena = None
             if self.multi_session:
                 akey = (B, training, bool(grad_inputs))
-                arena = self.arenas.get(akey)
+                arena = arenas.get(akey)
                 if arena is None:
                     # size the shared arena from the widest session (buffers grow monotonically with the channels);
                     # with input gradients, probe with every modality's
                     widest = max(self.sessions, key=lambda k: sum(m.C for m in self.sessions[k][1]))
                     gi = tuple(m.name for m in self.sessions[widest][1]) if grad_inputs else ()
-                    probe = Plan(self, B, training, widest, grad_inputs=gi)
+                    probe = cls(self, B, training, widest, grad_inputs=gi)
                     nbytes = probe.arena_bytes + (1 << 20)
                     del probe
-                    arena = self.arenas[akey] = Arena(nbytes, self.device)
-            pl = Plan(self, B, training, session, arena, u8_mods, grad_inputs)
-            self.plans[key] = pl
+                    arena = arenas[akey] = Arena(nbytes, self.device)
+            pl = cls(self, B, training, session, arena, u8_mods, grad_inputs)
+            plans[key] = pl
         return pl
 
     def reseed(self, value: int) -> None:
@@ -1115,7 +1191,7 @@ class Engine:
                                               "targets are data here; only inputs and parameters get gradients)")
         # modalities whose (floating-point) inputs require grad: extra inputs of the autograd node
         grad_inputs = tuple(m.name for m in mods if grad_on and mod_dict[m.name]["inputs"].requires_grad)
-        pl = self._plan(B, T, training, session, u8_mods, grad_inputs)
+        pl = self._plan(B, T, training, session, u8_mods, grad_inputs, fwd_only=not grad_on)
         thresh = [0] * len(mods)
         for k, m in enumerate(mods):
             d = mod_dict[m.name]
@@ -1152,10 +1228,7 @@ class Engine:
                     regions = d.get("inputs_regions") if m.name == "ap" else None          # mm.py:254
                     col = _masker.sample_mask_column(mk, (B, T, m.C), regions,
                                                      "fast" if stream == "device" else stream)
-                    # pinned staging: the H2D copy is asynchronous (a pageable source would make it a sync point)
-                    hb = pl._mask_host[m.name]
-                    hb.copy_(col)
-                    pl.mask[m.name].copy_(hb, non_blocking=True)
+                    pl._mask_stage[m.name].copy_to(pl.mask[m.name], col)
             elif isinstance(em, (bool, int)):
                 # compact form (SURVEY 8f rank 3): the trainer's encoding / decoding masks are all-ones or all-zeros
                 # (trainer/base.py:85-96); a scalar says so without a dense (B,T,N) int64 tensor
