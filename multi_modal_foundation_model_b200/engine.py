@@ -16,6 +16,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import warnings
 import weakref
 from typing import Any, Dict, List, Optional, Sequence, Tuple
 
@@ -84,6 +85,23 @@ def fuse_context_norms(named, n_dec: int) -> bool:
         return False
     H = w.numel()
     return H in (128, 256, 512) and (H // 128) * n_dec <= 12
+
+
+def memory_for_plan(free: int, total: int, reserved: int, allocated: int, fraction: float, margin: int) -> int:
+    """Bytes a new plan may take: what torch's caching allocator can still obtain from the device without exceeding its
+    per-process memory fraction, plus what it holds unused, less ``margin`` (the step's own allocations)."""
+    return min(free, int(fraction * total) - reserved) + (reserved - allocated) - margin
+
+
+def step_margin(transient: int, flat_bytes: int, moments: bool) -> int:
+    """Device bytes a training step allocates besides its plan: the output / input-gradient tensors (``transient``),
+    the flat-gradient copy of gradient accumulation and, until the fused AdamW has allocated them at its first step,
+    its two moment buffers."""
+    return transient + flat_bytes + (0 if moments else 2 * flat_bytes)
+
+
+def _round_alloc(n: int) -> int:
+    return (n + 511) // 512 * 512          # the caching allocator's block granularity
 
 
 def flat_layout(order: Sequence[str], named) -> Tuple[Dict[str, str], Dict[str, int], Dict[str, torch.Size], int]:
@@ -172,6 +190,7 @@ class ParamStore:
         self.params = {n: named[n] for n in self.offset}
         self.bucket_order = [n for n in order if self.alias[n] == n]
         self._grad_views: Optional[Dict[str, torch.Tensor]] = None
+        self.moments: "weakref.WeakSet[torch.Tensor]" = weakref.WeakSet()    # optim.AdamW's moment buffers, once bound
         self.adopt()
 
     @staticmethod
@@ -368,24 +387,35 @@ class PinnedStage:
 
 # ------------------------------------------------------------------------------------------------------------
 class Plan:
-    """All buffers + the recorded forward / backward launch lists for one (batch size, train/eval) shape."""
+    """All buffers + the recorded forward / backward launch lists for one (batch size, train/eval) shape.
+
+    ``recompute``: the plan saves only the fp32 residual stream at every layer boundary (plus the embedders, the context,
+    the final norms and the heads); each layer's other activations live in scratch buffers every layer reuses, and the
+    backward records that layer's forward again from its checkpoint before the layer's own backward.  Engine._plan picks
+    it when the plan that saves everything does not fit in device memory.
+
+    ``dry``: size the plan without allocating it -- every buffer is a meta tensor, the launches are recorded and dropped;
+    ``arena_bytes`` and ``nbytes`` come out as they would for the plan built."""
 
     fwd_only = False
 
     def __init__(self, eng: "Engine", B: int, training: bool, session=None, arena: Optional[Arena] = None,
-                 u8_mods: Tuple[str, ...] = (), grad_inputs: Tuple[str, ...] = ()):
+                 u8_mods: Tuple[str, ...] = (), grad_inputs: Tuple[str, ...] = (), recompute: bool = False,
+                 dry: bool = False):
         self.eng, self.B, self.training = eng, B, training
         self.u8_mods = tuple(u8_mods)      # modalities whose inputs / targets arrive as uint8 counts (wire format)
         self.grad_inputs = tuple(grad_inputs)   # modalities whose inputs get a gradient (recorded after the last mark)
-        self.arena_bytes = 0
-        if arena is not None:
+        self.recompute = bool(recompute) and not self.fwd_only
+        self.arena_bytes = 0               # bytes of the activation buffers (taken from `arena` when one is given)
+        self.nbytes = 0                    # every device buffer of the plan: arena_bytes + the rest + det workspace
+        if arena is not None and not dry:
             arena.reset()
         self.prefix, self.mods = eng.sessions[session]
-        dev = eng.device
+        dev = self._dev = torch.device("meta") if dry else eng.device
         # the session's index in eng.sessions (= in store.session_ranges), also as an int32 device scalar: the id this
         # plan contributes to the data-parallel session exchange
         self.session_index = list(eng.sessions).index(session)
-        self.session_id = torch.tensor([self.session_index], device=dev, dtype=torch.int32)
+        self.session_id = self._new(1, dtype=torch.int32).fill_(self.session_index)
         mods, T, H = self.mods, eng.T, eng.H
         S = T * len(mods)
         R, BT = B * S, B * T
@@ -395,15 +425,17 @@ class Plan:
         # deterministic mode (torch.use_deterministic_algorithms): the cross-CTA reductions of the backward go through
         # the *_det kernels on this one workspace, sized after recording to the largest call (one stream: shared)
         self.det_ws = ops.DetWorkspace() if ops.deterministic() and not self.fwd_only else None
-        self._bufs: Dict[Any, torch.Tensor] = {}     # forward-only plan: the scratch buffers every layer reuses (_scratch)
+        self._bufs: Dict[Any, torch.Tensor] = {}     # scratch buffers every layer reuses (_scratch)
 
         def raw(shape, dtype, esize):
             n = int(np.prod(shape)) * esize
-            self.arena_bytes += (n + Arena.ALIGN - 1) // Arena.ALIGN * Arena.ALIGN
-            if arena is not None:
+            a = (n + Arena.ALIGN - 1) // Arena.ALIGN * Arena.ALIGN
+            self.arena_bytes += a
+            self.nbytes += a
+            if arena is not None and not dry:
                 t = arena.take(n).view(dtype).view(*shape)
             else:
-                t = torch.empty(*shape, device=dev, dtype=dtype)
+                t = self._new(*shape, dtype=dtype, count=False)
             self._keep.append(t)      # recorded launches hold raw pointers: the plan owns (or pins) every buffer
             return t
 
@@ -414,39 +446,40 @@ class Plan:
             return raw((r, _pad(c)), bf16, 2)[:, :c]
 
         def i64(*s):
-            return torch.zeros(*s, device=dev, dtype=torch.int64)
+            return self._new(*s, dtype=torch.int64, zero=True)
 
         def u8(*s):
-            return torch.zeros(*s, device=dev, dtype=torch.uint8)
+            return self._new(*s, dtype=torch.uint8, zero=True)
 
+        self._f32, self._b16 = f32, b16
         # ---- static inputs -------------------------------------------------------------------------------
         self.inp = {m.name: f32(B, T, m.C) for m in mods}
         self.tgt = {m.name: f32(B, T, m.C) for m in mods}
         # byte staging of the uint8 wire format: expanded on the device (inputs -> bf16 GEMM operand, targets -> fp32)
-        self.inp_u8 = {n: torch.zeros(B, T, eng_c, device=dev, dtype=torch.uint8)
-                       for n, eng_c in ((m.name, m.C) for m in mods) if n in self.u8_mods}
-        self.tgt_u8 = {n: torch.zeros_like(t) for n, t in self.inp_u8.items()}
+        self.inp_u8 = {m.name: u8(B, T, m.C) for m in mods if m.name in self.u8_mods}
+        self.tgt_u8 = {m.name: u8(B, T, m.C) for m in mods if m.name in self.u8_mods}
         self.attn = {m.name: i64(B, T) for m in mods}
         self.ts = {m.name: i64(B, T) for m in mods}
         self.mask = {m.name: i64(B, T) for m in mods}
         self.seed = eng.seed               # ONE device seed per engine: every plan's launches capture the same pointer
-        self.gscale = torch.ones(1, device=dev, dtype=torch.float32)
-        self.one = torch.ones(1, device=dev, dtype=torch.float32)
+        self.gscale = self._new(1).fill_(1.0)
+        self.one = self._new(1).fill_(1.0)
         self._dpreds_dirty = False         # dpreds overwritten by head_grad since the last forward
         # per-modality 32-bit Bernoulli thresholds of the device-side mask sampler (0 = read the mask buffer); a device
         # array so that the captured graph sees per-step changes, staged through pinned host memory
-        self.sample_thresh = torch.zeros(len(mods), device=dev, dtype=torch.int32)
-        self._thresh_stage = PinnedStage((len(mods),), torch.int32)
+        self.sample_thresh = self._new(len(mods), dtype=torch.int32, zero=True)
+        self._thresh_stage = None if dry else PinnedStage((len(mods),), torch.int32)
         self._thresh_cur = [0] * len(mods)
-        self._mask_stage = {m.name: PinnedStage((B, T), torch.int64) for m in mods}
+        self._mask_stage = {} if dry else {m.name: PinnedStage((B, T), torch.int64) for m in mods}
         # ---- mask products -------------------------------------------------------------------------------
         self.zero, self.kvalid, self.tmask = u8(S), u8(B, S), u8(B, S)
         self.nex, self.inv_n = i64(len(mods)), f32(1)
-        self.mod_ids = torch.repeat_interleave(torch.tensor([m.index for m in mods], dtype=torch.int16), T).to(dev)
+        self.mod_ids = self._new(S, dtype=torch.int16)
+        self.mod_ids.copy_(torch.repeat_interleave(torch.tensor([m.index for m in mods], dtype=torch.int16), T))
         # ---- outputs -------------------------------------------------------------------------------------
         self.preds = {m.name: f32(B, T, m.C) for m in mods}
         self.n_partials = 2 * max(1, lib().mmfm_sm_count())
-        self.partials = torch.zeros(len(mods) * self.n_partials, device=dev)
+        self.partials = self._new(len(mods) * self.n_partials, zero=True)
         self.mod_loss, self.loss = f32(len(mods)), f32(1)
 
         self.wgrad_writes: List[Tuple[int, Tuple[str, ...]]] = []   # (wgrad call index, parameters it writes)
@@ -459,6 +492,7 @@ class Plan:
                 self._build_backward(f32, b16)
         finally:
             ops.set_recorder(None)
+            del self._f32, self._b16      # they hold the plan: a dropped plan must free its buffers right away
         self._g_fwd = self._g_bwd = None
         self._n_fwd_runs = self._n_bwd_runs = 0
         self.fwd_calls, self.bwd_calls = rec_f.calls, rec_b.calls
@@ -470,32 +504,49 @@ class Plan:
         self._variants: Dict[Tuple[int, ...], Dict[str, Any]] = {}
         self._keep += rec_f.keep + rec_b.keep
         if self.det_ws is not None:
-            self.det_ws.materialize(dev)
+            ws = self.det_ws       # materialize allocates max(16, bytes) and max(1, tickets) int32 for a new workspace
+            self.nbytes += _round_alloc(max(16, ws.want_bytes)) + _round_alloc(4 * max(1, ws.want_tickets))
+            if not dry:
+                ws.materialize(dev)
         self.n_fwd, self.n_bwd = len(self.fwd_calls), len(self.bwd_calls)
 
     # ---------------------------------------------------------------------------------------------------
+    def _new(self, *shape, dtype=torch.float32, zero: bool = False, count: bool = True) -> torch.Tensor:
+        """A device buffer of the plan (a meta tensor in a dry plan), counted in nbytes."""
+        t = (torch.zeros if zero else torch.empty)(*shape, device=self._dev, dtype=dtype)
+        if count:
+            self.nbytes += _round_alloc(t.numel() * t.element_size())
+        return t
+
     def _drop(self, kind: int, layer: int, side: int, p: float) -> DropSpec:
         if not self.training or p <= 0.0:
             return NO_DROP
         return DropSpec(self.seed, site_id(kind, layer, side), p)
 
-    def _scratch(self, key, make):
+    def _scratch(self, key, make, role=None, save: bool = False):
         """A buffer the forward writes.  The training plan takes a new one per call: the backward reads each.  The
         forward-only plan takes one per key and reuses it in every layer: the next layer overwrites it after its last
-        reader has run."""
-        if not self.fwd_only:
+        reader has run.  The recompute plan takes one per (key, role) -- `role` tells apart the buffers of one key that
+        a layer's backward reads together -- and a new one per call for what its backward reads unrecomputed (`save`)."""
+        if self.recompute and not save:
+            key = (key, role)
+        elif not self.fwd_only:
             return make()
         t = self._bufs.get(key)
         if t is None:
             t = self._bufs[key] = make()
         return t
 
-    def _ln_fwd(self, x, name, y, stats, modmajor=False):
+    def _act(self, key, r, c, role=None, save: bool = False):
+        """bf16 activation [r, c] (see _scratch)."""
+        return self._scratch((key, c), lambda: self._b16(r, c), role, save)
+
+    def _ln_fwd(self, x, name, y, role=None, save: bool = False, modmajor=False):
         st = self.eng.store
-        new = lambda: torch.empty(self.R, device=x.device)
-        mean, rstd = self._scratch("ln_mean", new), self._scratch("ln_rstd", new)
+        new = lambda: self._new(self.R)
+        mean, rstd = self._scratch("ln_mean", new, role, save), self._scratch("ln_rstd", new, role, save)
         self._keep += [mean, rstd]
-        stats[name] = (mean, rstd)
+        self.stats[name] = (mean, rstd)
         if st.has(name + ".scale"):       # ScaleNorm: `mean` unused, `rstd` holds 1 / max(||x||, eps)
             assert not modmajor
             ops.scalenorm_fwd(x, st.p(name + ".scale"), y, rstd, R=self.R, H=self.eng.H)
@@ -545,11 +596,11 @@ class Plan:
         B, S, H = self.B, self.S, self.eng.H
         d = H // nh
         if fwd:
-            self.lse[tag] = self._scratch(("lse", nh), lambda: torch.empty(B, nh, S, device=q.device))
+            self.lse[tag] = self._scratch(("lse", nh), lambda: self._new(B, nh, S), kind_p)
             dp = self._drop(kind_p, layer, side, p_drop)
             if dp.thresh:
-                self.pkeep[tag] = self._scratch(("pkeep", nh), lambda: torch.zeros(B * nh * S * ((S + 63) // 64) * 4,
-                                                                                   device=q.device, dtype=torch.int16))
+                self.pkeep[tag] = self._scratch(("pkeep", nh), lambda: self._new(B * nh * S * ((S + 63) // 64) * 4,
+                                                                                 dtype=torch.int16, zero=True), kind_p)
         dp = self._drop(kind_p, layer, side, p_drop)
         do = self._drop(kind_o, layer, side, p_drop)
         kw = dict(B=B, n_heads=nh, Sq=S, Sk=S, d_head=d, mask_mode=mode, mod_q=self.mod_ids if sep else None,
@@ -573,15 +624,18 @@ class Plan:
         A = self.act
         fo = self.fwd_only
 
-        def act(key, r, c):
-            return self._scratch((key, c), lambda: b16(r, c))
+        act = self._act
 
-        def resid(prev, pair):
+        def resid(prev, pair, mid=None):
             """Output of a residual sub-layer whose input is `prev`: a buffer of its own in the training plan (the backward
-            reads every one); in the forward-only plan the other buffer of `pair` (the residual GEMM never runs in place)."""
-            if not fo:
-                return f32(R, H)
-            return pair[1] if prev is pair[0] else pair[0]
+            reads every one); in the forward-only plan the other buffer of `pair` (the residual GEMM never runs in place).
+            The recompute plan owns the layer boundaries (its checkpoints) and reuses one buffer per mid-layer position
+            `mid` in every layer."""
+            if fo:
+                return pair[1] if prev is pair[0] else pair[0]
+            if mid is not None:
+                return self._scratch("resid", lambda: f32(R, H), mid)
+            return f32(R, H)
 
         sh.refresh()
         ops.mask_prep([self.mask[m.name] for m in mods], [self.attn[m.name] for m in mods], [m.C for m in mods],
@@ -624,64 +678,27 @@ class Plan:
                     ops.gemm_tn(A[pre + ".hid"], sh.nat[pre + ".projection"], x0, bias=st.p(pre + ".projection.bias"),
                                 drop=drop, remap=(T, S, off), row_zero=self.zero, res=self.emb[side])
 
-        def attn_block(pre, x_in, x_out, ln_name, mode, nh, p_drop, layer, side, sep):
-            A[ln_name] = act("ln", R, H)
-            self._ln_fwd(x_in, ln_name, A[ln_name], self.stats)
-            A[pre + ".qkv"] = act("qkv", R, 3 * H)
-            ops.gemm_tn(A[ln_name], sh.nat[pre + ".qkv"], A[pre + ".qkv"],
-                        bias=self._bias([f"{pre}.{k}.bias" for k in ("query", "key", "value")]))
-            qkv = A[pre + ".qkv"]
-            A[pre + ".ao"] = act("ao", R, H)
-            self._attention(True, pre, qkv[:, :H], qkv[:, H:2 * H], qkv[:, 2 * H:], A[pre + ".ao"], mode, nh, p_drop,
-                            SITE_ATTN_PROB, SITE_ATTN_OUT, layer, side, sep)
-            ops.gemm_tn(A[pre + ".ao"], sh.nat[pre + ".out_proj"], x_out, bias=self._bias([pre + ".out_proj.bias"]),
-                        res=x_in)
-
-        def mlp_block(pre, x_in, x_out, ln_name, p_drop, layer, side, inter):
-            A[ln_name] = act("ln", R, H)
-            self._ln_fwd(x_in, ln_name, A[ln_name], self.stats)
-            up_bias = self._bias([pre + ".up_proj.bias"])
-            if fo and inter > 64 and inter % 4 == 0:
-                # no backward to feed: gelu(u) alone, from the TMA-store kernel's TS_GELU epilogue (the evaluation of its
-                # TS_GELU_DG flavour, which the training plan's call below takes at these widths: the same bits)
-                A[pre + ".g"] = act("g", R, inter)
-                ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=up_bias, act=ACT_GELU)
-            else:
-                # saved for backward: gelu(u) (operand of the down projection and of its wgrad) and gelu'(u) -- the
-                # derivative instead of the pre-activation, so the backward epilogue is a single multiply
-                A[pre + ".dg"], A[pre + ".g"] = act("dg", R, inter), act("g", R, inter)
-                ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=up_bias, act=ACT_GELU_DG,
-                            D2=A[pre + ".dg"])
-            ops.gemm_tn(A[pre + ".g"], sh.nat[pre + ".down_proj"], x_out, bias=self._bias([pre + ".down_proj.bias"]),
-                        drop=self._drop(SITE_MLP, layer, side, p_drop), res=x_in)
-
         # ---- encoder (encoder_embeddings.py:106-116; mm.py:197-204) ----------------------------------------
-        hp = eng.hp
         # forward-only: the encoder alternates between its embedding output and the decoder's embedding sum (dead once
         # the embedders have run); it ends where it started, so the decoder then alternates with that buffer
         pair = (self.xs[0], self.emb[SIDE_DEC])
         for i in range(eng.Le):
-            pre = f"encoder.{i}"
-            for _ in range(2):
-                self.xs.append(resid(self.xs[-1], pair))
-            attn_block(pre + ".attn", self.xs[2 * i], self.xs[2 * i + 1], pre + ".ln1", MASK_KEY_OR_DIAG,
-                       hp["enc_heads"], hp["enc_dropout"], i, SIDE_ENC, False)
-            mlp_block(pre + ".mlp", self.xs[2 * i + 1], self.xs[2 * i + 2], pre + ".ln2", hp["enc_dropout"], i,
-                      SIDE_ENC, eng.enc_inter)
-        A["encoder_norm"] = act("ln", R, H)
-        self._ln_fwd(self.xs[-1], "encoder_norm", A["encoder_norm"], self.stats)
+            self.xs.append(resid(self.xs[-1], pair, 1))
+            self.xs.append(resid(self.xs[-1], pair))
+            self._enc_layer(i)
+        A["encoder_norm"] = act("ln", R, H, save=True)
+        self._ln_fwd(self.xs[-1], "encoder_norm", A["encoder_norm"], save=True)
         # context = decoder_proj_context(x) + encoder_emb (mm.py:292)
         self.ctx = f32(R, H)
         ops.gemm_tn(A["encoder_norm"], sh.nat["decoder_proj_context"], self.ctx,
                     bias=st.p("decoder_proj_context.bias"), res=self.emb[SIDE_ENC])
 
         # ---- decoder (decoder_embeddings.py:133-147; mm.py:207-214) ----------------------------------------
-        dec_mode = MASK_CAUSAL if eng.causal else MASK_KEY
         if eng.fuse_ctx:   # every layer's context_norm(context) from one read of the context
             names = [f"decoder.{i}.context_norm" for i in range(eng.Ld)]
             for n in names:
                 A[n] = b16(R, H)
-            cmean, crstd = torch.empty(R, device=self.ctx.device), torch.empty(R, device=self.ctx.device)
+            cmean, crstd = self._new(R), self._new(R)
             self._keep += [cmean, crstd]
             for n in names:
                 self.stats[n] = (cmean, crstd)
@@ -689,32 +706,12 @@ class Plan:
                                     [A[n] for n in names], cmean, crstd, R=R, H=H)
         pair = (self.ys[0], self.xs[-1])
         for i in range(eng.Ld):
-            pre = f"decoder.{i}"
-            for _ in range(3):
-                self.ys.append(resid(self.ys[-1], pair))
-            y0, y1, y2, y3 = self.ys[3 * i: 3 * i + 4]
-            attn_block(pre + ".attn", y0, y1, pre + ".ln1", dec_mode, hp["dec_heads"], hp["dec_dropout"], i, SIDE_DEC,
-                       eng.sep)
-            # cross attention: q from query_norm(y), k/v from context_norm(context), mask = ENCODER mask
-            xa = pre + ".cross_attn"
-            A[pre + ".query_norm"] = act("ln", R, H)
-            self._ln_fwd(y1, pre + ".query_norm", A[pre + ".query_norm"], self.stats)
-            if not eng.fuse_ctx:
-                A[pre + ".context_norm"] = act("context_norm", R, H)
-                self._ln_fwd(self.ctx, pre + ".context_norm", A[pre + ".context_norm"], self.stats)
-            A[xa + ".q"], A[xa + ".kv"] = act("xq", R, H), act("xkv", R, 2 * H)
-            ops.gemm_tn(A[pre + ".query_norm"], sh.nat[xa + ".query"], A[xa + ".q"], bias=self._bias([xa + ".query.bias"]))
-            ops.gemm_tn(A[pre + ".context_norm"], sh.nat[xa + ".kv"], A[xa + ".kv"],
-                        bias=self._bias([xa + ".key.bias", xa + ".value.bias"]))
-            A[xa + ".ao"] = act("ao", R, H)
-            self._attention(True, xa, A[xa + ".q"], A[xa + ".kv"][:, :H], A[xa + ".kv"][:, H:], A[xa + ".ao"],
-                            MASK_KEY_OR_DIAG, hp["dec_heads"], hp["dec_dropout"], SITE_XATTN_PROB, SITE_XATTN_OUT, i,
-                            SIDE_DEC, False)
-            ops.gemm_tn(A[xa + ".ao"], sh.nat[xa + ".out_proj"], y2, bias=self._bias([xa + ".out_proj.bias"]), res=y1)
-            mlp_block(pre + ".mlp", y2, y3, pre + ".ln2", hp["dec_dropout"], i, SIDE_DEC, eng.dec_inter)
+            for mid in (1, 2, None):
+                self.ys.append(resid(self.ys[-1], pair, mid))
+            self._dec_layer(i)
         # decoder_norm, written modality-major so that every head reads a contiguous [B*T, H] block
-        A["decoder_norm"] = act("ln", R, H)
-        self._ln_fwd(self.ys[-1], "decoder_norm", A["decoder_norm"], self.stats, modmajor=True)
+        A["decoder_norm"] = act("ln", R, H, save=True)
+        self._ln_fwd(self.ys[-1], "decoder_norm", A["decoder_norm"], save=True, modmajor=True)
 
         # ---- heads + fused masked loss / gradient (decoder_embeddings.py:95-109; mm.py:217-239) -------------
         self.dpreds: Dict[str, torch.Tensor] = {}
@@ -726,11 +723,80 @@ class Plan:
                 ops.smallc_head_fwd(ym, st.p(pre + ".weight"), st.p(pre + ".bias"), pr, R=BT, H=H, Cc=m.C)
             else:
                 ops.gemm_tn(ym, sh.nat[pre], pr, bias=st.p(pre + ".bias"))
-            self.dpreds[m.name] = act("dpreds", BT, m.C)      # forward-only: written, never read
+            self.dpreds[m.name] = act("dpreds", BT, m.C, save=True)      # forward-only: written, never read
             ops.loss_fwd_bwd(pr, self.tgt[m.name].view(BT, m.C), self.tmask, self.inv_n, m.loss_kind,
                              self.partials[k * self.n_partials:(k + 1) * self.n_partials], self.dpreds[m.name], B=B,
                              T=T, Cc=m.C, S=S, off=k * T)
         ops.loss_finalize(self.partials, self.n_partials, len(mods), self.inv_n, self.mod_loss, self.loss)
+
+    # -- one layer's forward: recorded by the forward, and again by the recompute plan's backward (replay=True) ----
+    def _attn_block(self, pre, x_in, x_out, ln_name, mode, nh, p_drop, layer, side, sep):
+        A, sh, R, H = self.act, self.eng.shadows, self.R, self.eng.H
+        A[ln_name] = self._act("ln", R, H, "ln1")
+        self._ln_fwd(x_in, ln_name, A[ln_name], "ln1")
+        A[pre + ".qkv"] = self._act("qkv", R, 3 * H)
+        ops.gemm_tn(A[ln_name], sh.nat[pre + ".qkv"], A[pre + ".qkv"],
+                    bias=self._bias([f"{pre}.{k}.bias" for k in ("query", "key", "value")]))
+        qkv = A[pre + ".qkv"]
+        A[pre + ".ao"] = self._act("ao", R, H, "self")
+        self._attention(True, pre, qkv[:, :H], qkv[:, H:2 * H], qkv[:, 2 * H:], A[pre + ".ao"], mode, nh, p_drop,
+                        SITE_ATTN_PROB, SITE_ATTN_OUT, layer, side, sep)
+        ops.gemm_tn(A[pre + ".ao"], sh.nat[pre + ".out_proj"], x_out, bias=self._bias([pre + ".out_proj.bias"]),
+                    res=x_in)
+
+    def _mlp_block(self, pre, x_in, x_out, ln_name, p_drop, layer, side, inter, replay):
+        A, sh, R, H = self.act, self.eng.shadows, self.R, self.eng.H
+        A[ln_name] = self._act("ln", R, H, "ln2")
+        self._ln_fwd(x_in, ln_name, A[ln_name], "ln2")
+        up_bias = self._bias([pre + ".up_proj.bias"])
+        if (self.fwd_only or (self.recompute and not replay)) and inter > 64 and inter % 4 == 0:
+            # no backward reads this call's outputs: gelu(u) alone, from the TMA-store kernel's TS_GELU epilogue (the
+            # evaluation of its TS_GELU_DG flavour, which the call below takes at these widths: the same bits)
+            A[pre + ".g"] = self._act("g", R, inter)
+            ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=up_bias, act=ACT_GELU)
+        else:
+            # saved for backward: gelu(u) (operand of the down projection and of its wgrad) and gelu'(u) -- the
+            # derivative instead of the pre-activation, so the backward epilogue is a single multiply
+            A[pre + ".dg"], A[pre + ".g"] = self._act("dg", R, inter), self._act("g", R, inter)
+            ops.gemm_tn(A[ln_name], sh.nat[pre + ".up_proj"], A[pre + ".g"], bias=up_bias, act=ACT_GELU_DG,
+                        D2=A[pre + ".dg"])
+        if not replay:     # the down projection's output is the next layer's checkpoint: never recomputed
+            ops.gemm_tn(A[pre + ".g"], sh.nat[pre + ".down_proj"], x_out, bias=self._bias([pre + ".down_proj.bias"]),
+                        drop=self._drop(SITE_MLP, layer, side, p_drop), res=x_in)
+
+    def _enc_layer(self, i, replay=False):
+        """Encoder layer i from xs[2i] to xs[2i+2]; replay stops before the down projection."""
+        eng, hp = self.eng, self.eng.hp
+        pre = f"encoder.{i}"
+        x0, x1, x2 = self.xs[2 * i: 2 * i + 3]
+        self._attn_block(pre + ".attn", x0, x1, pre + ".ln1", MASK_KEY_OR_DIAG, hp["enc_heads"], hp["enc_dropout"], i,
+                         SIDE_ENC, False)
+        self._mlp_block(pre + ".mlp", x1, x2, pre + ".ln2", hp["enc_dropout"], i, SIDE_ENC, eng.enc_inter, replay)
+
+    def _dec_layer(self, i, replay=False):
+        """Decoder layer i from ys[3i] to ys[3i+3]; replay stops before the down projection."""
+        eng, hp, A, sh, R, H = self.eng, self.eng.hp, self.act, self.eng.shadows, self.R, self.eng.H
+        pre = f"decoder.{i}"
+        y0, y1, y2, y3 = self.ys[3 * i: 3 * i + 4]
+        self._attn_block(pre + ".attn", y0, y1, pre + ".ln1", MASK_CAUSAL if eng.causal else MASK_KEY, hp["dec_heads"],
+                         hp["dec_dropout"], i, SIDE_DEC, eng.sep)
+        # cross attention: q from query_norm(y), k/v from context_norm(context), mask = ENCODER mask
+        xa = pre + ".cross_attn"
+        A[pre + ".query_norm"] = self._act("ln", R, H, "query_norm")
+        self._ln_fwd(y1, pre + ".query_norm", A[pre + ".query_norm"], "query_norm")
+        if not eng.fuse_ctx:
+            A[pre + ".context_norm"] = self._act("context_norm", R, H)
+            self._ln_fwd(self.ctx, pre + ".context_norm", A[pre + ".context_norm"], "context_norm")
+        A[xa + ".q"], A[xa + ".kv"] = self._act("xq", R, H), self._act("xkv", R, 2 * H)
+        ops.gemm_tn(A[pre + ".query_norm"], sh.nat[xa + ".query"], A[xa + ".q"], bias=self._bias([xa + ".query.bias"]))
+        ops.gemm_tn(A[pre + ".context_norm"], sh.nat[xa + ".kv"], A[xa + ".kv"],
+                    bias=self._bias([xa + ".key.bias", xa + ".value.bias"]))
+        A[xa + ".ao"] = self._act("ao", R, H, "cross")
+        self._attention(True, xa, A[xa + ".q"], A[xa + ".kv"][:, :H], A[xa + ".kv"][:, H:], A[xa + ".ao"],
+                        MASK_KEY_OR_DIAG, hp["dec_heads"], hp["dec_dropout"], SITE_XATTN_PROB, SITE_XATTN_OUT, i,
+                        SIDE_DEC, False)
+        ops.gemm_tn(A[xa + ".ao"], sh.nat[xa + ".out_proj"], y2, bias=self._bias([xa + ".out_proj.bias"]), res=y1)
+        self._mlp_block(pre + ".mlp", y2, y3, pre + ".ln2", hp["dec_dropout"], i, SIDE_DEC, eng.dec_inter, replay)
 
     # ---------------------------------------------------------------------------------------------------
     def _build_backward(self, f32, b16):
@@ -815,6 +881,8 @@ class Plan:
         for i in reversed(range(eng.Ld)):
             pre = f"decoder.{i}"
             y0, y1, y2, y3 = self.ys[3 * i: 3 * i + 4]
+            if self.recompute:
+                self._dec_layer(i, replay=True)
             mlp_bwd(pre + ".mlp", y2, pre + ".ln2", G, eng.dec_inter, Gb, NO_DROP)
             xa = pre + ".cross_attn"
             fused = out_proj_bwd(xa, hp["dec_heads"], hp["dec_dropout"], SITE_XATTN_OUT, i, SIDE_DEC)
@@ -854,6 +922,8 @@ class Plan:
         self._ln_bwd(dh, self.xs[-1], "encoder_norm", None, Genc, Gb, last_enc_drop)
         for i in reversed(range(eng.Le)):
             pre = f"encoder.{i}"
+            if self.recompute:
+                self._enc_layer(i, replay=True)
             mlp_bwd(pre + ".mlp", self.xs[2 * i + 1], pre + ".ln2", Genc, eng.enc_inter, Gb, NO_DROP)
             prev = self._drop(SITE_MLP, i - 1, SIDE_ENC, hp["enc_dropout"]) if i > 0 else NO_DROP
             attn_bwd(pre + ".attn", self.xs[2 * i], pre + ".ln1", Genc, MASK_KEY_OR_DIAG, hp["enc_heads"],
@@ -1135,22 +1205,59 @@ class Engine:
         key = (B, training, session, u8_mods, ops.deterministic(), grad_inputs)
         pl = plans.get(key)
         if pl is None:
+            recompute = False if fwd_only else self._choose_recompute(B, training, session, u8_mods, grad_inputs)
             arena = None
             if self.multi_session:
-                akey = (B, training, bool(grad_inputs))
+                akey = (B, training, bool(grad_inputs), recompute)
                 arena = arenas.get(akey)
                 if arena is None:
-                    # size the shared arena from the widest session (buffers grow monotonically with the channels);
-                    # with input gradients, probe with every modality's
-                    widest = max(self.sessions, key=lambda k: sum(m.C for m in self.sessions[k][1]))
-                    gi = tuple(m.name for m in self.sessions[widest][1]) if grad_inputs else ()
-                    probe = cls(self, B, training, widest, grad_inputs=gi)
-                    nbytes = probe.arena_bytes + (1 << 20)
-                    del probe
-                    arena = arenas[akey] = Arena(nbytes, self.device)
-            pl = cls(self, B, training, session, arena, u8_mods, grad_inputs)
+                    arena = arenas[akey] = Arena(self._arena_bytes(cls, B, training, grad_inputs, recompute),
+                                                 self.device)
+            pl = cls(self, B, training, session, arena, u8_mods, grad_inputs, recompute=recompute)
             plans[key] = pl
         return pl
+
+    def _arena_bytes(self, cls, B: int, training: bool, grad_inputs, recompute: bool) -> int:
+        """Size of the activation arena the sessions' plans share: the widest session's (buffers grow monotonically
+        with the channels; with input gradients, every modality's), from a dry plan."""
+        widest = max(self.sessions, key=lambda k: sum(m.C for m in self.sessions[k][1]))
+        gi = tuple(m.name for m in self.sessions[widest][1]) if grad_inputs else ()
+        return cls(self, B, training, widest, grad_inputs=gi, recompute=recompute, dry=True).arena_bytes + (1 << 20)
+
+    def _plan_need(self, B: int, training: bool, session, u8_mods, grad_inputs, recompute: bool) -> int:
+        """Device bytes that building this training plan allocates: the dry plan's nbytes, with the shared arena of a
+        multi-session model in place of the plan's share of it (nothing when that arena exists already)."""
+        dry = Plan(self, B, training, session, None, u8_mods, grad_inputs, recompute=recompute, dry=True)
+        if not self.multi_session:
+            return dry.nbytes
+        have = (B, training, bool(grad_inputs), recompute) in self.arenas
+        arena = 0 if have else _round_alloc(self._arena_bytes(Plan, B, training, grad_inputs, recompute))
+        return dry.nbytes - dry.arena_bytes + arena
+
+    def _step_transient_bytes(self, B: int, session, grad_inputs) -> int:
+        """Device bytes a training step allocates outside its plan: the loss / mod_loss / preds clones, the returned
+        masks and example counts, and the input gradients."""
+        mods, T = self.sessions[session][1], self.T
+        n = _round_alloc(4) + _round_alloc(4 * len(mods)) + _round_alloc(8 * len(mods)) + _round_alloc(8 * B * len(mods) * T)
+        n += sum(_round_alloc(4 * B * T * m.C) * (2 if m.name in grad_inputs else 1) for m in mods)
+        return n
+
+    def _choose_recompute(self, B: int, training: bool, session, u8_mods, grad_inputs) -> bool:
+        """True when the training plan that saves every activation does not fit in the memory torch may still use on
+        this device; it then records a recompute plan (Plan.recompute) instead, once, for this plan key."""
+        full = self._plan_need(B, training, session, u8_mods, grad_inputs, False)
+        free, total = torch.cuda.mem_get_info(self.device)
+        flat = _round_alloc(4 * self.store.total)
+        margin = step_margin(self._step_transient_bytes(B, session, grad_inputs), flat, len(self.store.moments) > 0)
+        avail = memory_for_plan(free, total, torch.cuda.memory_reserved(self.device),
+                                torch.cuda.memory_allocated(self.device),
+                                torch.cuda.get_per_process_memory_fraction(self.device), margin)
+        if full <= avail:
+            return False
+        rec = self._plan_need(B, training, session, u8_mods, grad_inputs, True)
+        warnings.warn(f"batch size {B}: the training plan needs {full} bytes of device memory, {avail} are available; "
+                      f"recomputing each layer's activations in the backward instead (plan of {rec} bytes)")
+        return True
 
     def reseed(self, value: int) -> None:
         """Set the step seed (the Philox key of the dropout / mask streams); the next step uses value + one increment."""

@@ -96,6 +96,7 @@ class AdamW(torch.optim.Optimizer):
                 self._names = list(st.params)
                 self._m = torch.zeros_like(st.flat)
                 self._v = torch.zeros_like(st.flat)
+                st.moments.update((self._m, self._v))      # the engine's plan sizing no longer reserves room for them
                 self._steps = torch.zeros(len(self._names), dtype=torch.float32)
                 return
         raise MmfmError("parameters are not owned by a B200 engine: move the model to CUDA and run one forward pass "
